@@ -24,6 +24,10 @@ Rank 0 prints ONE JSON line.
                kernels must beat), own process
 
 `--impl reference`: the reference arm — the unmodified reference module on the host CPU for the same config (batch 128).
+
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the headline path returned in its last timed step as
+DIR/<name>.npy: log_likelihood (float64, per image), x_reconstructed and the latents z0..z{L-1} (float32).  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -437,6 +441,24 @@ def ncu_traffic(kernel_key: str):
         return None
 
 
+DUMP_LIMIT = 64 * 1024 * 1024
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """--dump-outputs: each tensor (batch-major) -> path/<name>.npy on the host.  Above DUMP_LIMIT bytes in all, the first
+    n images of every array are written, n the most that fit (the inputs are seeded, so that sample is fixed)."""
+    import numpy as np
+    host = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    for k, a in host.items():
+        assert a.dtype in (np.float32, np.float64), (k, a.dtype)
+    B = next(iter(host.values())).shape[0]
+    per_image = sum(a.nbytes for a in host.values()) // B
+    n = min(B, DUMP_LIMIT // per_image)
+    os.makedirs(path, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(path, k + ".npy"), a[:n])
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -453,7 +475,13 @@ def main():
     ap.add_argument("--train-eager", action="store_true", help="do not capture the train step in a CUDA graph")
     ap.add_argument("--torch-optimizer", action="store_true",
                     help="train arm: torch clip_grad_value_/clip_grad_norm_/Adam instead of the fused optimiser step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline path returned in its last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.only_train):
+        ap.error("--dump-outputs records the headline path: it needs --impl ours and no --only-train")
     if args.impl == "reference":
         return run_reference(args, on_gpu=False)
     if args.impl == "reference-gpu":
@@ -502,7 +530,7 @@ def main():
 
     def step_dev():
         zs, ll = fwd_dev(x_dev)
-        return ll, flow.invert(zs)
+        return ll, flow.invert(zs), zs
 
     def step_e2e():
         xd = x_host.to(dev, non_blocking=True)
@@ -567,8 +595,16 @@ def main():
                 step_e2e()
             torch.cuda.synchronize()
             l0 = N.launch_count
-            ms = timed(step_dev, args.steps)
+            last = {}
+
+            def step_kept():
+                last["out"] = step_dev()
+            ms = timed(step_kept if full and args.dump_outputs else step_dev, args.steps)
             launches = N.launch_count - l0
+            if rank == 0 and "out" in last:
+                ll, xr, zs = last.pop("out")
+                dump_outputs(args.dump_outputs, {"log_likelihood": ll, "x_reconstructed": xr,
+                                                 **{f"z{i}": z for i, z in enumerate(zs)}})
             ms_e2e = timed(step_e2e, args.steps)
             zs, _ = fwd_dev(x_dev)
             flow.invert(zs)
@@ -587,7 +623,7 @@ def main():
                 out["sample_last_latent"] = {"value": rate(ms_s, args.steps), "unit": "img/s", "ms": ms_s / args.steps,
                                              "what": "Glow.invert([z_last]): every Split draws its half from the learned "
                                                      "conditional prior (glow.py:203-246), T=1"}
-            ll, xr = step_dev()
+            ll, xr, _ = step_dev()
             torch.cuda.synchronize()
             out["checks"] = {"recon_max_abs_err": float((xr - x_dev).abs().max())}
             if rank == 0 and not args.no_cpu_baseline:

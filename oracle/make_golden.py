@@ -1,7 +1,7 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference package.
 
-Runs only in the build container (needs /root/reference); the GPU box uses the committed
-fixtures.  Usage:  python oracle/make_golden.py
+Needs a checkout of the reference named by NFDPM_REFERENCE; the tests use the committed
+fixtures.  Usage:  NFDPM_REFERENCE=<checkout> python oracle/make_golden.py
 
 For every case: weights/inputs come from oracle.glow_oracle.seeded_state / seeded_input
 (numpy PCG64 — regenerated bit-identically by the tests; a checksum is stored to prove it),
@@ -20,7 +20,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = os.environ.get("NFDPM_REFERENCE", "/root/reference")
+REF = os.environ.get("NFDPM_REFERENCE", "")
 
 
 def import_reference():
@@ -29,6 +29,8 @@ def import_reference():
     for m in ["aim", "skimage", "skimage.transform", "cleanfid", "cleanfid.fid", "cleanfid.features",
               "cleanfid.utils", "cleanfid.resize", "ignite", "ignite.metrics"]:
         sys.modules.setdefault(m, MagicMock())
+    if not REF or not os.path.isdir(os.path.join(REF, "normalizing_flow")):
+        raise SystemExit("set NFDPM_REFERENCE to a checkout of the reference project")
     sys.path.insert(0, REF)
     import normalizing_flow as nf  # noqa
     assert os.path.realpath(nf.__file__).startswith(os.path.realpath(REF)), nf.__file__

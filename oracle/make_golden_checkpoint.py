@@ -1,11 +1,11 @@
 """Generate tests/golden/checkpoint_manifest.json from a checkpoint written by the UNMODIFIED reference.
 
-TEST INFRASTRUCTURE ONLY.  Runs in the build container (needs /root/reference).  The reference's own `save_model`
+TEST INFRASTRUCTURE ONLY.  Needs a checkout of the reference named by NFDPM_REFERENCE.  The reference's own `save_model`
 (normalizing_flow/prior.py:102-115) writes `model_gaussian_XXX.pt` for a small Glow + GaussianPrior + Adam after one
 real CPU training step (trainer.py:150-167 recipe); the manifest records the wire format that a drop-in must keep:
 file name, top-level keys, every state_dict key with shape and dtype (in order), the optimiser's param_group keys and
-per-parameter state keys / dtypes.  tests/test_checkpoint_cpu.py holds the product package to it on every box; when
-/root/reference is present the same test file also exchanges real checkpoint files with the reference both ways.
+per-parameter state keys / dtypes.  tests/test_checkpoint_cpu.py holds the product package to it everywhere; when
+NFDPM_REFERENCE names a checkout the same test file also exchanges real checkpoint files with the reference both ways.
 
 Usage:  python oracle/make_golden_checkpoint.py                 # (re)write the manifest
         python oracle/make_golden_checkpoint.py --write DIR     # the reference writes DIR/model_gaussian_007.pt

@@ -1,7 +1,7 @@
 """Generate tests/golden/formats.npz from the UNMODIFIED reference: CatFormater.process_latents / postprocess
 (diffusion_prior/latent_formaters.py), postprocess_batch over its whole clipping range and preprocess_batch + the
-dequantisation noise add (normalizing_flow/utils.py:175-210, trainer.py:155).  Build container only (needs
-/root/reference).  Usage:  python oracle/make_golden_formats.py
+dequantisation noise add (normalizing_flow/utils.py:175-210, trainer.py:155).  Needs a checkout of the reference
+named by NFDPM_REFERENCE.  Usage:  NFDPM_REFERENCE=<checkout> python oracle/make_golden_formats.py
 
 The reference's diffusion_prior/__init__.py imports its trainer (UNet, denoising_diffusion_pytorch ... absent here), so
 latent_formaters.py is loaded as a stand-alone module from its file; nothing in it is modified."""

@@ -3,10 +3,11 @@
 TEST INFRASTRUCTURE ONLY: used by ``bench.py --impl reference`` / ``--impl reference-gpu`` (the reference arms), by
 ``tests/test_dropin_overlay.py`` and by the golden-vector generators — never by the product path.
 
-The reference is pure Python on PyTorch, so "building" it is packing its source tree where the GPU box can see it:
-``stage()`` (called by ``__graft_entry__.build()`` in the build container, where ``/root/reference`` exists) writes ONE
-archive, ``baseline/_ref/reference_src.tar.gz`` — git-ignored, so no reference source enters the history or sits in the
-tree as files, but shipped to the GPU box with the working tree.  ``find()`` unpacks it into the system's temporary
+The reference is not part of this repository: point ``NFDPM_REFERENCE`` at a checkout of it to enable the comparisons
+(without it they are skipped).  It is pure Python on PyTorch, so "building" it is packing its source tree:
+``stage()`` (called by ``__graft_entry__.build()``) writes ONE archive, ``baseline/_ref/reference_src.tar.gz`` —
+git-ignored, so no reference source enters the history or sits in the tree as files, but it travels with a copy of the
+working tree to a machine without the checkout.  ``find()`` unpacks it into the system's temporary
 directory (once per archive content) and ``import_reference()`` imports ``normalizing_flow`` from there with the reference's
 non-hot-path dependencies that this image lacks (aim, skimage, cleanfid, ignite: logging / data / metrics code, reference
 normalizing_flow/utils.py:4, trainer.py:8-13, data/utils.py:9, metrics/compute.py:21-30) stubbed by MagicMock.
@@ -26,7 +27,7 @@ from unittest.mock import MagicMock
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 STAGED = os.path.join(ROOT, "baseline", "_ref")
-SOURCE = os.environ.get("NFDPM_REFERENCE", "/root/reference")
+SOURCE = os.environ.get("NFDPM_REFERENCE") or None
 STUBS = ["aim", "skimage", "skimage.transform", "cleanfid", "cleanfid.fid", "cleanfid.features", "cleanfid.utils",
          "cleanfid.resize", "ignite", "ignite.metrics"]
 
@@ -37,8 +38,8 @@ _SKIP = ("media", ".git", "__pycache__")
 
 def stage(src: str = SOURCE, dst: str = STAGED) -> bool:
     """Pack the reference's Python tree (no media, no VCS data) into ``dst``/reference_src.tar.gz.  Returns False when
-    ``src`` is absent."""
-    if not os.path.isdir(os.path.join(src, "normalizing_flow")):
+    ``src`` is unset or absent."""
+    if not src or not os.path.isdir(os.path.join(src, "normalizing_flow")):
         return False
     if os.path.isdir(dst):
         shutil.rmtree(dst)
@@ -57,7 +58,7 @@ def stage(src: str = SOURCE, dst: str = STAGED) -> bool:
 
 def find() -> str | None:
     """Directory holding an importable copy of the reference tree: the staged archive unpacked under the temporary directory,
-    else the original location (build container)."""
+    else the checkout NFDPM_REFERENCE names."""
     if os.path.isfile(ARCHIVE):
         h = hashlib.sha1(open(ARCHIVE, "rb").read()).hexdigest()[:12]
         out = os.path.join(tempfile.gettempdir(), f"nfdpm_reference_{h}")
@@ -71,7 +72,7 @@ def find() -> str | None:
             except OSError:                    # another process unpacked it meanwhile
                 shutil.rmtree(tmp, ignore_errors=True)
         return root
-    if os.path.isdir(os.path.join(SOURCE, "normalizing_flow")):
+    if SOURCE and os.path.isdir(os.path.join(SOURCE, "normalizing_flow")):
         return SOURCE
     return None
 
@@ -82,7 +83,7 @@ def import_reference(path: str | None = None):
     path = path or find()
     if path is None:
         raise ImportError("no copy of the reference: neither baseline/_ref/reference_src.tar.gz (staged by "
-                          f"__graft_entry__.build()) nor {SOURCE} exists")
+                          f"__graft_entry__.build()) nor NFDPM_REFERENCE={SOURCE!r} exists")
     have = sys.modules.get("normalizing_flow")
     if have is not None:
         if os.path.realpath(getattr(have, "__file__", "")).startswith(os.path.realpath(path)):

@@ -33,6 +33,33 @@ def test_reference_arm_prints_the_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "img/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_dump_outputs_writes_float_arrays_within_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    g = torch.Generator().manual_seed(0)
+    arrays = {"log_likelihood": torch.randn(16, dtype=torch.float64, generator=g),
+              "x_reconstructed": torch.randn(16, 3, 4, 4, generator=g)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    for k, v in arrays.items():
+        a = np.load(tmp_path / "all" / f"{k}.npy")
+        assert a.dtype == v.numpy().dtype and np.array_equal(a, v.numpy()), k
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 5 * (8 + 3 * 4 * 4 * 4) + 7)          # room for five images
+    bench.dump_outputs(str(tmp_path / "cut"), arrays)
+    for k, v in arrays.items():
+        assert np.array_equal(np.load(tmp_path / "cut" / f"{k}.npy"), v.numpy()[:5]), k
+
+
+def test_bench_rejects_bad_step_and_dump_arguments(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)],
+                  ["--only-train", "--dump-outputs", str(tmp_path)]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                           timeout=60, cwd=ROOT)
+        assert r.returncode == 2 and r.stdout == "", (extra, r.stderr)
+    assert os.listdir(tmp_path) == []
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],

@@ -4,8 +4,9 @@ run_baseline_experiment.py:112-114).  CPU only: constructing modules and moving 
 * against tests/golden/checkpoint_manifest.json — written by oracle/make_golden_checkpoint.py from a file the UNMODIFIED
   reference's own save_model produced after one real training step: file name, top-level keys, every key / shape / dtype
   in order, the optimiser layout;
-* when /root/reference is present (the build container; never on the GPU box): real files travel both ways — the reference
-  writes, this package loads strictly, saves again, the reference loads strictly — and every tensor must be bit-identical.
+* when NFDPM_REFERENCE names a checkout of the reference (it is not part of this repository): real files travel both
+  ways — the reference writes, this package loads strictly, saves again, the reference loads strictly — and every tensor
+  must be bit-identical.
 """
 import json
 import os
@@ -18,7 +19,7 @@ import torch
 import normalizing_flow as nf
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("NFDPM_REFERENCE", "/root/reference")
+REF = os.environ.get("NFDPM_REFERENCE", "")
 GEN = os.path.join(ROOT, "oracle", "make_golden_checkpoint.py")
 
 
@@ -92,8 +93,8 @@ def _run_reference(*args):
     return r.stdout.strip().splitlines()[-1]
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "normalizing_flow")),
-                    reason="needs the reference tree (build container only)")
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "normalizing_flow")),
+                    reason="needs a checkout of the reference project named by NFDPM_REFERENCE")
 def test_checkpoints_travel_both_ways_with_the_reference(golden_dir, tmp_path):
     man = _manifest(golden_dir)
     case = man["case"]

@@ -195,3 +195,28 @@ def test_sampling_variant_decodes_what_it_drew(cfg):
     assert torch.isfinite(e).all()
     # with near-zero split ZeroConvs (zero_sigma 1e-3) mean ~ 0 and exp(logs) ~ 1: the latents themselves are ~N(0,1)
     assert abs(float(e.mean())) < 0.02 and abs(float(e.std()) - 1.0) < 0.02, (float(e.mean()), float(e.std()))
+
+
+def test_bench_dump_outputs_hold_what_the_headline_path_returns(tmp_path):
+    """bench.py --dump-outputs writes what its timed headline step returned: the same arrays the public API gives for the
+    bench's own weights and inputs in this process."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--no-train",
+                        "--no-cpu-baseline", "--no-eager-gpu", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, timeout=900, cwd=str(tmp_path))
+    assert r.returncode == 0, r.stderr[-4000:]
+    c, L, K, B, S = 3, 3, 16, 128, 32
+    flow, prior, _, _, x = bench_style_model(c, L, K, B, S, 1e-3)
+    ld, lp = nf.initialize_with_zeros(2, B, DEV)
+    zs, ld, lp = flow.transform(x.to(DEV), ld, lp)
+    lp += prior.compute_log_prob(zs[-1])
+    want = {"log_likelihood": ld + lp, "x_reconstructed": flow.invert(zs), **{f"z{i}": z for i, z in enumerate(zs)}}
+    assert sorted(os.listdir(out)) == sorted(k + ".npy" for k in want)
+    for k, v in want.items():
+        a = np.load(out / f"{k}.npy")
+        v = v.cpu().numpy()
+        assert a.dtype == v.dtype and a.shape == v.shape, (k, a.dtype, a.shape)
+        np.testing.assert_allclose(a, v, rtol=1e-6, atol=1e-6, err_msg=k)
