@@ -193,6 +193,13 @@ int nfdpm_flow_boundary_stash(const float* in, int64_t in_bs, int squeeze_in, co
                               const float* bias3, const float* logs3, float* ld_part, const float* mt, const float* beta,
                               float* y, int64_t y_bs, float* xs, int64_t xs_bs, void* a1, int a1_dtype, int64_t lda1,
                               int B, int C, int H, int W, nfdpm_stream_t stream);
+/* The INVERSE step boundary (coupling^-1 from pm, then the inverse mix mt/beta = inv_mt/inv_beta) with the sinks the
+ * backward of Glow.invert needs: xs [B,C,P] receives the coupling^-1 output u (the inverse mix's input), y the step's
+ * output, a1 (may be NULL) the next network's im2col rows.  No squeeze source, no log-det.  One CTA per image. */
+int nfdpm_flow_boundary_inv_stash(const float* in, int64_t in_bs, const float* pm, int64_t ldp, const float* bias3,
+                                  const float* logs3, const float* mt, const float* beta, float* y, int64_t y_bs, float* xs,
+                                  int64_t xs_bs, void* a1, int a1_dtype, int64_t lda1, int B, int C, int H, int W,
+                                  nfdpm_stream_t stream);
 
 /* ZeroConv GEMM + step boundary in ONE launch (tensor-core mode): pm = h2[M,K] * w3p[ldp,K]^T is accumulated in tensor
  * memory, staged in shared memory and consumed by the arithmetic of nfdpm_flow_boundary (coupling source), so the
@@ -237,6 +244,14 @@ int nfdpm_coupling_bwd(const float* dy, int64_t dy_bs, const float* dld, const f
 /* 1: one CTA per image (dp_scratch unused).  > 1: the image is processed in pixel tiles: dpar has B*tiles rows (reduce
  * with nfdpm_reduce_rows2), dp_scratch [B*H*W*C] floats is required and counter must be NULL. */
 int nfdpm_coupling_bwd_tiles(int C, int H, int W);
+/* Backward of the INVERSE coupling x_b = y_b/(s+1e-6) - t, x_a = y_a (transforms.py:196-200): y is the inverse's input,
+ * dx the gradient of its output.  dy_a = dx_a (the coupling-network part is added later through col2im),
+ * dy_b = dx_b/(s+1e-6); ds = -dx_b*y_b/(s+1e-6)^2, dt = -dx_b.  dpm, dpar, dbias/dlogs/counter, dp_scratch and the
+ * one-CTA-per-image / pixel-tiled choice (nfdpm_coupling_bwd_tiles) are exactly those of nfdpm_coupling_bwd; no log-det. */
+int nfdpm_coupling_inv_bwd(const float* dx, int64_t dx_bs, const float* y, int64_t y_bs, const float* pm, int64_t ldp,
+                           const float* bias3, const float* logs3, float* dy, int64_t dy_bs, void* dpm, int dpm_dtype,
+                           int64_t ld_dpm, float* dpar, float* dbias, float* dlogs, int32_t* counter, float* dp_scratch,
+                           int B, int C, int H, int W, nfdpm_stream_t stream);
 /* ActNorm+ReLU backward on rows (utils.py:69,84-87): dpre = dh*(h>0)*exp(scale); part[cta][2N] partial d(scale), d(bias);
  * ctas = ceil(M/rows_per_cta).  dtypes: any mix of F32 / BF16, or the fp32-faithful form (F32 dh, BF16X2 h) -> BF16X2 dpre. */
 int nfdpm_actnorm_relu_bwd(const void* dh, int dh_dtype, int64_t ld_dh, const void* h, int h_dtype, int64_t ld_h,
@@ -263,6 +278,11 @@ typedef struct {
   float* d_weight; float* d_scale; float* d_bias; float* scratch; /* scratch: C*C + C floats */
 } nfdpm_mix_grad_item;
 int nfdpm_mix_param_grad(const nfdpm_mix_grad_item* items_host, int n, nfdpm_stream_t stream);
+/* Parameter gradients of the INVERSE mix x = M u - b, M = diag(e^-s) W^-1 (transforms.py:92-94,142-145), from the
+ * partials of an nfdpm_mix_bwd run with mt = inv_mt (its x = the inverse input u, its du = grad wrt the output x):
+ * d_bias = -g, d_scale_c = -sum_j G_cj M_cj, d_weight = -W^-T diag(e^-s) G W^-T.  weight may be NULL; winv is W^-1 (the
+ * identity for a lone ActNorm); dld_sum and P are unused; any of d_weight / d_scale / d_bias may be NULL. */
+int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items_host, int n, nfdpm_stream_t stream);
 /* Weight gradients: D[N1,N2] (+)= sum_m A[m,N1]*B[m,N2] (A, B row-major, F32, BF16 or both BF16X2; D fp32 with ldd == N2).
  * Split pairs (needs counters): the tensor-core accumulator holds hi*hi, hi*lo, lo*hi, lo*lo of every logical element and the
  * in-kernel reduction adds the four: the exact product of the represented values.
@@ -285,6 +305,14 @@ int nfdpm_split_prior_bwd(const float* dlp, const float* h, int64_t ldh, const f
 /* GaussianPrior backward (prior.py:79-83): dz [B,C,P]; dpar [B][4C] per-image partials: d(bias)[2C], d(logs)[2C]. */
 int nfdpm_gauss_const_bwd(const float* dl, const float* z, const float* bias, const float* logs, float* dz, float* dpar,
                           int B, int C, int P, nfdpm_stream_t stream);
+/* Backward of the reparameterised prior draw z = mean + exp(lg)*T*eps (transforms.py:305-307, prior.py:49-50,97-99):
+ * (mean, lg) = (h + bias)*exp(3*logs) split into channel halves; C = 2 x latent channels.  dz: [B, C/2, P] with batch
+ * stride dz_bs; eps: [B, C/2, P] contiguous.  d mean = dz, d lg = dz*exp(lg)*T*eps.  Writes dh rows [M, ldh] (columns
+ * C..ldh zero) for the conv's wgrad / dgrad GEMMs and dpar [B][2C]: per-image d(bias)[C], d(logs)[C].  h == NULL: mean / lg
+ * are the per-channel constants bias*exp(3*logs) (GaussianPrior) and dh is not written. */
+int nfdpm_split_sample_bwd(const float* dz, int64_t dz_bs, const float* eps, float temperature, const float* h, int64_t ldh,
+                           const float* bias, const float* logs, float* dh, float* dpar, int B, int C, int H, int W,
+                           nfdpm_stream_t stream);
 /* dstate[b,c,p] += col2im(da)[b,c,p] for c < Cin (input gradient of a 3x3 "same" conv expressed as im2col rows). */
 int nfdpm_col2im_add(const float* da, int64_t lda, float* dstate, int64_t dbs, int B, int Cin, int H, int W,
                      nfdpm_stream_t stream);

@@ -106,7 +106,9 @@ __host__ __device__ __forceinline__ size_t coupling_bwd_floats(int C, int H, int
 // One CTA per image.  Same structure as the forward step boundary (boundary_body.cuh): the image's pm block arrives by
 // bulk copy while the gradients are staged; index divisions are multiply-high; the dpm rows (the transposed-conv scatter
 // dpm[p, tap*C+co] = dP[co][p - shift(tap)]) are gathered from a zero-bordered copy of dP through a column table.
-template <typename TD>
+// INV: backward of the inverse x_b = y_b/(s+1e-6) - t (a.u = the inverse's input y, a.dy = grad wrt its output x; no
+// log-det term): du_b = dx_b/(s+eps), ds = -dx_b*y_b/(s+eps)^2, dt = -dx_b.
+template <typename TD, bool INV>
 __global__ void __launch_bounds__(1024) coupling_bwd_kernel(const CouplingBwdArgs a) {
   extern __shared__ __align__(128) float sm_raw[];
   __shared__ __align__(8) uint64_t pm_bar;
@@ -196,10 +198,19 @@ __global__ void __launch_bounds__(1024) coupling_bwd_kernel(const CouplingBwdArg
     const float t = (tt + par_s[Ch + j]) * g_t;
     const float s = 1.f / (1.f + expf(-(log_s + 2.f)));
     const float dyv = g_s[(Ch + j) * PS + p];
-    const float ds = dyv * (ub_s[j * PS + p] + t) + gld / (s + 1e-6f);
-    const float dt = dyv * s;
+    float ds, dt, dub;
+    if (INV) {
+      const float r = 1.f / (s + 1e-6f);
+      dub = dyv * r;
+      ds = -dub * ub_s[j * PS + p] * r;
+      dt = -dyv;
+    } else {
+      ds = dyv * (ub_s[j * PS + p] + t) + gld / (s + 1e-6f);
+      dt = dyv * s;
+      dub = dyv * s;
+    }
     const float dls = ds * s * (1.f - s);
-    g_s[(Ch + j) * PS + p] = dyv * s;            // du_b
+    g_s[(Ch + j) * PS + p] = dub;                // du_b
     const int pq = (py + 1) * W2p + px + 1;
     dP_pad[j * PP + pq] = dls * g_l;
     dP_pad[(Ch + j) * PP + pq] = dt * g_t;
@@ -311,6 +322,7 @@ __global__ void __launch_bounds__(1024) coupling_bwd_kernel(const CouplingBwdArg
 // Tiled variant for images (or channel counts) that do not fit one CTA: CTA = (image, tile of TP pixels), direct global
 // access; the gradient wrt the gathered conv output goes to dP [M, C] and dpm_expand_kernel scatters it into the
 // taps-as-N rows afterwards (a pixel's dpm row needs dP of its 8 neighbours, which may live in other tiles).
+template <bool INV>
 __global__ void __launch_bounds__(256) coupling_bwd_tiled_kernel(const CouplingBwdArgs a, float* __restrict__ dP, int TP) {
   extern __shared__ __align__(16) float sm[];        // r_s [4][Ch][TP] + par_s [2C]
   const int C = a.C, H = a.H, W = a.W, P = H * W, Ch = C >> 1;
@@ -353,10 +365,19 @@ __global__ void __launch_bounds__(256) coupling_bwd_tiled_kernel(const CouplingB
     const float tv = (tt + par_s[Ch + j]) * g_t;
     const float s = 1.f / (1.f + expf(-(log_s + 2.f)));
     const float dyv = dyb[(int64_t)(Ch + j) * P + p];
-    const float ds = dyv * (ub[(int64_t)(Ch + j) * P + p] + tv) + gld / (s + 1e-6f);
-    const float dt = dyv * s;
+    float ds, dt, duv;
+    if (INV) {
+      const float r = 1.f / (s + 1e-6f);
+      duv = dyv * r;
+      ds = -duv * ub[(int64_t)(Ch + j) * P + p] * r;
+      dt = -dyv;
+    } else {
+      ds = dyv * (ub[(int64_t)(Ch + j) * P + p] + tv) + gld / (s + 1e-6f);
+      dt = dyv * s;
+      duv = dyv * s;
+    }
     const float dls = ds * s * (1.f - s);
-    dub[(int64_t)(Ch + j) * P + p] = dyv * s;
+    dub[(int64_t)(Ch + j) * P + p] = duv;
     float* dpr = dP + ((int64_t)b * P + p) * C;
     dpr[j] = dls * g_l;
     dpr[Ch + j] = dt * g_t;
@@ -644,13 +665,13 @@ struct MixParamItem {
 constexpr int kParamBatch = 16;
 struct MixParamBatch { MixParamItem it[kParamBatch]; };
 
-__global__ void __launch_bounds__(256) mix_param_grad_kernel(const MixParamBatch batch) {
-  const MixParamItem it = batch.it[blockIdx.x];
-  const int C = it.C, n = C * C + C, tid = threadIdx.x;
-  for (int e = tid; e < n; e += 256) {
+// sum of the B per-image partial rows of one item into it.scratch (eight loads in flight, added in order: deterministic)
+__device__ __forceinline__ void mix_reduce_partials(const MixParamItem& it, int tid) {
+  const int n = it.C * it.C + it.C;
+  for (int e = tid; e < n; e += blockDim.x) {
     float acc = 0.f;
     int b = 0;
-    for (; b + 8 <= it.B; b += 8) {                        // eight loads in flight, added in order (deterministic)
+    for (; b + 8 <= it.B; b += 8) {
       float v[8];
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = __ldcg(it.part + (int64_t)(b + j) * n + e);
@@ -660,6 +681,12 @@ __global__ void __launch_bounds__(256) mix_param_grad_kernel(const MixParamBatch
     for (; b < it.B; ++b) acc += __ldcg(it.part + (int64_t)b * n + e);
     it.scratch[e] = acc;
   }
+}
+
+__global__ void __launch_bounds__(256) mix_param_grad_kernel(const MixParamBatch batch) {
+  const MixParamItem it = batch.it[blockIdx.x];
+  const int C = it.C, tid = threadIdx.x;
+  mix_reduce_partials(it, tid);
   __syncthreads();
   const float G = it.dld_sum[0] * it.P;
   // dW^_total[o][i] = dW^x[o][i] + db^[o]*b[i];  W^[o][i] = W[o][i]*exp(s[i])
@@ -680,6 +707,41 @@ __global__ void __launch_bounds__(256) mix_param_grad_kernel(const MixParamBatch
     }
     if (it.ds) it.ds[i] = ds + G;
     if (it.db) it.db[i] = db;
+  }
+}
+
+// The inverse mix x = M u - b, M = diag(e^-s) W^-1, from the partials of a mix_bwd run with mt = inv_mt (G = sum dx u^T,
+// g = sum dx):  db = -g,  ds_c = -sum_j G_cj M_cj,  dW = -W^-T (diag(e^-s) G) W^-T.  One CTA per StepFlow; shared memory
+// holds diag(e^-s) G W^-T [C][C].
+__global__ void __launch_bounds__(256) mix_inv_param_grad_kernel(const MixParamBatch batch) {
+  extern __shared__ float t_s[];
+  const MixParamItem it = batch.it[blockIdx.x];
+  const int C = it.C, tid = threadIdx.x;
+  mix_reduce_partials(it, tid);
+  __syncthreads();
+  const float* G = it.scratch;
+  const float* g = it.scratch + C * C;
+  for (int c = tid; c < C; c += 256) {
+    if (it.db) it.db[c] = -g[c];
+    if (it.ds) {
+      float acc = 0.f;
+      for (int j = 0; j < C; ++j) acc = fmaf(G[c * C + j], it.winv[c * C + j], acc);
+      it.ds[c] = -expf(-it.s[c]) * acc;
+    }
+  }
+  if (it.dW == nullptr) return;
+  for (int e = tid; e < C * C; e += 256) {
+    const int c = e / C, k = e - c * C;
+    float acc = 0.f;
+    for (int d = 0; d < C; ++d) acc = fmaf(G[c * C + d], it.winv[k * C + d], acc);
+    t_s[e] = expf(it.s ? -it.s[c] : 0.f) * acc;
+  }
+  __syncthreads();
+  for (int e = tid; e < C * C; e += 256) {
+    const int a = e / C, k = e - a * C;
+    float acc = 0.f;
+    for (int c = 0; c < C; ++c) acc = fmaf(it.winv[c * C + a], t_s[c * C + k], acc);
+    it.dW[e] = -acc;
   }
 }
 
@@ -846,6 +908,60 @@ __global__ void __launch_bounds__(256) gauss_const_bwd_kernel(const float* __res
   }
 }
 
+// Backward of the reparameterised draw z = mean + exp(lg)*T*eps with (mean, lg) = ((h + bias)*exp(3*logs)) split into
+// channel halves (Split prior, C = 2 x latent channels).  With h == nullptr mean / lg are the per-channel constants
+// bias*exp(3*logs) (GaussianPrior).  d mean = dz, d lg = dz*exp(lg)*T*eps.  One CTA per image, channels in chunks of up to
+// 256: thread t owns channel j0 + t % cw and every rg-th pixel (rg = 256 / cw row groups), so the dh / h rows are read and
+// written along consecutive channels; per-channel partials are combined over the row groups in a fixed order
+// (deterministic).  Writes dh rows [M, ldh] (columns C..ldh zero) when h is given, and dpar [B][2C] (dbias[C], dlogs[C]).
+__global__ void __launch_bounds__(256) split_sample_bwd_kernel(const float* __restrict__ dz, int64_t dz_bs,
+                                                               const float* __restrict__ eps, float temperature,
+                                                               const float* __restrict__ h, int64_t ldh,
+                                                               const float* __restrict__ bias, const float* __restrict__ logs,
+                                                               float* __restrict__ dh, float* __restrict__ dpar, int C, int P) {
+  __shared__ float red[4][256];
+  const int Ch = C >> 1, b = blockIdx.x, tid = threadIdx.x;
+  for (int j0 = 0; j0 < Ch; j0 += 256) {
+    const int cw = min(256, Ch - j0), rg = 256 / cw;
+    const int jl = tid % cw, r = tid / cw, j = j0 + jl;
+    float s_bm = 0.f, s_bl = 0.f, s_lm = 0.f, s_ll = 0.f;
+    if (r < rg) {
+      const float em = expf(3.f * logs[j]), el = expf(3.f * logs[Ch + j]);
+      const float bm = bias[j], bl = bias[Ch + j];
+      for (int p = r; p < P; p += rg) {
+        const int64_t m = (int64_t)b * P + p;
+        const float hm = (h != nullptr) ? h[m * ldh + j] : 0.f, hl = (h != nullptr) ? h[m * ldh + Ch + j] : 0.f;
+        const float mean = (hm + bm) * em, lg = (hl + bl) * el;
+        const float g = dz[b * dz_bs + (int64_t)j * P + p];
+        const float dlg = g * expf(lg) * temperature * eps[((int64_t)b * Ch + j) * P + p];
+        const float dhm = g * em, dhl = dlg * el;
+        if (h != nullptr) {
+          dh[m * ldh + j] = dhm;
+          dh[m * ldh + Ch + j] = dhl;
+        }
+        s_bm += dhm; s_bl += dhl;
+        s_lm += 3.f * g * mean; s_ll += 3.f * dlg * lg;
+      }
+    }
+    red[0][tid] = s_bm; red[1][tid] = s_bl; red[2][tid] = s_lm; red[3][tid] = s_ll;
+    __syncthreads();
+    for (int i = tid; i < 4 * cw; i += 256) {
+      const int k = i / cw, jj = i % cw;
+      float acc = 0.f;
+      for (int q = 0; q < rg; ++q) acc += red[k][q * cw + jj];
+      const int dst[4] = {j0 + jj, Ch + j0 + jj, C + j0 + jj, C + Ch + j0 + jj};
+      dpar[(int64_t)b * 2 * C + dst[k]] = acc;
+    }
+    __syncthreads();
+  }
+  if (h != nullptr) {
+    for (int i = tid; i < P * (int)(ldh - C); i += 256) {
+      const int p = i / (int)(ldh - C), c = C + i % (int)(ldh - C);
+      dh[((int64_t)b * P + p) * ldh + c] = 0.f;
+    }
+  }
+}
+
 // dstate[b, c, p] += sum_tap dA[(b,p - shift(tap)), c*9+tap]   for c < Cin  (col2im of a 3x3 "same" conv input gradient)
 __global__ void col2im_add_kernel(const float* __restrict__ da, int64_t lda, float* __restrict__ dstate, int64_t dbs, int Cin,
                                   int H, int W, int64_t n) {
@@ -894,25 +1010,26 @@ extern "C" int nfdpm_coupling_bwd_tiles(int C, int H, int W) {
   return (P + tp - 1) / tp;
 }
 
-extern "C" int nfdpm_coupling_bwd(const float* dy, int64_t dy_bs, const float* dld, const float* u, int64_t u_bs,
-                                  const float* pm, int64_t ldp, const float* bias3, const float* logs3, float* du,
-                                  int64_t du_bs, void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias,
-                                  float* dlogs, int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
-                                  nfdpm_stream_t stream) {
-  NFDPM_REQUIRE(dy && u && pm && bias3 && logs3 && du && dpm && dpar, "nfdpm_coupling_bwd: null pointer");
+template <bool INV>
+static int coupling_bwd_launch(const float* dy, int64_t dy_bs, const float* dld, const float* u, int64_t u_bs,
+                               const float* pm, int64_t ldp, const float* bias3, const float* logs3, float* du,
+                               int64_t du_bs, void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias,
+                               float* dlogs, int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
+                               cudaStream_t st) {
+  const char* name = INV ? "nfdpm_coupling_inv_bwd" : "nfdpm_coupling_bwd";
+  NFDPM_REQUIRE(dy && u && pm && bias3 && logs3 && du && dpm && dpar, "%s: null pointer", name);
   NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0 && ldp >= 9 * (int64_t)C && ld_dpm >= 9 * (int64_t)C,
-                "nfdpm_coupling_bwd: bad shape");
+                "%s: bad shape", name);
   NFDPM_REQUIRE(dpm_dtype == NFDPM_F32 || dpm_dtype == NFDPM_BF16 || (dpm_dtype == NFDPM_BF16X2 && ld_dpm % 32 == 0),
-                "nfdpm_coupling_bwd: bad dpm dtype");
-  NFDPM_REQUIRE(counter == nullptr || (dbias && dlogs), "nfdpm_coupling_bwd: the fused reduction needs dbias/dlogs");
+                "%s: bad dpm dtype", name);
+  NFDPM_REQUIRE(counter == nullptr || (dbias && dlogs), "%s: the fused reduction needs dbias/dlogs", name);
   const int P = H * W, Ch = C / 2;
-  cudaStream_t st = as_stream(stream);
   static bool attr_set = false;
   if (!attr_set) {
-    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_kernel<bf16x2_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_kernel<float, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_kernel<__nv_bfloat16, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_kernel<bf16x2_t, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    NFDPM_CUDA(cudaFuncSetAttribute(coupling_bwd_tiled_kernel<INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
     attr_set = true;
   }
   size_t smem = coupling_bwd_smem(C, H, W);
@@ -926,14 +1043,14 @@ extern "C" int nfdpm_coupling_bwd(const float* dy, int64_t dy_bs, const float* d
     if (a.pm_bulk) smem += pm_bytes;
     int threads = (P * Ch + 31) / 32 * 32;
     threads = threads > 1024 ? 1024 : (threads < 128 ? 128 : threads);
-    if (dpm_dtype == NFDPM_F32) coupling_bwd_kernel<float><<<B, threads, smem, st>>>(a);
-    else if (dpm_dtype == NFDPM_BF16X2) coupling_bwd_kernel<bf16x2_t><<<B, threads, smem, st>>>(a);
-    else coupling_bwd_kernel<__nv_bfloat16><<<B, threads, smem, st>>>(a);
+    if (dpm_dtype == NFDPM_F32) coupling_bwd_kernel<float, INV><<<B, threads, smem, st>>>(a);
+    else if (dpm_dtype == NFDPM_BF16X2) coupling_bwd_kernel<bf16x2_t, INV><<<B, threads, smem, st>>>(a);
+    else coupling_bwd_kernel<__nv_bfloat16, INV><<<B, threads, smem, st>>>(a);
     NFDPM_CHECK_LAUNCH("coupling_bwd_kernel");
     return 0;
   }
   NFDPM_REQUIRE(dp_scratch != nullptr && counter == nullptr,
-                "nfdpm_coupling_bwd: this image needs the tiled path (dp_scratch, no fused reduction): see nfdpm_coupling_bwd_tiles");
+                "%s: this image needs the tiled path (dp_scratch, no fused reduction): see nfdpm_coupling_bwd_tiles", name);
   const int TP = coupling_bwd_tile(C, P), T = (P + TP - 1) / TP;
   CouplingBwdArgs a{dy, dy_bs, dld, u, u_bs, pm, ldp, bias3, logs3, du, du_bs, dpm, ld_dpm, dpar, B, C, H, W, nullptr,
                     nullptr, nullptr};
@@ -941,7 +1058,7 @@ extern "C" int nfdpm_coupling_bwd(const float* dy, int64_t dy_bs, const float* d
   a.dNg = make_fastdiv(ld_dpm >= 8 ? (int)(ld_dpm >> 3) : 1); a.d2C = make_fastdiv(2 * C);
   a.pm_bulk = 0;
   const size_t smem_t = sizeof(float) * (4 * (size_t)Ch * TP + 2 * C);
-  coupling_bwd_tiled_kernel<<<B * T, 256, smem_t, st>>>(a, dp_scratch, TP);
+  coupling_bwd_tiled_kernel<INV><<<B * T, 256, smem_t, st>>>(a, dp_scratch, TP);
   NFDPM_CHECK_LAUNCH("coupling_bwd_tiled_kernel");
   const int64_t n = (int64_t)B * P * ld_dpm;
   int64_t g = (n + 255) / 256;
@@ -951,6 +1068,24 @@ extern "C" int nfdpm_coupling_bwd(const float* dy, int64_t dy_bs, const float* d
   else dpm_expand_kernel<__nv_bfloat16><<<(int)g, 256, 0, st>>>(dp_scratch, (__nv_bfloat16*)dpm, ld_dpm, C, H, W, n);
   NFDPM_CHECK_LAUNCH("dpm_expand_kernel");
   return 0;
+}
+
+extern "C" int nfdpm_coupling_bwd(const float* dy, int64_t dy_bs, const float* dld, const float* u, int64_t u_bs,
+                                  const float* pm, int64_t ldp, const float* bias3, const float* logs3, float* du,
+                                  int64_t du_bs, void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias,
+                                  float* dlogs, int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
+                                  nfdpm_stream_t stream) {
+  return coupling_bwd_launch<false>(dy, dy_bs, dld, u, u_bs, pm, ldp, bias3, logs3, du, du_bs, dpm, dpm_dtype, ld_dpm, dpar,
+                                    dbias, dlogs, counter, dp_scratch, B, C, H, W, as_stream(stream));
+}
+
+extern "C" int nfdpm_coupling_inv_bwd(const float* dx, int64_t dx_bs, const float* y, int64_t y_bs, const float* pm,
+                                      int64_t ldp, const float* bias3, const float* logs3, float* dy, int64_t dyo_bs,
+                                      void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias, float* dlogs,
+                                      int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
+                                      nfdpm_stream_t stream) {
+  return coupling_bwd_launch<true>(dx, dx_bs, nullptr, y, y_bs, pm, ldp, bias3, logs3, dy, dyo_bs, dpm, dpm_dtype, ld_dpm,
+                                   dpar, dbias, dlogs, counter, dp_scratch, B, C, H, W, as_stream(stream));
 }
 
 extern "C" int nfdpm_actnorm_relu_bwd(const void* dh, int dh_dtype, int64_t ld_dh, const void* h, int h_dtype, int64_t ld_h,
@@ -1071,6 +1206,35 @@ extern "C" int nfdpm_mix_param_grad(const nfdpm_mix_grad_item* items, int n, nfd
   return 0;
 }
 
+extern "C" int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items, int n, nfdpm_stream_t stream) {
+  NFDPM_REQUIRE(items && n > 0, "nfdpm_mix_inv_param_grad: no items");
+  for (int i = 0; i < n; ++i) {
+    const nfdpm_mix_grad_item& s = items[i];
+    NFDPM_REQUIRE(s.part && s.winv && s.scratch && s.C > 0 && s.B > 0 && (s.d_scale == nullptr || s.scale != nullptr),
+                  "nfdpm_mix_inv_param_grad: item %d incomplete", i);
+    NFDPM_REQUIRE(sizeof(float) * (size_t)s.C * s.C <= 200 * 1024, "nfdpm_mix_inv_param_grad: %d channels do not fit", s.C);
+  }
+  static bool attr_set = false;
+  if (!attr_set) {
+    NFDPM_CUDA(cudaFuncSetAttribute(mix_inv_param_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    attr_set = true;
+  }
+  for (int base = 0; base < n; base += kParamBatch) {
+    MixParamBatch pb;
+    const int cnt = (n - base < kParamBatch) ? n - base : kParamBatch;
+    int cmax = 0;
+    for (int i = 0; i < cnt; ++i) {
+      const nfdpm_mix_grad_item& s = items[base + i];
+      pb.it[i] = MixParamItem{s.part, s.B, s.weight, s.scale, s.bias, s.winv, nullptr, s.P, s.d_weight, s.d_scale,
+                              s.d_bias, s.scratch, s.C};
+      if (s.C > cmax) cmax = s.C;
+    }
+    mix_inv_param_grad_kernel<<<cnt, 256, sizeof(float) * (size_t)cmax * cmax, as_stream(stream)>>>(pb);
+    NFDPM_CHECK_LAUNCH("mix_inv_param_grad_kernel");
+  }
+  return 0;
+}
+
 extern "C" int64_t nfdpm_gemm_tn_workspace(int M, int N1, int N2, int* splits_out) {
   // enough splits to fill the GPU (~296 CTAs) but at least 256 rows per split
   const int tiles = ((N1 + 127) / 128) * ((N2 + 127) / 128);
@@ -1156,6 +1320,18 @@ extern "C" int nfdpm_gauss_const_bwd(const float* dl, const float* z, const floa
   NFDPM_REQUIRE(B > 0 && C > 0 && P > 0, "nfdpm_gauss_const_bwd: bad shape");
   gauss_const_bwd_kernel<<<B, 256, 0, as_stream(stream)>>>(dl, z, bias, logs, dz, dpar, C, P);
   NFDPM_CHECK_LAUNCH("gauss_const_bwd_kernel");
+  return 0;
+}
+
+extern "C" int nfdpm_split_sample_bwd(const float* dz, int64_t dz_bs, const float* eps, float temperature, const float* h,
+                                      int64_t ldh, const float* bias, const float* logs, float* dh, float* dpar, int B, int C,
+                                      int H, int W, nfdpm_stream_t stream) {
+  NFDPM_REQUIRE(dz && eps && bias && logs && dpar, "nfdpm_split_sample_bwd: null pointer");
+  NFDPM_REQUIRE(h == nullptr || (dh && ldh >= C), "nfdpm_split_sample_bwd: the conditional form needs dh with ldh >= C");
+  NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_sample_bwd: bad shape");
+  split_sample_bwd_kernel<<<B, 256, 0, as_stream(stream)>>>(dz, dz_bs, eps, temperature, h, ldh, bias,
+                                                                                 logs, dh, dpar, C, H * W);
+  NFDPM_CHECK_LAUNCH("split_sample_bwd_kernel");
   return 0;
 }
 

@@ -135,3 +135,12 @@ extern "C" int nfdpm_flow_boundary_stash(const float* in, int64_t in_bs, int squ
   return flow_boundary_impl(in, in_bs, squeeze_in, pm, ldp, bias3, logs3, ld_part, mt, beta, y, y_bs, xs, xs_bs, a1,
                             a1_dtype, lda1, B, C, H, W, 0, stream);
 }
+
+extern "C" int nfdpm_flow_boundary_inv_stash(const float* in, int64_t in_bs, const float* pm, int64_t ldp,
+                                             const float* bias3, const float* logs3, const float* mt, const float* beta,
+                                             float* y, int64_t y_bs, float* xs, int64_t xs_bs, void* a1, int a1_dtype,
+                                             int64_t lda1, int B, int C, int H, int W, nfdpm_stream_t stream) {
+  NFDPM_REQUIRE(in && pm && bias3 && logs3 && mt && beta && y && xs, "nfdpm_flow_boundary_inv_stash: null pointer");
+  return flow_boundary_impl(in, in_bs, 0, pm, ldp, bias3, logs3, nullptr, mt, beta, y, y_bs, xs, xs_bs, a1, a1_dtype, lda1, B,
+                            C, H, W, 1, stream);
+}

@@ -60,6 +60,12 @@ def coupling_dtype(train: bool = False) -> torch.dtype:
     return torch.bfloat16 if train else N.SPLIT
 
 
+def invert_grad_enabled() -> bool:
+    """``NFDPM_INVERT_GRAD=1``: ``invert`` (Glow, the granular transforms) and the priors' ``sample`` record an autograd
+    node with hand-written backward kernels.  Off by default: ``invert`` then refuses to back-propagate."""
+    return os.environ.get("NFDPM_INVERT_GRAD", "0") == "1"
+
+
 def round_up(a: int, b: int) -> int:
     return (a + b - 1) // b * b
 
@@ -429,12 +435,13 @@ last_coupling_stash = None
 
 
 def coupling_rows(cp, y: torch.Tensor, ybs: int, B: int, C: int, H: int, W: int, init: bool = False,
-                  stash: bool = False) -> Tuple[torch.Tensor, int]:
+                  stash: bool = False, fmt: Optional[torch.dtype] = None) -> Tuple[torch.Tensor, int]:
     """Run the coupling network of AffineCoupling ``cp`` on the first C/2 channels of ``y`` ([B,C,P], batch
     stride ``ybs``).  Returns (pm, ldp): the taps-as-N ZeroConv rows consumed by nfdpm_coupling_apply.
     ``init`` performs the data-dependent initialisation of inner ActNorms that are not initialised yet
     (always in exact fp32).  ``stash``: the training form — operands in the TRAINING format, in fresh tensors that are
-    published as ``last_coupling_stash`` for the module's backward."""
+    published as ``last_coupling_stash`` for the module's backward.  ``fmt`` overrides the operand format (the inverse
+    keeps the no-grad inference format, see coupling_dtype)."""
     global last_coupling_stash
     conv1, an1, conv2, an2, zc = cp._parts()
     F = conv1.weight.shape[0]
@@ -444,7 +451,7 @@ def coupling_rows(cp, y: torch.Tensor, ybs: int, B: int, C: int, H: int, W: int,
     if stash and need_init:
         coupling_rows(cp, y, ybs, B, C, H, W, init=True)          # initialise first (exact fp32), then run the stash pass
         need_init = False
-    dt = torch.float32 if need_init else coupling_dtype(train=stash)     # the data-dependent initialisation runs in exact fp32
+    dt = torch.float32 if need_init else (fmt or coupling_dtype(train=stash))   # the data-dependent init runs in exact fp32
     cache = _pack_coupling(cp._cache, conv1.weight, conv2.weight, zc.weight, dt)
     dev = y.device
     M = B * H * W

@@ -78,10 +78,14 @@ def _load() -> C.CDLL:
                                  i32, vp], C.c_int),
         "nfdpm_coupling_bwd": ([vp, i64, vp, vp, i64, vp, i64, vp, vp, vp, i64, vp, i32, i64, vp, vp, vp, vp, vp, i32, i32,
                                 i32, i32, vp], C.c_int),
+        "nfdpm_coupling_inv_bwd": ([vp, i64, vp, i64, vp, i64, vp, vp, vp, i64, vp, i32, i64, vp, vp, vp, vp, vp, i32, i32,
+                                    i32, i32, vp], C.c_int),
         "nfdpm_coupling_bwd_tiles": ([i32, i32, i32], C.c_int),
         "nfdpm_mix_bwd_tiles": ([i32, i32, i32], C.c_int),
         "nfdpm_flow_boundary_stash": ([vp, i64, i32, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp, i64, vp, i32, i64, i32, i32,
                                        i32, i32, vp], C.c_int),
+        "nfdpm_flow_boundary_inv_stash": ([vp, i64, vp, i64, vp, vp, vp, vp, vp, i64, vp, i64, vp, i32, i64, i32, i32, i32, i32,
+                                           vp], C.c_int),
         "nfdpm_actnorm_relu_bwd": ([vp, i32, i64, vp, i32, i64, vp, vp, i32, i64, vp, i32, i32, i32, vp], C.c_int),
         "nfdpm_reduce_rows2": ([vp, vp, vp, i32, i32, i32, i64, vp], C.c_int),
         "nfdpm_gemm3_boundary_ok": ([i32, i32, i32, i32, i32, i64], C.c_int),
@@ -97,10 +101,12 @@ def _load() -> C.CDLL:
         "nfdpm_reduce_rows": ([vp, vp, i32, i32, i64, i32, vp], C.c_int),
         "nfdpm_mix_bwd": ([vp, i64, vp, i64, vp, i64, vp, vp, i64, vp, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_mix_param_grad": ([C.POINTER(MixGradItem), i32, vp], C.c_int),
+        "nfdpm_mix_inv_param_grad": ([C.POINTER(MixGradItem), i32, vp], C.c_int),
         "nfdpm_gemm_tn_workspace": ([i32, i32, i32, C.POINTER(C.c_int)], C.c_int64),
         "nfdpm_gemm_tn": ([vp, i32, i64, vp, i32, i64, vp, i64, i32, i32, i32, vp, i32, vp, i32, i32, vp], C.c_int),
         "nfdpm_split_prior_bwd": ([vp, vp, i64, vp, vp, vp, i64, vp, i64, vp, vp, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_gauss_const_bwd": ([vp, vp, vp, vp, vp, vp, i32, i32, i32, vp], C.c_int),
+        "nfdpm_split_sample_bwd": ([vp, i64, vp, f32, vp, i64, vp, vp, vp, vp, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_col2im_add": ([vp, i64, vp, i64, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_accumulate": ([vp, i32, vp, i32, i32, vp, vp, i32, vp], C.c_int),
         "nfdpm_flow_boundary_tiles": ([i32, i32, i32, i32, i32, i32, i32], C.c_int),
@@ -126,17 +132,22 @@ _FAMILIES = (("gemm", ("nfdpm_gemm_nt", "nfdpm_gemm_tn")),
                                 "nfdpm_im2col3x3", "nfdpm_actnorm_apply", "nfdpm_squeeze", "nfdpm_unsqueeze", "nfdpm_copy_channels")),
              ("prior", ("nfdpm_split_prior", "nfdpm_gauss", "nfdpm_accumulate")),
              ("prepare", ("nfdpm_mix_prepare", "nfdpm_pack", "nfdpm_channel_stats", "nfdpm_rows_to_nchw", "nfdpm_nchw_to_rows")),
-             ("backward", ("nfdpm_coupling_bwd", "nfdpm_mix_bwd", "nfdpm_mix_param_grad", "nfdpm_actnorm_relu_bwd", "nfdpm_reduce_rows",
+             ("backward", ("nfdpm_coupling_bwd", "nfdpm_coupling_inv_bwd", "nfdpm_mix_bwd", "nfdpm_mix_param_grad",
+                           "nfdpm_mix_inv_param_grad", "nfdpm_split_sample_bwd", "nfdpm_flow_boundary_inv_stash",
+                           "nfdpm_actnorm_relu_bwd", "nfdpm_reduce_rows",
                            "nfdpm_col2im_add")),
              ("optimizer", ("nfdpm_fused_clip_adam",)),
              ("formats", ("nfdpm_latent_format", "nfdpm_postprocess_u8", "nfdpm_preprocess")))
 
 
 def _family(name: str) -> str:
+    """The family of the longest listed prefix of ``name``."""
+    best, fam_best = 0, "misc"
     for fam, prefixes in _FAMILIES:
-        if any(name.startswith(p) for p in prefixes):
-            return fam
-    return "misc"
+        for p in prefixes:
+            if name.startswith(p) and len(p) > best:
+                best, fam_best = len(p), fam
+    return fam_best
 
 
 class _RangedLib:
@@ -173,7 +184,8 @@ EXPORTS = ["nfdpm_version", "nfdpm_last_error_string", "nfdpm_sm_count", "nfdpm_
            "nfdpm_opt_chunk", "nfdpm_fused_clip_adam", "nfdpm_pack_elems", "nfdpm_pack_batch",
            "nfdpm_gemm3_boundary_ok", "nfdpm_gemm3_boundary", "nfdpm_coupling_bwd_tiles", "nfdpm_mix_bwd_tiles", "nfdpm_gemm_debug", "nfdpm_flow_boundary_debug",
            "nfdpm_latent_format", "nfdpm_postprocess_u8", "nfdpm_preprocess",
-           "nfdpm_flow_boundary_tiles", "nfdpm_flow_boundary_tiled"]
+           "nfdpm_flow_boundary_tiles", "nfdpm_flow_boundary_tiled",
+           "nfdpm_coupling_inv_bwd", "nfdpm_mix_inv_param_grad", "nfdpm_split_sample_bwd", "nfdpm_flow_boundary_inv_stash"]
 
 #: number of kernels launched through this binding (bench.py reports it as ``gpu_launches``)
 launch_count = 0
@@ -327,11 +339,26 @@ def coupling_bwd(dy, dy_bs, dld, u, u_bs, pm, ldp, bias3, logs3, du, du_bs, dpm,
                                H, W, _st()), 1 if dp_scratch is None else 2)
 
 
+def coupling_inv_bwd(dx, dx_bs, y, y_bs, pm, ldp, bias3, logs3, dy, dy_bs, dpm, ld_dpm, dpar, B, Cc, H, W, dbias=None,
+                     dlogs=None, dp_scratch=None) -> None:
+    """Backward of the inverse coupling; reductions and tiling as in ``coupling_bwd``."""
+    cnt = _tn_counters(dx.device)[1023:] if dbias is not None else None
+    _ok(lib.nfdpm_coupling_inv_bwd(_p(dx), dx_bs, _p(y), y_bs, _p(pm), ldp, _p(bias3), _p(logs3), _p(dy), dy_bs, _p(dpm),
+                                   _dt(dpm), ld_dpm, _p(dpar), _p(dbias), _p(dlogs), _p(cnt), _p(dp_scratch), B, Cc, H, W,
+                                   _st()), 1 if dp_scratch is None else 2)
+
+
 def flow_boundary_stash(src, src_bs, squeeze_in, pm, ldp, bias3, logs3, ld_part, mt, beta, y, y_bs, xs, xs_bs, a1, lda1,
                         B, Cc, H, W) -> None:
     _ok(lib.nfdpm_flow_boundary_stash(_p(src), src_bs, int(squeeze_in), _p(pm), ldp, _p(bias3), _p(logs3), _p(ld_part),
                                       _p(mt), _p(beta), _p(y), y_bs, _p(xs), xs_bs, _p(a1),
                                       _dt(a1) if a1 is not None else F32, lda1, B, Cc, H, W, _st()))
+
+
+def flow_boundary_inv_stash(src, src_bs, pm, ldp, bias3, logs3, mt, beta, y, y_bs, xs, xs_bs, a1, lda1, B, Cc, H, W) -> None:
+    _ok(lib.nfdpm_flow_boundary_inv_stash(_p(src), src_bs, _p(pm), ldp, _p(bias3), _p(logs3), _p(mt), _p(beta), _p(y), y_bs,
+                                          _p(xs), xs_bs, _p(a1), _dt(a1) if a1 is not None else F32, lda1, B, Cc, H, W,
+                                          _st()))
 
 
 def actnorm_relu_bwd(dh, ld_dh, h, ld_h, scale, dpre, ld_o, part, M, Nn, rows_per_cta) -> None:
@@ -354,6 +381,11 @@ def mix_bwd(du, du_bs, da1, lda1, x, x_bs, mt, dx, dx_bs, part, B, Cc, H, W) -> 
 def mix_param_grad(items) -> None:
     arr = (MixGradItem * len(items))(*items)
     _ok(lib.nfdpm_mix_param_grad(arr, len(items), _st()), (len(items) + 15) // 16)
+
+
+def mix_inv_param_grad(items) -> None:
+    arr = (MixGradItem * len(items))(*items)
+    _ok(lib.nfdpm_mix_inv_param_grad(arr, len(items), _st()), (len(items) + 15) // 16)
 
 
 def gemm_tn_workspace(M, N1, N2) -> int:
@@ -388,6 +420,11 @@ def split_prior_bwd(dlp, h, ldh, bias, logs, x, xbs, dstate, dbs, dh, dpar, B, C
 
 def gauss_const_bwd(dl, z, bias, logs, dz, dpar, B, Cc, P) -> None:
     _ok(lib.nfdpm_gauss_const_bwd(_p(dl), _p(z), _p(bias), _p(logs), _p(dz), _p(dpar), B, Cc, P, _st()))
+
+
+def split_sample_bwd(dz, dz_bs, eps, temperature, h, ldh, bias, logs, dh, dpar, B, Cc, H, W) -> None:
+    _ok(lib.nfdpm_split_sample_bwd(_p(dz), dz_bs, _p(eps), float(temperature), _p(h), ldh, _p(bias), _p(logs), _p(dh),
+                                   _p(dpar), B, Cc, H, W, _st()))
 
 
 def col2im_add(da, lda, dstate, dbs, B, Cin, H, W) -> None:

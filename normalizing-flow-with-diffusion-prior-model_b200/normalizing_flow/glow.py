@@ -92,6 +92,10 @@ class StepFlow(Transform):
             N.accumulate(log_det_jac, part, T, B, self._mix.logdet, E.scalar_f32(x.device, H * W), 1)
         return y, log_det_jac, logp
 
+    def _invert_composed(self, y: Tensor) -> Tensor:
+        """Under autograd (NFDPM_INVERT_GRAD=1) the inverse is the composition of the three parts' inverses."""
+        return self.actnorm.invert(self.invconv2d.invert(self.affcoupling.invert(y)))
+
     @_granular("StepFlow")
     def invert(self, y: Tensor) -> Tensor:
         y = E.check_input(y)
@@ -468,17 +472,20 @@ class Glow(Transform):
     # ---- inverse: latents -> x
     def invert(self, latents: list, temperature: float = 1.0) -> Tensor:
         z_last = E.check_input(latents[-1], "latents[-1]")
+        B, Cf, h, w = z_last.shape
+        if Cf != 2 ** (self.L + 1) * self.in_channel:
+            raise ValueError(f"final latent has {Cf} channels, expected {2 ** (self.L + 1) * self.in_channel}")
         if E.autograd_needed(z_last, self) or any(isinstance(t, Tensor) and t.requires_grad for t in latents):
-            # the inverse has no backward kernels: compute it without recording and fail loudly on back-propagation
+            if E.invert_grad_enabled():
+                from ._invgrad import glow_invert
+                return glow_invert(self, latents, temperature)
+            # without NFDPM_INVERT_GRAD: compute it without recording and fail loudly on back-propagation
             from .transforms import _NoBackward
             deps = [t for t in latents if isinstance(t, Tensor) and t.requires_grad] + \
                    [p for p in self.parameters() if p.requires_grad]
             with torch.no_grad():
                 out = self.invert([t.detach() if isinstance(t, Tensor) else t for t in latents], temperature)
             return _NoBackward.apply(out, "Glow.invert", False, *deps)
-        B, Cf, h, w = z_last.shape
-        if Cf != 2 ** (self.L + 1) * self.in_channel:
-            raise ValueError(f"final latent has {Cf} channels, expected {2 ** (self.L + 1) * self.in_channel}")
         dev = z_last.device
         levels = self._levels()
         slots = self._slots(dev)

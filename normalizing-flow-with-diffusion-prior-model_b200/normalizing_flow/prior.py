@@ -50,6 +50,9 @@ class IsotropicGaussian(Prior):
 
     def sample(self, shape: tuple = None, temperature: float = 1.0) -> Tensor:
         mean, logsd = E.check_input(self.mean, "mean"), E.check_input(self.logsd, "logsd")
+        if E.invert_grad_enabled() and torch.is_grad_enabled() and (mean.requires_grad or logsd.requires_grad):
+            from ._invgrad import IsotropicSampleFn
+            return IsotropicSampleFn.apply(float(temperature), mean, logsd)
         B = mean.shape[0]
         n = mean[0].numel()
         eps = torch.empty_like(mean).normal_()
@@ -99,8 +102,11 @@ class GaussianPrior(Prior):
         if C != self._C:
             raise ValueError(f"GaussianPrior built for {self._C} channels got {C}")
         dev = self.__conv.bias.device if self.__conv is not None else self.device
-        eps = torch.empty(B, C, H, W, dtype=torch.float32, device=dev).normal_()
         bias, logs = self._params()
+        if E.invert_grad_enabled() and bias is not None and E.autograd_needed(bias, self):
+            from ._invgrad import GaussianSampleFn
+            return GaussianSampleFn.apply((B, C, H, W), float(temperature), bias, logs)
+        eps = torch.empty(B, C, H, W, dtype=torch.float32, device=dev).normal_()
         out = torch.empty_like(eps)
         N.gauss_sample_const(eps, bias, logs, temperature, out, B, C, H * W)
         return out

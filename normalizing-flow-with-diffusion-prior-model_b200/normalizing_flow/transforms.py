@@ -20,7 +20,7 @@ from .utils import ZeroConv2d, coupling_network
 class _NoBackward(torch.autograd.Function):
     """Identity whose backward raises.  ``transform`` of the granular modules (ActNorm, InvConv2d, AffineCoupling, Squeeze,
     Split — and StepFlow / GlowBlock, which compose them) is differentiable through normalizing_flow/_modgrad.py; ``invert``
-    has no backward kernels (the reference inverts only under ``torch.no_grad()``: sampling and decoding), so its forward
+    is differentiable only with NFDPM_INVERT_GRAD=1 (the reference inverts under ``torch.no_grad()``: sampling and decoding); without it its forward
     runs in any grad mode — the reference's own unit tests call it with autograd enabled (tests/transformations.py) —
     and back-propagating through it fails loudly instead of silently dropping gradients."""
 
@@ -48,10 +48,13 @@ def _no_autograd(x: Tensor, mod: nn.Module, what: str) -> None:
 def _granular(what: str):
     """Decorator for stand-alone transform / invert methods.  Without autograd: the kernels, nothing recorded.  Under
     autograd ``transform`` goes through the module's autograd Function (normalizing_flow/_modgrad.py; StepFlow composes its
-    three parts); ``invert`` runs the kernels without recording and attaches the loud-failure node to its result."""
+    three parts); ``invert`` does the same with ``NFDPM_INVERT_GRAD=1`` and otherwise runs the kernels without recording
+    and attaches the loud-failure node to its result."""
     def deco(fn):
         def wrapper(self, x, *args, **kw):
-            if not E.autograd_needed(x, self):
+            latent_grad = fn.__name__ == "invert" and E.invert_grad_enabled() and torch.is_grad_enabled() and \
+                any(isinstance(t, Tensor) and t.requires_grad for t in tuple(args) + tuple(kw.values()))
+            if not E.autograd_needed(x, self) and not latent_grad:
                 return fn(self, x, *args, **kw)
             if fn.__name__ == "transform":
                 from . import _modgrad as MG
@@ -61,6 +64,15 @@ def _granular(what: str):
                     return self._transform_composed(x, ld, lp)
                 if what in MG.SUPPORTED:
                     return MG.transform(self, what, fn, E.check_input(x), ld, lp)
+            elif E.invert_grad_enabled():
+                from . import _modgrad as MG
+                if what == "StepFlow":
+                    return self._invert_composed(x)
+                if what == "Split":
+                    latent = args[0] if len(args) > 0 else kw.get("inv_y_split")
+                    temperature = args[1] if len(args) > 1 else kw.get("temperature", 1.0)
+                    return MG.invert(self, what, fn, x, latent, temperature)
+                return MG.invert(self, what, fn, x)
             ins = [t for t in (x,) + tuple(args) + tuple(kw.values()) if isinstance(t, Tensor)]
             deps = [t for t in ins if t.requires_grad] + [p for p in self.parameters() if p.requires_grad]
             with torch.no_grad():
@@ -325,9 +337,10 @@ class Split(Transform):
         return out
 
     def _fill_second_half(self, out: Tensor, obs: int, B: int, C: int, H: int, W: int, z: Optional[Tensor],
-                          temperature: float) -> None:
+                          temperature: float, eps_sink: Optional[list] = None) -> None:
         """Write the latent (given, or drawn from the conditional prior, reference transforms.py:305-307 and
-        prior.py:49-50) into channels C/2..C of ``out`` whose first half is already in place."""
+        prior.py:49-50) into channels C/2..C of ``out`` whose first half is already in place.  ``eps_sink`` receives the
+        standard-normal tensor a draw used (the inverse's backward needs it)."""
         Ch, P = C // 2, H * W
         second = out.view(-1)[Ch * P:]
         if z is not None:
@@ -337,6 +350,8 @@ class Split(Transform):
             N.copy_channels(z, second, B, Ch, P, Ch * P, obs)
             return
         eps = torch.empty(B, Ch, H, W, dtype=torch.float32, device=out.device).normal_()
+        if eps_sink is not None:
+            eps_sink.append(eps)
         h, ldh = E.split_rows(self, out, obs, B, C, H, W)
         bias = self.conv.bias if self.conv is not None else None
         logs = self.conv.logs if self.conv is not None else None
