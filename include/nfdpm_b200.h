@@ -144,9 +144,10 @@ int nfdpm_gemm_nt(const void* A, int64_t lda, const void* Bw, int64_t ldb, void*
  *   pm   [M, ldp]: taps-as-N output of the ZeroConv GEMM (column = tap*C + co, tap = ky*3+kx)
  *   net[co] = (sum_tap pm[m + (ky-1)*W + (kx-1), tap*C+co] (zero outside the image) + bias3[co]) * exp(3*logs3[co])
  *   log_s = net[0:C/2], t = net[C/2:C], s = sigmoid(log_s + 2)
- *   forward: y_b = (x_b + t)*s, ld_part += sum log(s + 1e-6);   inverse: y_b = x_b/(s + 1e-6) - t
+ *   forward: y_b = (x_b + t)*s;   inverse: y_b = x_b/(s + 1e-6) - t;   both: ld_part = sum log(s + 1e-6)
  * x,y [B,C,P] NCHW (batch strides); the first C/2 channels are copied through when y != x.
- * ld_part (forward only, may be NULL): fp32 [T][B] partial sums, T = nfdpm_ld_tiles(P); entry t*B+b. */
+ * ld_part (either direction, may be NULL): fp32 [T][B] partial sums, T = nfdpm_ld_tiles(P); entry t*B+b.  The inverse's
+ * partial equals the forward's bit for bit for the same pm: it is -log|det| of the inverse at its output. */
 int nfdpm_ld_tiles(int P);
 int nfdpm_coupling_apply(const float* pm, int64_t ldp, const float* bias3, const float* logs3, const float* x,
                          float* y, float* ld_part, int B, int C, int H, int W, int64_t x_bstride,
@@ -179,7 +180,8 @@ int nfdpm_gauss_sample_const(const float* eps, const float* bias, const float* l
  * Equivalent to nfdpm_coupling_apply + nfdpm_channel_mix + nfdpm_im2col3x3 (+ nfdpm_squeeze when squeeze_in) in ONE
  * launch with coalesced traffic; replaces the same reference lines (transforms.py:80,132,144,93,179-184,196-200,226).
  *   in  [B,C,P] (batch stride in_bs) or, with squeeze_in, [B,C/4,2H,2W];  pm == NULL: no coupling;
- *   mt == NULL: no mix;  y == NULL / a1 == NULL: sink disabled;  ld_part [B] (forward coupling only, may be NULL);
+ *   mt == NULL: no mix;  y == NULL / a1 == NULL: sink disabled;  ld_part [B] (coupling in either direction, may be
+ *   NULL: the sum of log(s + 1e-6), as in nfdpm_coupling_apply);
  *   a1: rows [B*P, lda1] of dtype a1_dtype (F32/BF16), column = c*9 + ky*3 + kx over the first C/2 channels. */
 size_t nfdpm_flow_boundary_smem(int C, int H, int W, int coupling, int mix);
 int nfdpm_flow_boundary(const float* in, int64_t in_bs, int squeeze_in, const float* pm, int64_t ldp,
@@ -206,7 +208,8 @@ int nfdpm_flow_boundary_inv_stash(const float* in, int64_t in_bs, const float* p
  * taps-as-N rows never reach L2/HBM.  Same reference lines as nfdpm_gemm_nt (utils.py:44) + nfdpm_flow_boundary.
  * h2, w3p: h_dtype = NFDPM_BF16 or NFDPM_BF16X2 (K, ldh count logical columns); CTAs own whole images: needs H*W == 256 or
  * H*W dividing 128, ldp <= 512 (nfdpm_gemm3_boundary_ok, whose K counts bf16 columns: 2 x logical K for split pairs).
- * pm_out (optional, fp32 [M, ld_pm_out]): copy of pm for the training stash; xs: pre-mix stash as in ..._stash. */
+ * pm_out (optional, fp32 [M, ld_pm_out]): copy of pm for the training stash; xs: pre-mix stash as in ..._stash;
+ * ld_part [B] in either direction, as in nfdpm_flow_boundary. */
 int nfdpm_gemm3_boundary_ok(int B, int C, int H, int W, int K, int64_t ldp);
 int nfdpm_gemm3_boundary(const void* h2, int h_dtype, int64_t ldh, const void* w3p, float* pm_out, int64_t ld_pm_out, const float* in,
                          int64_t in_bs, const float* bias3, const float* logs3, float* ld_part, const float* mt,
@@ -341,8 +344,8 @@ int nfdpm_accumulate(void* acc, int acc_dtype, const float* part, int R, int B, 
  * band of image rows (plus one recomputed halo row above and below when there is an im2col sink), so images of any size
  * take the fused boundary and small batches spread over B * tiles CTAs.  `in` and `y` / `xs` must NOT alias (a band reads
  * halo rows another band writes).  nfdpm_flow_boundary_tiles() returns the number of bands per image for a shape and
- * sink combination (0: one row does not fit in shared memory); the forward log-det is written as `tiles` partial rows:
- * ld_part[t * B + b].  Replaces, like nfdpm_flow_boundary: transforms.py:179-184 / :196-200 (coupling), :80 + :132 /
+ * sink combination (0: one row does not fit in shared memory); the log-det (either direction) is written as `tiles`
+ * partial rows: ld_part[t * B + b].  Replaces, like nfdpm_flow_boundary: transforms.py:179-184 / :196-200 (coupling), :80 + :132 /
  * :144 + :93 (ActNorm + 1x1 conv), :226 (squeeze) and the im2col of utils.py:64's 3x3 conv. */
 int nfdpm_flow_boundary_tiles(int B, int C, int H, int W, int coupling, int mix, int want_a1);
 int nfdpm_flow_boundary_tiled(const float* in, int64_t in_bs, int squeeze_in, const float* pm, int64_t ldp,

@@ -10,7 +10,7 @@ struct BoundaryArgs {
   const float* in; int64_t in_bs;       // source state [B,C,P] (or [B,C/4,2H,2W] when squeeze_in)
   const float* pm; int64_t ldp;         // SRC_COUPLING: taps-as-N rows [B*P, ldp]
   const float* bias3; const float* logs3;
-  float* ld_part;                       // forward coupling: [B] per-image log-det partial (may be null)
+  float* ld_part;                       // coupling, either direction: [B] per-image sum of log(s + 1e-6) (may be null)
   const float* mt; const float* beta;   // mix (null = identity)
   float* y; int64_t y_bs;               // NCHW sink (may be null)
   float* xs; int64_t xs_bs;             // NCHW sink of the PRE-mix state (training stash of the next step's input; may be null)
@@ -243,6 +243,8 @@ __device__ __forceinline__ void flow_boundary_body(const BoundaryArgs& a, const 
       const float xb = x_s[(Ch + j) * PS + p];
       if (a.inverse) {
         x_s[(Ch + j) * PS + p] = xb / (s + 1e-6f) - sh_t;
+        // the forward's term: the same s (from the same pass-through half) that the inverse divides by
+        if (a.ld_part != nullptr) ls_s[it] = logf(s + 1e-6f);
       } else {
         x_s[(Ch + j) * PS + p] = (xb + sh_t) * s;
         ls_s[it] = logf(s + 1e-6f);
@@ -250,7 +252,7 @@ __device__ __forceinline__ void flow_boundary_body(const BoundaryArgs& a, const 
     }
     __syncthreads();
     stamp(2);
-    if (!a.inverse && a.ld_part != nullptr && tid < 32) {
+    if (a.ld_part != nullptr && tid < 32) {
       // deterministic per-image sum: fixed lane-strided order + shuffle tree
       float acc = 0.f;
 #pragma unroll 8

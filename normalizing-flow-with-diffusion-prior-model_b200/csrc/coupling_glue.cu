@@ -146,7 +146,8 @@ static int pix_grid(int B, int P) {
 }
 
 // Affine coupling epilogue.  One thread per pixel; loops over the C/2 transformed channels two at a time
-// (8-byte loads of the taps-as-N rows).  INVERSE selects x_b = y_b/(s+1e-6) - t.
+// (8-byte loads of the taps-as-N rows).  INVERSE selects x_b = y_b/(s+1e-6) - t.  In either direction a non-null ld_part
+// receives the per-image sum of log(s + 1e-6): the inverse divides by exactly the s the forward multiplies by.
 template <bool INVERSE, int VEC>
 __global__ void __launch_bounds__(TPB) coupling_apply_kernel(const float* __restrict__ pm, int64_t ldp,
                                                              const float* __restrict__ bias3,
@@ -215,6 +216,7 @@ __global__ void __launch_bounds__(TPB) coupling_apply_kernel(const float* __rest
         const float xv = xb[(int64_t)(Ch + jj) * P];
         if (INVERSE) {
           yb[(int64_t)(Ch + jj) * P] = xv / (s + 1e-6f) - sh_t;
+          if (ld_part != nullptr) ld_acc += logf(s + 1e-6f);
         } else {
           yb[(int64_t)(Ch + jj) * P] = (xv + sh_t) * s;
           ld_acc += logf(s + 1e-6f);
@@ -222,7 +224,7 @@ __global__ void __launch_bounds__(TPB) coupling_apply_kernel(const float* __rest
       }
     }
   }
-  if (!INVERSE && ld_part != nullptr) {
+  if (ld_part != nullptr) {
     tile_image_reduce<TPB>(ld_acc, sh, tile.first_m, tile.n_valid, P,
                            [&](int64_t b, int ti, float s) { ld_part[(int64_t)ti * B + b] = s; });
   }

@@ -7,7 +7,8 @@
 // below (coupling + mix of the halo pixels; their pm rows are in L2): no inter-CTA exchange, at (R + 2) / R of the elementwise
 // arithmetic.  The band is addressed as Rv = R + 2*halo "virtual" rows starting at image row r0 - halo; rows outside the image
 // are skipped, so every index division is by a launch constant (multiply-high, common.cuh).
-// The per-image log-det is written as one partial per band: ld_part[t * B + b] (nfdpm_accumulate sums the rows in order).
+// The per-image log-det is written as one partial per band: ld_part[t * B + b] (nfdpm_accumulate sums the rows in order);
+// the inverse writes the same partial, from the s it divides by.
 #include "boundary_body.cuh"
 #include <stdlib.h>
 
@@ -152,13 +153,14 @@ __global__ void __launch_bounds__(1024) flow_boundary_tiled_kernel(const Boundar
       const float xb = x_s[(Ch + j) * PS + q];
       if (a.inverse) {
         x_s[(Ch + j) * PS + q] = xb / (s + 1e-6f) - sh_t;
+        if (a.ld_part != nullptr && v >= halo && v < halo + R) ls_s[(q - halo * W) * Ch + j] = logf(s + 1e-6f);
       } else {
         x_s[(Ch + j) * PS + q] = (xb + sh_t) * s;
         if (v >= halo && v < halo + R) ls_s[(q - halo * W) * Ch + j] = logf(s + 1e-6f);
       }
     }
     __syncthreads();
-    if (!a.inverse && a.ld_part != nullptr && tid < 32) {
+    if (a.ld_part != nullptr && tid < 32) {
       const int n_own = (min(H, r0 + R) - r0) * W * Ch;            // own rows are contiguous from r0: entries [0, n_own) are set
       float acc = 0.f;
 #pragma unroll 8

@@ -23,7 +23,7 @@ struct G3Args {
   float* pm_out; int64_t ld_pm_out;      // optional copy of pm for the training stash (may be null)
   const float* in; int64_t in_bs;        // flow state entering the coupling [B,C,P]
   const float* bias3; const float* logs3;
-  float* ld_part;                        // [B] (forward, may be null)
+  float* ld_part;                        // [B] per-image sum of log(s + 1e-6), either direction (may be null)
   const float* mt; const float* beta;    // next mix (null = none)
   float* y; int64_t y_bs;                // NCHW sink (may be null)
   float* xs; int64_t xs_bs;              // pre-mix stash sink (may be null)
@@ -230,6 +230,7 @@ __global__ void __launch_bounds__(G3_THREADS, 1) gemm3_boundary_kernel(const __g
         float* xb = x_s + ((im_lo + im) * C + Ch + j) * PS + p;
         if (a.inverse) {
           *xb = *xb / (s + 1e-6f) - sh_t;
+          if (a.ld_part != nullptr) ls_s[it] = logf(s + 1e-6f);
         } else {
           *xb = (*xb + sh_t) * s;
           ls_s[it] = logf(s + 1e-6f);
@@ -237,7 +238,7 @@ __global__ void __launch_bounds__(G3_THREADS, 1) gemm3_boundary_kernel(const __g
       }
     }
     __syncthreads();
-    if (!a.inverse && a.ld_part != nullptr && warp < im_n) {
+    if (a.ld_part != nullptr && warp < im_n) {
       // deterministic per-image sum: one warp per image, fixed lane-strided order + shuffle tree
       float acc = 0.f;
       const float* l = ls_s + warp * P * Ch;

@@ -5,7 +5,7 @@ normalizing_flow/__init__.py:8-13, :109-111): the transforms, StepFlow / GlowBlo
 and the step glue.  The trainers, data loaders, metrics and logging helpers of the reference are outside the hot
 path; INTEGRATION.md shows how the reference tree picks this package up.
 """
-from typing import Tuple
+from typing import Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -51,12 +51,15 @@ class NFBackbone(nn.Module):
         parts, log_det_jac, _ = self.model.transform(x, log_det_jac, None)
         return parts, log_det_jac
 
-    def invert(self, latents: list) -> Tensor:
-        return self.model.invert(latents)
+    def invert(self, latents: list, log_det_jac: Optional[Tensor] = None) -> Tensor:
+        """Glow.invert; ``log_det_jac`` (optional) receives the flow's log|det dz/dx| at the returned x, as ``transform``
+        would add it (the Split priors are not evaluated, as in ``transform``)."""
+        return self.model.invert(latents, log_det_jac=log_det_jac)
 
     @torch.no_grad()
-    def sample(self, latents: list, postprocess_func=None) -> Tensor:
-        return self.model.sample(latents, postprocess_func)
+    def sample(self, latents: list, postprocess_func=None, log_det_jac: Optional[Tensor] = None) -> Tensor:
+        """Glow.sample; ``log_det_jac`` as in ``invert``, at the sample before ``postprocess_func``."""
+        return self.model.sample(latents, postprocess_func, log_det_jac=log_det_jac)
 
 
 __all__ = ["InvConv2d", "ActNorm", "AffineCoupling", "StepFlow", "Squeeze", "Split", "GlowBlock", "Glow",

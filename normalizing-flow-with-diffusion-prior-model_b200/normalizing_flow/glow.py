@@ -63,11 +63,12 @@ class StepFlow(Transform):
         self.affcoupling._run(y, ybs, y, ybs, B, C, H, W, False, ld_part)
 
     def _inverse_views(self, y: Tensor, ybs: int, t: Tensor, tbs: int, x: Tensor, xbs: int, B: int, H: int,
-                       W: int) -> None:
-        """y --coupling^-1--> t (t may be y: in place) --K-A^-1--> x."""
+                       W: int, ld_part: Optional[Tensor] = None) -> None:
+        """y --coupling^-1--> t (t may be y: in place) --K-A^-1--> x.  ``ld_part``: the coupling's log-det partials at x,
+        the rows the forward writes."""
         C, P = self._C, H * W
         E.prepare_mix([self._mix_entry(None)])
-        self.affcoupling._run(y, ybs, t, tbs, B, C, H, W, True, None)
+        self.affcoupling._run(y, ybs, t, tbs, B, C, H, W, True, ld_part)
         N.channel_mix(t, x, self._mix.inv_mt, self._mix.inv_beta, B, C, P, tbs, xbs)
 
     def _transform_composed(self, x: Tensor, log_det_jac: Tensor, logp: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
@@ -470,13 +471,34 @@ class Glow(Transform):
         return latents, ld_part, R_ld, lp_part, R_lp
 
     # ---- inverse: latents -> x
-    def invert(self, latents: list, temperature: float = 1.0) -> Tensor:
+    def invert(self, latents: list, temperature: float = 1.0, log_det_jac: Optional[Tensor] = None,
+               logp: Optional[Tensor] = None) -> Tensor:
+        """latents -> x.  ``latents`` holds all L parts (decoding) or the last ones only: every Split without a latent draws
+        its half from its conditional prior at ``temperature``.
+
+        ``log_det_jac`` / ``logp`` (optional [B] fp32/fp64 CUDA vectors, ``+=`` in place, ``None`` = not requested) receive
+        exactly the terms ``transform(x, log_det_jac, logp)`` would add at the returned x, without a second pass:
+          log_det_jac += sum over steps of P*sum(actnorm scale) + P*log|det W| + sum log(s + 1e-6), which is
+                         -log|det dx/dz| of this inverse (it divides by exactly s + 1e-6);
+          logp        += sum over the L-1 Split halves of log N(z_l; mean_l, exp(logs_l)), supplied or drawn; the final
+                         latent's prior is not included, as in ``transform``.
+        Under a temperature this is the model's density at the returned sample, not the tempered one.  The accumulated
+        density is not differentiable: a call that NFDPM_INVERT_GRAD=1 would record raises NotImplementedError."""
         z_last = E.check_input(latents[-1], "latents[-1]")
         B, Cf, h, w = z_last.shape
         if Cf != 2 ** (self.L + 1) * self.in_channel:
             raise ValueError(f"final latent has {Cf} channels, expected {2 ** (self.L + 1) * self.in_channel}")
+        E.check_acc(log_det_jac, B, "log_det_jac")
+        E.check_acc(logp, B, "logp")
+        accs = [a for a in (log_det_jac, logp) if a is not None]
+        if torch.is_grad_enabled() and any(a.requires_grad for a in accs):
+            raise RuntimeError("log_det_jac / logp are updated in place and must not require grad on entry")
         if E.autograd_needed(z_last, self) or any(isinstance(t, Tensor) and t.requires_grad for t in latents):
             if E.invert_grad_enabled():
+                if accs:
+                    raise NotImplementedError(
+                        "Glow.invert: the accumulated log_det_jac / logp are not differentiable; a recorded invert "
+                        "(NFDPM_INVERT_GRAD=1) takes no accumulators.  Call it under torch.no_grad() for the density.")
                 from ._invgrad import glow_invert
                 return glow_invert(self, latents, temperature)
             # without NFDPM_INVERT_GRAD: compute it without recording and fail loudly on back-propagation
@@ -484,13 +506,16 @@ class Glow(Transform):
             deps = [t for t in latents if isinstance(t, Tensor) and t.requires_grad] + \
                    [p for p in self.parameters() if p.requires_grad]
             with torch.no_grad():
-                out = self.invert([t.detach() if isinstance(t, Tensor) else t for t in latents], temperature)
+                out = self.invert([t.detach() if isinstance(t, Tensor) else t for t in latents], temperature,
+                                  log_det_jac, logp)
             return _NoBackward.apply(out, "Glow.invert", False, *deps)
+        with_ld, with_lp = log_det_jac is not None, logp is not None
         dev = z_last.device
         levels = self._levels()
         slots = self._slots(dev)
         steps = [s for flows, _ in levels for s in flows]
         ready = all(s._ready() for s in steps)
+        H, W = h << self.L, w << self.L
         if self._use_graph(ready) and 1 <= len(latents) <= self.L and all(isinstance(t, Tensor) for t in latents):
             # decoding (all L latents supplied) and sampling (fewer: every Split without a latent draws its half from the
             # learned conditional prior, transforms.py:305-307) replay one captured chain; the normal draws inside a
@@ -498,13 +523,17 @@ class Glow(Transform):
             lat_in = [E.check_input(t, "latent") for t in latents]
             if self._params_changed():
                 self._refresh_caches(steps, slots)
-            key = ("inv", B, h, w, E.precision(), dev.index) if len(latents) == self.L else \
-                  ("inv", B, h, w, E.precision(), dev.index, len(latents), float(temperature))
+            sampling = len(latents) < self.L
+            key = ("inv", B, h, w, E.precision(), dev.index)
+            if sampling:
+                key += (len(latents), float(temperature))
+            if with_ld or with_lp:                    # a chain that also writes the density partials
+                key += ((with_ld, with_lp),)
             ent = self._graphs.get(key)
-            if ent is None and len(key) > 6:
+            if ent is None and sampling:
                 # the temperature is baked into a sampling graph: keep at most four of them (a temperature sweep would
                 # otherwise pin one captured chain and its workspace per value)
-                old = [k for k in self._graphs if k[0] == "inv" and len(k) > 6]
+                old = [k for k in self._graphs if k[0] == "inv" and len(k) >= 8]
                 for k in old[:max(0, len(old) - 3)]:
                     E.WS.drop_scope(("glow", id(self), k))
                     del self._graphs[k]
@@ -519,7 +548,7 @@ class Glow(Transform):
 
             def build():
                 outs = self._fork_join(nsub, lambda i: self._invert_core(
-                    [t[i * Bs:(i + 1) * Bs] for t in statics], temperature, levels, slots, steps, True))
+                    [t[i * Bs:(i + 1) * Bs] for t in statics], temperature, levels, slots, steps, True, with_ld, with_lp))
                 return {"lat": statics, "outs": outs}
             ent = self._graph_entry(key, build)
             if ent["lat"] is not statics:
@@ -527,27 +556,52 @@ class Glow(Transform):
                     s_.copy_(t)
             ent["graph"].replay()
             N.launch_count += ent["n_launch"]
-            return torch.cat(ent["outs"]) if nsub > 1 else ent["outs"][0].clone()
-        return self._invert_core(latents, temperature, levels, slots, steps, ready)
+            outs = ent["outs"]
+            for i, (_, ld_part, R_ld, lp_part, R_lp) in enumerate(outs):     # after the replay, into the caller's tensors
+                sl = slice(i * Bs, (i + 1) * Bs)
+                self._add_density(log_det_jac[sl] if with_ld else None, logp[sl] if with_lp else None, ld_part, R_ld,
+                                  lp_part, R_lp, Bs, H, W, slots)
+            return torch.cat([o[0] for o in outs]) if nsub > 1 else outs[0][0].clone()
+        x, ld_part, R_ld, lp_part, R_lp = self._invert_core(latents, temperature, levels, slots, steps, ready, with_ld,
+                                                            with_lp)
+        self._add_density(log_det_jac, logp, ld_part, R_ld, lp_part, R_lp, B, H, W, slots)
+        return x
+
+    def _add_density(self, log_det_jac, logp, ld_part, R_ld: int, lp_part, R_lp: int, B: int, H: int, W: int,
+                     slots: Tensor) -> None:
+        """The final accumulates of an inverse, as ``transform`` runs them: the log-det partial rows plus the L*K
+        data-independent constants, and the Split log-prob rows."""
+        if log_det_jac is not None:
+            N.accumulate(log_det_jac, ld_part, R_ld, B, slots, self._multipliers(H, W, slots.device), self.L * self.K)
+        if logp is not None and R_lp > 0:
+            N.accumulate(logp, lp_part, R_lp, B)
+
+    def _part_rows(self, B: int, H: int, W: int, inverse: bool = False, fused: bool = True) -> Tuple[int, int]:
+        """Rows of B per-image partials that one call writes for [B, c, H, W] images: (log-det rows, Split log-prob rows).
+        Log-det: one per step at "image" levels, ld_tiles(P) per step at unfused ones, one per band at "tiled" levels, where
+        K-1 boundaries carry an im2col sink and the level's last one does not (and has a mix in the inverse only, which can
+        change the band height).  ``fused=False``: every level unfused (NFDPM_FUSED_BOUNDARY=0, or a model not ready)."""
+        R_ld = R_lp = 0
+        hh, ww, cc = H, W, self.in_channel
+        for li in range(self.L):
+            hh, ww, CC = hh // 2, ww // 2, cc * 4
+            mode = self._level_mode(B, CC, hh, ww) if fused else "unfused"
+            if mode == "tiled":
+                R_ld += (self.K - 1) * N.flow_boundary_tiles(B, CC, hh, ww, 1, 1, 1) + \
+                    N.flow_boundary_tiles(B, CC, hh, ww, 1, int(inverse), 0)
+            else:
+                R_ld += self.K * (1 if mode == "image" else N.ld_tiles(hh * ww))
+            if li < self.L - 1:
+                R_lp += N.ld_tiles(hh * ww)
+            cc = CC // 2
+        return R_ld, R_lp
 
     def _transform_fast(self, x: Tensor, with_logp: bool, levels, slots, steps):
         """Forward with the fused step-boundary kernel: 4 launches per StepFlow (boundary + 3 GEMMs)."""
         B, c, H, W = x.shape
         dev = x.device
         E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
-        # partial-sum rows: one per step at fused levels, ld_tiles(P) per step at unfused ones
-        R_ld = R_lp = 0
-        hh, ww, cc = H, W, c
-        for li in range(self.L):
-            hh, ww, CC = hh // 2, ww // 2, cc * 4
-            mode = self._level_mode(B, CC, hh, ww)
-            if mode == "tiled":     # K-1 boundaries with an im2col sink and the level's last one without
-                R_ld += (self.K - 1) * N.flow_boundary_tiles(B, CC, hh, ww, 1, 1, 1) + N.flow_boundary_tiles(B, CC, hh, ww, 1, 0, 0)
-            else:
-                R_ld += self.K * (1 if mode == "image" else N.ld_tiles(hh * ww))
-            if li < self.L - 1:
-                R_lp += N.ld_tiles(hh * ww)
-            cc = CC // 2
+        R_ld, R_lp = self._part_rows(B, H, W)
         ld_part = E.WS.get("ld_part", R_ld * B, torch.float32, dev)
         lp_part = E.WS.get("lp_part", max(R_lp, 1) * B, torch.float32, dev) if with_logp else None
         latents: List[Tensor] = []
@@ -629,43 +683,60 @@ class Glow(Transform):
             cur, cur_bs, ch = st, C * P, C // 2
         return latents, ld_part, R_ld, lp_part, (R_lp if with_logp else 0)
 
-    def _invert_fast(self, latents, temperature, levels, slots, steps) -> Tensor:
-        """Inverse with the fused step-boundary kernel."""
+    def _density_parts(self, B: int, H: int, W: int, dev, with_ld: bool, with_lp: bool, fused: bool):
+        """Partial buffers of one inverse that also returns its density (None where not requested), with their row
+        counts: the rows the forward writes (`_part_rows`)."""
+        R_ld, R_lp = self._part_rows(B, H, W, inverse=True, fused=fused)
+        ld_part = E.WS.get("ld_part", R_ld * B, torch.float32, dev) if with_ld else None
+        lp_part = E.WS.get("lp_part", max(R_lp, 1) * B, torch.float32, dev) if with_lp else None
+        return ld_part, R_ld, lp_part, R_lp
+
+    def _invert_fast(self, latents, temperature, levels, slots, steps, with_ld: bool = False, with_lp: bool = False):
+        """Inverse with the fused step-boundary kernel -> (x, ld_part, R_ld, lp_part, R_lp); the partials are written
+        only when requested (``with_ld`` / ``with_lp``), in level order from the deepest level."""
         z_last = latents[-1]
         B, C, h, w = z_last.shape
         dev = z_last.device
         E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
+        ld_part, R_ld, lp_part, R_lp = self._density_parts(B, h << self.L, w << self.L, dev, with_ld, with_lp, True)
         src = z_last                                   # caller memory: read only
+        row = lrow = 0
         for li in range(self.L - 1, -1, -1):
             flows, _ = levels[li]
             P = h * w
             mode = self._level_mode(B, C, h, w)
             if mode == "tiled":
-                st = self._invert_level_tiled(flows, src, B, C, h, w, dev)
+                st, rows = self._invert_level_tiled(flows, src, B, C, h, w, dev, ld_part, row)
+                row += rows
             elif mode == "unfused":
                 # NFDPM_TILED=0: unfused inverse steps (coupling^-1 in place, then K-A^-1)
                 cur, own = src, li < self.L - 1        # the deepest level reads caller memory
                 other = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
                 for step in reversed(flows):
+                    part = ld_part[row * B:] if ld_part is not None else None
                     if own:
-                        step._inverse_views(cur, C * P, cur, C * P, other, C * P, B, h, w)
+                        step._inverse_views(cur, C * P, cur, C * P, other, C * P, B, h, w, part)
                         cur, other = other, cur
                     else:
                         tmp = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-                        step._inverse_views(cur, C * P, tmp, C * P, other, C * P, B, h, w)
+                        step._inverse_views(cur, C * P, tmp, C * P, other, C * P, B, h, w, part)
                         cur, other, own = other, tmp, True
+                    row += N.ld_tiles(P)
                 st = cur
             else:
-                st = self._invert_level_fast(flows, src, li < self.L - 1, B, C, h, w, dev)
+                st = self._invert_level_fast(flows, src, li < self.L - 1, B, C, h, w, dev, ld_part, row)
+                row += len(flows)
             if li == 0:
                 out = torch.empty(B, C // 4, h * 2, w * 2, dtype=torch.float32, device=dev)
                 N.unsqueeze(st, out, B, C, h, w, C * P, (C // 4) * P * 4)
-                return out
+                return out, ld_part, R_ld, lp_part, R_lp
             Cn, hn, wn = 2 * (C // 4), h * 2, w * 2
             nxt = torch.empty(B, Cn, hn, wn, dtype=torch.float32, device=dev)
             N.unsqueeze(st, nxt, B, C, h, w, C * P, Cn * hn * wn)
             latent = get_item(latents, -(self.L - li + 1))
-            levels[li - 1][1]._fill_second_half(nxt, Cn * hn * wn, B, Cn, hn, wn, latent, temperature)
+            levels[li - 1][1]._fill_second_half(nxt, Cn * hn * wn, B, Cn, hn, wn, latent, temperature,
+                                                logp_part=lp_part[lrow * B:] if lp_part is not None else None)
+            lrow += N.ld_tiles(hn * wn)
             src, C, h, w = nxt, Cn, hn, wn
         raise AssertionError("unreachable")
 
@@ -695,10 +766,12 @@ class Glow(Transform):
             rows += T
         return bufs[src], rows
 
-    def _invert_level_tiled(self, flows, src, B: int, C: int, h: int, w: int, dev) -> Tensor:
+    def _invert_level_tiled(self, flows, src, B: int, C: int, h: int, w: int, dev, ld_part=None, row: int = 0):
         """K inverse StepFlows of one level with the row-band boundary kernel (state ping-pongs between two buffers;
-        `src` — caller memory or the previous level's output — is only read)."""
+        `src` — caller memory or the previous level's output — is only read).  Returns (state, log-det partial rows used
+        from `row` on; written only when `ld_part` is given)."""
         P = h * w
+        rows = 0
         bufs = [torch.empty(B, C, h, w, dtype=torch.float32, device=dev) for _ in range(2)]
         A1, K1p = E.coupling_a1(flows[-1].affcoupling, B, C, h, w, dev)
         N.flow_boundary_tiled(src, C * P, False, None, 0, None, None, None, None, None, None, 0, None, 0, A1, K1p, B, C,
@@ -707,20 +780,24 @@ class Glow(Transform):
         for k in range(len(flows) - 1, -1, -1):
             step = flows[k]
             T = N.flow_boundary_tiles(B, C, h, w, 1, 1, int(k > 0))
+            part = ld_part[(row + rows) * B:] if ld_part is not None else None
             if k > 0:
                 A1n, K1p = E.coupling_a1(flows[k - 1].affcoupling, B, C, h, w, dev)
-                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, cur, C * P, None, step._mix.inv_mt,
+                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, cur, C * P, part, step._mix.inv_mt,
                                     step._mix.inv_beta, bufs[dst], C * P, A1n, K1p, True, tiles=T)
                 A1 = A1n
             else:
-                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, cur, C * P, None, step._mix.inv_mt,
+                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, cur, C * P, part, step._mix.inv_mt,
                                     step._mix.inv_beta, bufs[dst], C * P, None, 0, True, tiles=T)
             cur, dst = bufs[dst], 1 - dst
-        return cur
+            rows += T
+        return cur, rows
 
-    def _invert_level_fast(self, flows, src, own: bool, B: int, C: int, h: int, w: int, dev) -> Tensor:
+    def _invert_level_fast(self, flows, src, own: bool, B: int, C: int, h: int, w: int, dev, ld_part=None,
+                           row: int = 0) -> Tensor:
         """K inverse StepFlows of one level with the fused kernels; returns the level's input state.  Deep levels run as
-        concurrent sub-batches inside a captured graph (`_deep_sub`)."""
+        concurrent sub-batches inside a captured graph (`_deep_sub`).  Step k writes its log-det partial to row `row + k`
+        of `ld_part` when given."""
         P = h * w
         st = src if own else torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
         nsub = self._deep_sub(B, h, w) if torch.cuda.is_current_stream_capturing() else 1
@@ -735,59 +812,73 @@ class Glow(Transform):
             for k in range(len(flows) - 1, -1, -1):
                 step = flows[k]
                 cp = step.affcoupling
+                part = ld_part[(row + k) * B + i * Bs:] if ld_part is not None else None
                 if k > 0:
                     A1n, K1p = E.coupling_a1(flows[k - 1].affcoupling, Bs, C, h, w, dev)
-                    E.coupling_boundary(cp, A1, Bs, C, h, w, src_i, C * P, None, step._mix.inv_mt, step._mix.inv_beta,
+                    E.coupling_boundary(cp, A1, Bs, C, h, w, src_i, C * P, part, step._mix.inv_mt, step._mix.inv_beta,
                                         st_i, C * P, A1n, K1p, True)
                     A1 = A1n
                 else:
-                    E.coupling_boundary(cp, A1, Bs, C, h, w, src_i, C * P, None, step._mix.inv_mt, step._mix.inv_beta,
+                    E.coupling_boundary(cp, A1, Bs, C, h, w, src_i, C * P, part, step._mix.inv_mt, step._mix.inv_beta,
                                         st_i, C * P, None, 0, True)
                 src_i = st_i
         self._fork_join(nsub, level_chain, pool="_deep_streams")
         return st
 
-    def _invert_core(self, latents, temperature, levels, slots, steps, ready: bool) -> Tensor:
+    def _invert_core(self, latents, temperature, levels, slots, steps, ready: bool, with_ld: bool = False,
+                     with_lp: bool = False):
+        """-> (x, ld_part, R_ld, lp_part, R_lp), as `_invert_fast`."""
         z_last = E.check_input(latents[-1], "latents[-1]")
         B, Cf, h, w = z_last.shape
         dev = z_last.device
         if ready and self._fast_ok(h * 2 ** self.L, w * 2 ** self.L):
-            return self._invert_fast([z_last] if len(latents) == 1 else list(latents), temperature, levels, slots, steps)
-        if ready:
+            return self._invert_fast([z_last] if len(latents) == 1 else list(latents), temperature, levels, slots, steps,
+                                     with_ld, with_lp)
+        if ready or with_ld:
+            # (the inverse initialises no StepFlow ActNorm, so the log-det constants of a model that is not ready are
+            # final here too)
             E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
+        ld_part, R_ld, lp_part, R_lp = self._density_parts(B, h << self.L, w << self.L, dev, with_ld, with_lp, False)
         C, P = Cf, h * w
         cur = z_last
         own = False          # `cur` is caller memory until the first step has produced a copy
+        row = lrow = 0
         for li in range(self.L - 1, -1, -1):
             flows, _ = levels[li]
             other = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
             for step in reversed(flows):
+                part = ld_part[row * B:] if ld_part is not None else None
                 if own:
-                    step._inverse_views(cur, C * P, cur, C * P, other, C * P, B, h, w)
+                    step._inverse_views(cur, C * P, cur, C * P, other, C * P, B, h, w, part)
                     cur, other = other, cur
                 else:
                     tmp = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-                    step._inverse_views(cur, C * P, tmp, C * P, other, C * P, B, h, w)
+                    step._inverse_views(cur, C * P, tmp, C * P, other, C * P, B, h, w, part)
                     cur, other, own = other, tmp, True
+                row += N.ld_tiles(P)
             # undo the squeeze of this level into the first half of the previous level's tensor
             if li == 0:
                 out = torch.empty(B, C // 4, h * 2, w * 2, dtype=torch.float32, device=dev)
                 N.unsqueeze(cur, out, B, C, h, w, C * P, (C // 4) * P * 4)
-                return out
+                return out, ld_part, R_ld, lp_part, R_lp
             Cn, hn, wn = 2 * (C // 4), h * 2, w * 2
             nxt = torch.empty(B, Cn, hn, wn, dtype=torch.float32, device=dev)
             N.unsqueeze(cur, nxt, B, C, h, w, C * P, Cn * hn * wn)
             latent = get_item(latents, -(self.L - li + 1))   # None -> draw from the conditional prior
-            levels[li - 1][1]._fill_second_half(nxt, Cn * hn * wn, B, Cn, hn, wn, latent, temperature)
+            levels[li - 1][1]._fill_second_half(nxt, Cn * hn * wn, B, Cn, hn, wn, latent, temperature,
+                                                logp_part=lp_part[lrow * B:] if lp_part is not None else None)
+            lrow += N.ld_tiles(hn * wn)
             cur, own, C, h, w, P = nxt, True, Cn, hn, wn, hn * wn
         raise AssertionError("unreachable")
 
     @torch.no_grad()
-    def sample(self, latents: list, postprocess_func=None, temperature: float = 1.0) -> Tensor:
+    def sample(self, latents: list, postprocess_func=None, temperature: float = 1.0,
+               log_det_jac: Optional[Tensor] = None, logp: Optional[Tensor] = None) -> Tensor:
         """eval() -> invert -> optional postprocess -> train(), like the reference (glow.py:230-246; note the
-        unconditional switch back to train mode)."""
+        unconditional switch back to train mode).  ``log_det_jac`` / ``logp`` as in ``invert``: the density of the
+        continuous sample before ``postprocess_func``."""
         self.eval()
-        new_samples = self.invert(latents, temperature)
+        new_samples = self.invert(latents, temperature, log_det_jac, logp)
         out = postprocess_func(new_samples.float()) if postprocess_func else new_samples.float()
         self.train()
         return out

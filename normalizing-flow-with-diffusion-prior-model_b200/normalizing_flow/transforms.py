@@ -337,22 +337,30 @@ class Split(Transform):
         return out
 
     def _fill_second_half(self, out: Tensor, obs: int, B: int, C: int, H: int, W: int, z: Optional[Tensor],
-                          temperature: float, eps_sink: Optional[list] = None) -> None:
+                          temperature: float, eps_sink: Optional[list] = None,
+                          logp_part: Optional[Tensor] = None) -> None:
         """Write the latent (given, or drawn from the conditional prior, reference transforms.py:305-307 and
         prior.py:49-50) into channels C/2..C of ``out`` whose first half is already in place.  ``eps_sink`` receives the
-        standard-normal tensor a draw used (the inverse's backward needs it)."""
+        standard-normal tensor a draw used (the inverse's backward needs it).  ``logp_part`` receives the partials of
+        log N(z; mean, exp(logs)) of the written half, as ``transform`` writes them (the model's density, whatever the
+        temperature of a draw)."""
         Ch, P = C // 2, H * W
         second = out.view(-1)[Ch * P:]
+        bias = self.conv.bias if self.conv is not None else None
+        logs = self.conv.logs if self.conv is not None else None
         if z is not None:
             z = E.check_input(z, "latent")
             if tuple(z.shape) != (B, Ch, H, W):
                 raise ValueError(f"latent has shape {tuple(z.shape)}, expected {(B, Ch, H, W)}")
             N.copy_channels(z, second, B, Ch, P, Ch * P, obs)
+            if logp_part is not None:
+                h, ldh = E.split_rows(self, out, obs, B, C, H, W)
+                N.split_prior_logp(h, ldh, bias, logs, out, obs, None, logp_part, B, C, H, W)
             return
         eps = torch.empty(B, Ch, H, W, dtype=torch.float32, device=out.device).normal_()
         if eps_sink is not None:
             eps_sink.append(eps)
         h, ldh = E.split_rows(self, out, obs, B, C, H, W)
-        bias = self.conv.bias if self.conv is not None else None
-        logs = self.conv.logs if self.conv is not None else None
         N.split_prior_sample(h, ldh, bias, logs, eps, temperature, out, obs, B, C, H, W)
+        if logp_part is not None:           # the prior conv rows h of the draw serve the density too
+            N.split_prior_logp(h, ldh, bias, logs, out, obs, None, logp_part, B, C, H, W)
