@@ -111,6 +111,12 @@ def graphs_enabled() -> bool:
     return os.environ.get("NFDPM_GRAPHS", "1") != "0"
 
 
+def fused_boundary_enabled() -> bool:
+    """``NFDPM_FUSED_BOUNDARY=0`` runs every level of Glow's inference chains on the unfused kernels: the reference the
+    fused and row-band step boundaries are tested against."""
+    return os.environ.get("NFDPM_FUSED_BOUNDARY", "1") != "0"
+
+
 def scalar_f32(device: torch.device, value: float) -> torch.Tensor:
     """Cached 1-element device tensor (multipliers for nfdpm_accumulate)."""
     key = (device.index, float(value))
@@ -162,6 +168,33 @@ def cache_hit(cached_key, key) -> bool:
     if cached_key != key:
         return False
     return own_capture or not torch.cuda.is_current_stream_capturing()
+
+
+def capture(scope, build, own: bool):
+    """``build()`` once eagerly (parameter caches, one-time kernel attributes), then under capture into a CUDA graph ->
+    (graph, what the captured ``build()`` returned, launches per replay).  Workspace buffers taken inside the captured
+    chain live under ``scope``.  ``own``: the caller refreshed the parameter caches outside the graph (``own_capture``);
+    a chain whose parameters change between replays refreshes them inside it."""
+    global own_capture
+    warm = ("warm",) + tuple(scope)
+    prev = WS.scope
+    try:
+        WS.scope = warm
+        build()
+        torch.cuda.current_stream().synchronize()
+        WS.drop_scope(warm)
+        WS.scope = scope                              # buffers baked into the graph live (only) under this scope
+        g = torch.cuda.CUDAGraph()
+        n0 = N.launch_count
+        own_capture = own
+        with torch.cuda.graph(g):
+            out = build()
+        n_launch = N.launch_count - n0
+    finally:
+        own_capture = False
+        WS.scope = prev
+    N.launch_count -= n_launch                        # counted per replay instead
+    return g, out, n_launch
 
 
 # ------------------------------------------------------------------------------------------- mix cache
@@ -377,19 +410,13 @@ def coupling_gemms(cp, A1: torch.Tensor, B: int, C: int, H: int, W: int) -> Tupl
     return pm, ldp
 
 
-def fused_g3_enabled() -> bool:
-    return os.environ.get("NFDPM_FUSED_G3", "1") != "0"
-
-
 def fused_g3_ok(B: int, C: int, H: int, W: int, F: int, ldp: int, dt: torch.dtype = torch.bfloat16) -> bool:
     """Use nfdpm_gemm3_boundary?  Measured in situ (tools/bench_levels.py, profiles/): with ONE image per CTA
     (16x16 images: 128 CTAs) it beats GEMM3 + boundary (54.6 vs 61.4 us per StepFlow chain); at the deeper levels a
-    128-row tile holds 2..8 images, only 64 / 16 CTAs exist and the separate kernels win — so only H*W == 256 takes it
-    unless NFDPM_FUSED_G3=all."""
-    v = os.environ.get("NFDPM_FUSED_G3", "1")
-    if v == "0" or dt not in TC_DTYPES or not N.gemm3_boundary_ok(B, C, H, W, F * (2 if dt == N.SPLIT else 1), ldp):
+    128-row tile holds 2..8 images, only 64 / 16 CTAs exist and the separate kernels win — so only H*W == 256 takes it."""
+    if dt not in TC_DTYPES or not N.gemm3_boundary_ok(B, C, H, W, F * (2 if dt == N.SPLIT else 1), ldp):
         return False
-    return v == "all" or H * W == 256
+    return H * W == 256
 
 
 def coupling_boundary(cp, A1: torch.Tensor, B: int, C: int, H: int, W: int, src, src_bs, ld_part, mt, beta, y, y_bs,

@@ -1,10 +1,11 @@
 """Autograd through ``Glow.invert`` and the priors' ``sample`` (``NFDPM_INVERT_GRAD=1``).
 
-``Glow.invert`` records ONE ``GlowInvertFn``.  Its forward is the no-grad inverse's kernel chain, level by level with the
-same per-level kernel choice (``Glow._level_mode``), with sinks added: fresh per-step buffers for the coupling network's
-operands (im2col rows A1, hidden maps h1 / h2, ZeroConv taps pm) and the step boundary's pre-mix sink for u_k, the coupling
-inverse's output (``gemm3_boundary(pm_out, xs, inverse)`` where the fused GEMM runs, ``flow_boundary_inv_stash`` at the
-other one-CTA-per-image levels, ``flow_boundary_tiled(xs)`` at row-band levels, the unfused kernels elsewhere).  Each step
+``Glow.invert`` records ONE ``GlowInvertFn``.  Its forward is the no-grad inverse's walk (``Glow._invert_walk``: the same
+level transitions and per-level kernel choice, ``Glow._level_mode``) with each level's StepFlows run by ``_level_stash``,
+which adds sinks: fresh per-step buffers for the coupling network's operands (im2col rows A1, hidden maps h1 / h2,
+ZeroConv taps pm) and the step boundary's pre-mix sink for u_k, the coupling inverse's output (``gemm3_boundary(pm_out,
+xs, inverse)`` where the fused GEMM runs, ``flow_boundary_inv_stash`` at the other one-CTA-per-image levels,
+``flow_boundary_tiled(xs)`` at row-band levels, the unfused kernels elsewhere).  Each step
 writes a fresh state tensor, so the state stack y_k costs no extra writes; x is the output of that one chain.  Per
 sampling Split it keeps the eps its prior draw used (drawn eagerly by ``normal_()`` on torch's CUDA generator, deepest
 first, as the no-grad inverse draws it).  The backward walks the levels 0..L-1 and the steps k = 0..K-1: mix_bwd with
@@ -26,7 +27,6 @@ from torch import Tensor
 from . import _engine as E
 from . import _modgrad as MG
 from . import _native as N
-from .utils import get_item
 
 
 def _net_rows(cp, A1: Tensor, M: int, dt: torch.dtype):
@@ -103,40 +103,19 @@ def _level_stash(flows, src: Tensor, mode: str, B: int, C: int, h: int, w: int):
 
 
 def invert_stash(glow, latents, temperature: float):
-    """Glow.invert returning (x, per-level step records, per-Split (input, eps)).  The kernels are those of the no-grad
-    inverse (uncaptured), with sinks added; an uninitialised model takes the unfused chain, which initialises the coupling
-    networks' ActNorms on the way (without gradient), as the no-grad inverse does."""
-    levels = glow._levels()
-    L = glow.L
-    z_last = latents[-1]
-    B, C, h, w = z_last.shape
-    dev = z_last.device
-    steps = [s for flows, _ in levels for s in flows]
-    ready = all(s._ready() for s in steps)
-    fast = ready and glow._fast_ok(h * 2 ** L, w * 2 ** L)
-    if ready:
-        slots = glow._slots(dev)
-        E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
-    steps_rec, split_rec = [None] * L, [None] * L
-    cur = z_last
-    for li in range(L - 1, -1, -1):
-        flows, _ = levels[li]
-        P = h * w
-        mode = glow._level_mode(B, C, h, w) if fast else "unfused"
-        cur, steps_rec[li] = _level_stash(flows, cur, mode, B, C, h, w)
-        if li == 0:
-            out = torch.empty(B, C // 4, h * 2, w * 2, dtype=torch.float32, device=dev)
-            N.unsqueeze(cur, out, B, C, h, w, C * P, (C // 4) * P * 4)
-            return out, steps_rec, split_rec
-        Cn, hn, wn = 2 * (C // 4), h * 2, w * 2
-        nxt = torch.empty(B, Cn, hn, wn, dtype=torch.float32, device=dev)
-        N.unsqueeze(cur, nxt, B, C, h, w, C * P, Cn * hn * wn)
-        sink = []
-        levels[li - 1][1]._fill_second_half(nxt, Cn * hn * wn, B, Cn, hn, wn, get_item(latents, -(L - li + 1)),
-                                            temperature, eps_sink=sink)
-        split_rec[li - 1] = (nxt, sink[0] if sink else None)
-        cur, C, h, w = nxt, Cn, hn, wn
-    raise AssertionError("unreachable")
+    """Glow.invert returning (x, per-level step records, per-Split (input, eps)).  The walk and the kernels are those of the
+    no-grad inverse (uncaptured, ``Glow._invert_walk``), with `_level_stash` for each level's StepFlows; an uninitialised
+    model takes the unfused chain, which initialises the coupling networks' ActNorms on the way (without gradient), as the
+    no-grad inverse does."""
+    steps_rec, split_rec = [], []
+
+    def level(mode, flows, src, B, C, h, w):
+        x, recs = _level_stash(flows, src, mode, B, C, h, w)
+        steps_rec.insert(0, recs)                       # the walk runs deepest first
+        return x
+
+    x, _ = glow._invert_walk(latents, temperature, glow._ready(), level=level, eps_sink=split_rec)
+    return x, steps_rec, split_rec[::-1]
 
 
 class GlowInvertFn(torch.autograd.Function):
@@ -160,17 +139,15 @@ class GlowInvertFn(torch.autograd.Function):
         glow, T, n_lat = ctx.glow, ctx.temperature, ctx.n_lat
         steps_rec, split_rec = ctx.rec
         ctx.rec = None
-        levels = glow._levels()
         L = glow.L
-        dx = dx.to(torch.float32).contiguous()
-        B, c, H, W = dx.shape
-        C, h, w = 4 * c, H // 2, W // 2
-        d = torch.empty(B, C, h, w, dtype=torch.float32, device=dx.device)
-        N.squeeze(dx, d, B, c, H, W, c * H * W, C * h * w)
+        dy = dx.to(torch.float32).contiguous()
+        B, _, H, W = dy.shape
         g = {}
         d_lat: List[Optional[Tensor]] = [None] * n_lat
-        for li in range(L):
-            flows, split = levels[li]
+        for li, (flows, split, C, h, w) in enumerate(glow._geometry(H, W)):
+            # gradient of the level's output state: squeeze of the gradient of what it unsqueezed into
+            d = torch.empty(B, C, h, w, dtype=torch.float32, device=dy.device)
+            N.squeeze(dy, d, B, C // 4, 2 * h, 2 * w, C * h * w, C * h * w)
             da1, lda1 = None, 0
             for step, (y_k, st_k, u_k) in zip(flows, steps_rec[li]):
                 an, ic = step.actnorm, step.invconv2d
@@ -182,7 +159,7 @@ class GlowInvertFn(torch.autograd.Function):
                 lda1 = st_k.K1p
                 g.update(gc)
             N.col2im_add(da1, lda1, d, C * h * w, B, C // 2, h, w)
-            if li == L - 1:
+            if split is None:
                 d_lat[n_lat - 1] = d
                 break
             nxt, eps = split_rec[li]
@@ -190,10 +167,6 @@ class GlowInvertFn(torch.autograd.Function):
             g.update(gs)
             if dz is not None:
                 d_lat[n_lat - (L - li)] = dz
-            Ch, P = C // 2, h * w
-            C, h, w = 4 * Ch, h // 2, w // 2
-            d = torch.empty(B, C, h, w, dtype=torch.float32, device=dx.device)
-            N.squeeze(dy, d, B, Ch, 2 * h, 2 * w, Ch * P, C * h * w)
         lat_g = [gl if ctx.needs_input_grad[3 + i] else None for i, gl in enumerate(d_lat)]
         par_g = [g.get(p) if p.requires_grad else None for p in ctx.params]
         return (None, None, None) + tuple(lat_g) + tuple(par_g)

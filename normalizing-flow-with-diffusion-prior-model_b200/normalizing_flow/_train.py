@@ -75,45 +75,26 @@ class Stash:
         self.dt = torch.bfloat16
 
 
-def supported(glow, H: int, W: int) -> bool:
-    return True
-
-
-def _level_fast(C: int, h: int, w: int) -> bool:
-    """Can the fused step-boundary kernel hold one image of this level in a CTA?"""
-    return h * w <= 256 and N.flow_boundary_smem(C, h, w, 1, 1) <= 200 * 1024
-
-
 def forward_train(glow, x: Tensor, with_logp: bool):
     """Glow.transform with every tensor the backward needs kept alive: per StepFlow the K-A input x_k, the K-A output
     u_k (= coupling input), the im2col rows A1_k, the hidden maps h1_k / h2_k and the taps-as-N rows pm_k."""
     B, c, H, W = x.shape
     dev = x.device
-    levels = glow._levels()
-    slots = glow._slots(dev)
-    steps = [s for flows, _ in levels for s in flows]
-    E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
+    glow._prepare_mix(dev)
     K = glow.K
     dt = E.coupling_dtype(train=True)
-    glow._pack_plan(steps, dt, True).refresh()      # every forward / transposed weight layout in one launch
+    glow._pack_plan(glow._steps(), dt, True).refresh()      # every forward / transposed weight layout in one launch
     st = Stash()
     st.B, st.with_logp, st.in_shape, st.dt = B, with_logp, (B, c, H, W), dt
-    R_ld, R_lp = 0, 0
-    hh, ww, cc = H, W, c
-    for li_ in range(glow.L):
-        hh, ww, CC = hh // 2, ww // 2, cc * 4
-        R_ld += K * (1 if _level_fast(CC, hh, ww) else N.ld_tiles(hh * ww))
-        if li_ < glow.L - 1:
-            R_lp += N.ld_tiles(hh * ww)
-        cc = CC // 2
+    geo = glow._geometry(H, W)
+    R_ld = sum(K * (1 if glow._level_fast(C, h, w) else N.ld_tiles(h * w)) for _, _, C, h, w in geo)
+    R_lp = sum(N.ld_tiles(h * w) for _, split, _, h, w in geo if split is not None)
     ld_part = torch.empty(R_ld * B, dtype=torch.float32, device=dev)
     lp_part = torch.empty(max(R_lp, 1) * B, dtype=torch.float32, device=dev) if with_logp else None
     latents: List[Tensor] = []
     cur, cur_bs = x, c * H * W
-    h, w, ch = H, W, c
     row = lrow = 0
-    for li, (flows, split) in enumerate(levels):
-        h, w, C = h // 2, w // 2, ch * 4
+    for flows, split, C, h, w in geo:
         P, M = h * w, B * h * w
         first = flows[0].affcoupling
         conv1 = first._parts()[0]
@@ -130,7 +111,7 @@ def forward_train(glow, x: Tensor, with_logp: bool):
         lv.pm = torch.empty(K, M, ldp, **f32)
         lv.state_out = torch.empty(B, C, h, w, **f32)
         fused_g3 = E.fused_g3_ok(B, C, h, w, F, ldp, dt)
-        fast = _level_fast(C, h, w)
+        fast = glow._level_fast(C, h, w)
         T_ld = 1 if fast else N.ld_tiles(P)
         if fast:
             # level entry: squeeze + stash x_0 + K-A of step 0 + im2col
@@ -167,8 +148,7 @@ def forward_train(glow, x: Tensor, with_logp: bool):
                 N.flow_boundary_stash(lv.u[k], C * P, False, lv.pm[k], ldp, zc.bias, zc.logs, ld_part[row * B:],
                                       mt, beta, y, C * P, xs, C * P if xs is not None else 0, a1n,
                                       K1p if a1n is not None else 0, B, C, h, w)
-            row += T_ld - 1
-            row += 1
+            row += T_ld
         st.levels.append(lv)
         if split is None:
             latents.append(lv.state_out)
@@ -177,7 +157,8 @@ def forward_train(glow, x: Tensor, with_logp: bool):
         split._forward_views(lv.state_out, C * P, B, C, h, w, z, lp_part[lrow * B:] if lp_part is not None else None)
         lrow += N.ld_tiles(P)
         latents.append(z)
-        cur, cur_bs, ch = lv.state_out, C * P, C // 2
+        cur, cur_bs = lv.state_out, C * P
+    assert (row, lrow) == (R_ld, R_lp), f"wrote {row} / {lrow} partial rows, allotted {R_ld} / {R_lp}"
     return latents, ld_part, R_ld, lp_part, (R_lp if with_logp else 0), st
 
 
@@ -495,27 +476,6 @@ class _TrainChains:
         self.owner = None
 
 
-def _capture(scope, build):
-    """build() once eagerly (parameter caches, one-time kernel attributes), then under capture; buffers taken from the
-    workspace pool inside the chain live under ``scope``."""
-    prev = E.WS.scope
-    try:
-        E.WS.scope = ("warm",) + tuple(scope)
-        build()
-        torch.cuda.current_stream().synchronize()
-        E.WS.drop_scope(("warm",) + tuple(scope))
-        E.WS.scope = scope
-        g = torch.cuda.CUDAGraph()
-        n0 = N.launch_count
-        with torch.cuda.graph(g):
-            out = build()
-        n = N.launch_count - n0
-    finally:
-        E.WS.scope = prev
-    N.launch_count -= n                               # counted per replay
-    return g, out, n
-
-
 def _train_chains(glow, x: Tensor, with_logp: bool) -> Optional["_TrainChains"]:
     if not train_graphs_enabled() or torch.cuda.is_current_stream_capturing() or \
             getattr(glow, "_grad_hook", None) is not None:
@@ -533,7 +493,8 @@ def _train_chains(glow, x: Tensor, with_logp: bool) -> Optional["_TrainChains"]:
         tc.scope = ("train", id(glow), key)
         tc.x = torch.empty_like(x)
         tc.x.copy_(x)
-        tc.fwd, tc.fwd_out, tc.n_fwd = _capture(tc.scope + ("fwd",), lambda: forward_train(glow, tc.x, with_logp))
+        tc.fwd, tc.fwd_out, tc.n_fwd = E.capture(tc.scope + ("fwd",), lambda: forward_train(glow, tc.x, with_logp),
+                                                 own=False)
         tc.epoch = E.alloc_epoch
         store[key] = tc
     return None if tc.busy else tc
@@ -559,7 +520,7 @@ def _bwd_chain(tc: "_TrainChains", glow, params, g_lat, g_ld, g_lp, need_dx: boo
                 if p.requires_grad and id(p) not in sink.written:
                     sink.get(p).zero_()
             return sink, dx
-        g, (sink, dx), n = _capture(tc.scope + ("bwd", len(tc.bwd)), build)
+        g, (sink, dx), n = E.capture(tc.scope + ("bwd", len(tc.bwd)), build, own=False)
         ent = tc.bwd[key] = dict(graph=g, sink=sink, dx=dx, n=n, lat=s_lat, ld=s_ld, lp=s_lp)
     return ent
 
@@ -571,7 +532,7 @@ class GlowTransformFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, glow, x, ld, lp, *params):
         with_logp = lp is not None
-        B, c, H, W = x.shape
+        H, W = x.shape[2:]
         tc = _train_chains(glow, x, with_logp)
         if tc is not None:
             tc.x.copy_(x)
@@ -583,14 +544,8 @@ class GlowTransformFn(torch.autograd.Function):
         else:
             latents, ld_part, R_ld, lp_part, R_lp, st = forward_train(glow, x, with_logp)
         ctx.chains = tc
-        dev = x.device
-        N.accumulate(ld, ld_part, R_ld, B, glow._slots(dev), glow._multipliers(H, W, dev), glow.L * glow.K)
-        dirty = [ld]
-        if with_logp:
-            if R_lp > 0:
-                N.accumulate(lp, lp_part, R_lp, B)
-            dirty.append(lp)
-        ctx.mark_dirty(*dirty)
+        glow._add_density(ld, lp, (ld_part, R_ld, lp_part, R_lp), H, W)
+        ctx.mark_dirty(*([ld, lp] if with_logp else [ld]))
         ctx.glow, ctx.stash, ctx.with_logp = glow, st, with_logp
         ctx.params = params
         if with_logp:

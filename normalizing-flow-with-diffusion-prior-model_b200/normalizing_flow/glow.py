@@ -207,44 +207,38 @@ class Glow(Transform):
             return True
         return False
 
-    def _refresh_caches(self, steps, slots) -> None:
+    def _refresh_caches(self, device: torch.device) -> None:
         """Re-run LU/fold and weight packing for parameters that changed (outside any graph)."""
-        E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
-        self._pack_plan(steps, E.coupling_dtype(), False).refresh()
+        self._prepare_mix(device)
+        self._pack_plan(self._steps(), E.coupling_dtype(), False).refresh()
         for blk in self.blocks:
             E.refresh_split(blk.split, blk.flows[0]._C)
 
     def _use_graph(self, ready: bool) -> bool:
         return ready and E.graphs_enabled() and not torch.cuda.is_current_stream_capturing()
 
-    def _graph_entry(self, key, build):
-        """build() -> dict of static tensors; called once eagerly (warm-up) and once under capture."""
+    def _replay(self, key, inputs: List[Tensor], walk):
+        """The captured call ``key``: refresh the parameter caches if a parameter changed, copy ``inputs`` into the entry's
+        static tensors, capture ``walk(statics)`` when the entry is missing or stale, replay.  Returns what the captured
+        walk returned (graph-static tensors)."""
+        if self._params_changed():
+            self._refresh_caches(inputs[0].device)
         ent = self._graphs.get(key)
-        if ent is not None and ent["epoch"] == E.alloc_epoch:
-            return ent
-        scope = ("glow", id(self), key)
-        E.WS.drop_scope(scope)
-        prev = E.WS.scope
-        try:
-            E.WS.scope = ("warm", id(self))
-            build()                                   # eager warm-up: parameter caches, one-time kernel attributes
-            torch.cuda.current_stream().synchronize()
-            E.WS.drop_scope(("warm", id(self)))
-            E.WS.scope = scope                        # buffers baked into the graph live (only) under this scope
-            g = torch.cuda.CUDAGraph()
-            n0 = N.launch_count
-            E.own_capture = True                      # parameter caches were refreshed above, outside the graph
-            with torch.cuda.graph(g):
-                out = build()
-            n_launch = N.launch_count - n0
-        finally:
-            E.own_capture = False
-            E.WS.scope = prev
-        N.launch_count -= n_launch                    # counted per replay instead
-        ent = dict(out)
-        ent["graph"], ent["epoch"], ent["n_launch"] = g, E.alloc_epoch, n_launch
-        self._graphs[key] = ent
-        return ent
+        statics = ent["in"] if ent is not None else [torch.empty_like(t) for t in inputs]
+        for s_, t in zip(statics, inputs):
+            if s_.shape != t.shape:
+                raise ValueError(f"input has shape {tuple(t.shape)}, expected {tuple(s_.shape)}")
+            s_.copy_(t)
+        if ent is None or ent["epoch"] != E.alloc_epoch:
+            scope = ("glow", id(self), key)
+            E.WS.drop_scope(scope)
+            # parameter caches were refreshed above, outside the graph
+            g, out, n_launch = E.capture(scope, lambda: walk(statics), own=True)
+            ent = self._graphs[key] = {"in": statics, "out": out, "graph": g, "n_launch": n_launch,
+                                       "epoch": E.alloc_epoch}
+        ent["graph"].replay()
+        N.launch_count += ent["n_launch"]
+        return ent["out"]
 
     # ---- helpers
     def _levels(self) -> List[Tuple[nn.ModuleList, Optional[Split]]]:
@@ -252,21 +246,36 @@ class Glow(Transform):
         lv.append((self.final_flows, None))
         return lv
 
+    def _geometry(self, H: int, W: int) -> List[Tuple[nn.ModuleList, Optional[Split], int, int, int]]:
+        """Per level, in forward order, for [B, c, H, W] images: (StepFlows, Split or None at the last level, channels C,
+        height h and width w of the level's squeezed flow state)."""
+        return [(flows, split, (4 * self.in_channel) << li, H >> (li + 1), W >> (li + 1))
+                for li, (flows, split) in enumerate(self._levels())]
+
+    def _steps(self) -> List[StepFlow]:
+        return [s for flows, _ in self._levels() for s in flows]
+
+    def _ready(self) -> bool:
+        """Every StepFlow's ActNorms are initialised (the first transform of a fresh model initialises them)."""
+        return all(s._ready() for s in self._steps())
+
     def _slots(self, device: torch.device) -> Tensor:
         n = self.L * self.K
         if self._logdet_all is None or self._logdet_all.device != device:
             self._logdet_all = torch.zeros(n, dtype=torch.float32, device=device)
         return self._logdet_all
 
+    def _prepare_mix(self, device: torch.device) -> None:
+        """One batched LU/fold launch for every StepFlow whose parameters changed since the last call; step i's
+        log|det W| lands in slot i, which the final accumulate reads."""
+        slots = self._slots(device)
+        E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(self._steps())])
+
     def _multipliers(self, H: int, W: int, device: torch.device) -> Tensor:
         key = (H, W, device.index)
         t = self._cmul.get(key)
         if t is None:
-            vals = []
-            h, w = H, W
-            for _ in range(self.L):
-                h, w = h // 2, w // 2
-                vals += [float(h * w)] * self.K
+            vals = [float(h * w) for _, _, _, h, w in self._geometry(H, W) for _ in range(self.K)]
             t = torch.tensor(vals, dtype=torch.float32, device=device)
             self._cmul[key] = t
         return t
@@ -287,115 +296,28 @@ class Glow(Transform):
             raise ValueError("log_det_jac accumulator is required")
         E.check_acc(log_det_jac, B, "log_det_jac")
         E.check_acc(logp, B, "logp")
-        dev = x.device
-        levels = self._levels()
-        slots = self._slots(dev)
-        steps = [s for flows, _ in levels for s in flows]
-        ready = all(s._ready() for s in steps)
+        ready = self._ready()
         if E.autograd_needed(x, self):
-            return self._transform_autograd(x, log_det_jac, logp, levels, slots, steps, ready)
+            return self._transform_autograd(x, log_det_jac, logp, ready)
+        with_logp = logp is not None
         if self._use_graph(ready):
-            if self._params_changed():
-                self._refresh_caches(steps, slots)
-            key = ("fwd", B, H, W, logp is not None, E.precision(), dev.index)
-            x_static = self._graphs.get(key, {}).get("x")
-            if x_static is None:
-                x_static = torch.empty_like(x)
-            x_static.copy_(x)
-
-            nsub = self._n_sub(B)
-            Bs = B // nsub
-
-            def build():
-                # images are independent: sub-batches run on concurrent streams inside the graph, so that the deep
-                # levels (few rows per kernel, < 148 CTAs) of one sub-batch overlap with kernels of the other
-                parts = self._fork_join(nsub, lambda i: self._transform_core(
-                    x_static[i * Bs:(i + 1) * Bs], logp is not None, levels, slots, steps, True))
-                return {"x": x_static, "parts": parts}
-            ent = self._graph_entry(key, build)
-            if ent["x"] is not x_static:              # entry was (re)built around another buffer
-                ent["x"].copy_(x)
-            ent["graph"].replay()
-            N.launch_count += ent["n_launch"]
-            parts = ent["parts"]
-            latents = [torch.cat([p[0][j] for p in parts]) if nsub > 1 else parts[0][0][j].clone()
-                       for j in range(len(parts[0][0]))]
-            cm = self._multipliers(H, W, dev)
-            for i, (_, ld_part, R_ld, lp_part, R_lp) in enumerate(parts):
-                N.accumulate(log_det_jac[i * Bs:(i + 1) * Bs], ld_part, R_ld, Bs, slots, cm, self.L * self.K)
-                if logp is not None and R_lp > 0:
-                    N.accumulate(logp[i * Bs:(i + 1) * Bs], lp_part, R_lp, Bs)
-            return latents, log_det_jac, logp
-        latents, ld_part, R_ld, lp_part, R_lp = self._transform_core(x, logp is not None, levels, slots, steps, ready)
-        N.accumulate(log_det_jac, ld_part, R_ld, B, slots, self._multipliers(H, W, dev), self.L * self.K)
-        if logp is not None and R_lp > 0:
-            N.accumulate(logp, lp_part, R_lp, B)
+            key = ("fwd", B, H, W, with_logp, E.precision(), x.device.index)
+            latents, parts = self._replay(key, [x], lambda xs: self._transform_walk(xs[0], with_logp, True))
+            latents = [z.clone() for z in latents]
+        else:
+            latents, parts = self._transform_walk(x, with_logp, ready)
+        self._add_density(log_det_jac, logp, parts, H, W)
         return latents, log_det_jac, logp
 
-    # ---- concurrent sub-batches inside a captured graph
-    def _n_sub(self, B: int) -> int:
-        # measured (profiles/): with batch 128 two concurrent sub-batches are 6% SLOWER than one stream (the deep-level
-        # kernels are latency-, not occupancy-bound), so the default is one stream; the knob stays for large batches
-        n = int(os.environ.get("NFDPM_STREAMS", "1"))
-        if n <= 1 or B % n != 0 or B // n < 16:
-            return 1
-        return n
-
-    @staticmethod
-    def _deep_sub(B: int, h: int, w: int) -> int:
-        """Concurrent sub-batches for ONE level's StepFlow chain.  At the deep levels (8x8 and smaller) every kernel of the
-        chain is latency-bound on a fraction of the SMs (one 128-row tile per CTA: 16...128 CTAs, 8-15 us per launch of which
-        2-6 us are MMA work), and the images of a batch are independent: running the chain of several image groups on
-        concurrent streams inside the captured graph overlaps those latencies.  Level 0 stays on one stream (its persistent
-        GEMM grids already fill the GPU; splitting it was measured 6 % slower).  NFDPM_DEEP_STREAMS="n1:n2" = sub-batches
-        at 64-pixel / 16-pixel-and-smaller levels.  MEASURED SLOWER in every combination (profiles/r02_deep_streams.txt:
-        5.60 ms per config-2 step on one stream, 5.90 / 5.92 / 6.71 ms with 2:2 / 2:4 / 4:4) — the deep-level GEMMs turn out
-        to be bound by the depth of their TMA operand ring (two 32 KB stages in flight per ~1 us L2 round trip = 64 GB/s per
-        CTA), not by idle SMs, and concurrent chains compete for the same L2 — so the default is one stream ("1:1")."""
-        if h * w >= 256:
-            return 1
-        spec = os.environ.get("NFDPM_DEEP_STREAMS", "1:1").split(":")
-        try:
-            n = int(spec[0] if h * w >= 64 else spec[-1])
-        except ValueError:
-            n = 1
-        while n > 1 and (B % n != 0 or (B // n) * h * w < 256):      # whole sub-batches of at least two 128-row tiles
-            n -= 1
-        return max(n, 1)
-
-    def _fork_join(self, n: int, fn, pool: str = "_streams"):
-        """fn(0) ... fn(n-1) on n concurrent streams forked from / joined into the current one (inside a capture: parallel
-        branches of the graph).  `pool`: attribute holding the streams, so that nested forks do not share them."""
-        if n == 1:
-            return [fn(0)]
-        cur = torch.cuda.current_stream()
-        if getattr(self, pool, None) is None or len(getattr(self, pool)) < n:
-            setattr(self, pool, [torch.cuda.Stream() for _ in range(n)])
-        streams = getattr(self, pool)
-        out = []
-        for i in range(n):
-            s = streams[i]
-            s.wait_stream(cur)
-            with torch.cuda.stream(s):
-                out.append(fn(i))
-        for i in range(n):
-            cur.wait_stream(streams[i])
-        return out
-
-    def _transform_autograd(self, x, log_det_jac, logp, levels, slots, steps, ready):
+    def _transform_autograd(self, x, log_det_jac, logp, ready: bool):
         """Training path (reference trainer.py:155-164): forward with activation stash, hand-written backward kernels
         behind one autograd Function (normalizing_flow/_train.py)."""
         from . import _train as T
-        B, c, H, W = x.shape
-        if not T.supported(self, H, W):
-            raise NotImplementedError(
-                f"Glow.transform under autograd: the training kernels need every level's image to fit one CTA "
-                f"(H*W/4 <= 256 at level 0); got {H}x{W}.  Use torch.no_grad() for likelihood evaluation.")
         if not ready:
             # data-dependent ActNorm initialisation happens inside the first transform (transforms.py:74-78), without
             # gradient; run it once on this batch, then take the training path
             with torch.no_grad():
-                self._transform_core(x.detach(), logp is not None, levels, slots, steps, False)
+                self._transform_walk(x.detach(), logp is not None, False)
         if torch.is_grad_enabled() and (log_det_jac.requires_grad or (logp is not None and logp.requires_grad)):
             raise RuntimeError("log_det_jac / logp are updated in place and must not require grad on entry")
         out = T.GlowTransformFn.apply(self, x, log_det_jac, logp, *list(self.parameters()))
@@ -403,14 +325,9 @@ class Glow(Transform):
             return list(out[2:]), out[0], out[1]
         return list(out[1:]), out[0], None
 
-    def _fast_ok(self, H: int, W: int) -> bool:
-        """Use the fused step-boundary kernels?  They are chosen PER LEVEL (`_level_fast`): a level whose image does not
-        fit one CTA (more than 256 pixels, e.g. the 64x64 and 32x32 levels of a 128x128 input) runs the unfused
-        kernels, the deeper levels of the same model still run the fused ones."""
-        return os.environ.get("NFDPM_FUSED_BOUNDARY", "1") != "0"
-
     @staticmethod
     def _level_fast(C: int, h: int, w: int) -> bool:
+        """Can the fused step-boundary kernel hold one image of this level in a CTA?"""
         return h * w <= 256 and N.flow_boundary_smem(C, h, w, 1, 1) <= 200 * 1024
 
     @classmethod
@@ -421,54 +338,139 @@ class Glow(Transform):
                     128x128 input) and small batches (config 4: 8 images per GPU would occupy 8 of 148 SMs)
           "unfused" separate K-A / im2col / coupling kernels (NFDPM_TILED=0, or a single image row beyond shared memory)"""
         tiled = os.environ.get("NFDPM_TILED", "1") != "0" and N.flow_boundary_tiles(B, C, h, w, 1, 1, 1) > 0
-        deep = os.environ.get("NFDPM_TILED_DEEP", "0") == "1" and h * w < 256        # experiment knob
-        if cls._level_fast(C, h, w) and ((B >= 64 and not deep) or not tiled):
+        if cls._level_fast(C, h, w) and (B >= 64 or not tiled):
             return "image"
         return "tiled" if tiled else "unfused"
 
-    def _transform_core(self, x: Tensor, with_logp: bool, levels, slots, steps, ready: bool):
+    def _part_rows(self, B: int, H: int, W: int, inverse: bool = False, fused: bool = True) -> Tuple[int, int]:
+        """Rows of B per-image partials that one call writes for [B, c, H, W] images: (log-det rows, Split log-prob rows).
+        Log-det: one per step at "image" levels, ld_tiles(P) per step at unfused ones, one per band at "tiled" levels, where
+        K-1 boundaries carry an im2col sink and the level's last one does not (and has a mix in the inverse only, which can
+        change the band height).  ``fused=False``: every level unfused (NFDPM_FUSED_BOUNDARY=0, or a model not ready)."""
+        R_ld = R_lp = 0
+        for _, split, C, h, w in self._geometry(H, W):
+            mode = self._level_mode(B, C, h, w) if fused else "unfused"
+            if mode == "tiled":
+                R_ld += (self.K - 1) * N.flow_boundary_tiles(B, C, h, w, 1, 1, 1) + \
+                    N.flow_boundary_tiles(B, C, h, w, 1, int(inverse), 0)
+            else:
+                R_ld += self.K * (1 if mode == "image" else N.ld_tiles(h * w))
+            if split is not None:
+                R_lp += N.ld_tiles(h * w)
+        return R_ld, R_lp
+
+    def _density_parts(self, B: int, H: int, W: int, dev, inverse: bool, fused: bool, with_ld: bool, with_lp: bool):
+        """(ld_part, R_ld, lp_part, R_lp): the partial buffers of one call (None where not requested) with the row counts
+        of `_part_rows`."""
+        R_ld, R_lp = self._part_rows(B, H, W, inverse, fused)
+        ld_part = E.WS.get("ld_part", R_ld * B, torch.float32, dev) if with_ld else None
+        lp_part = E.WS.get("lp_part", max(R_lp, 1) * B, torch.float32, dev) if with_lp else None
+        return ld_part, R_ld, lp_part, R_lp
+
+    def _add_density(self, log_det_jac, logp, parts, H: int, W: int) -> None:
+        """The final accumulates of a call, after its chain or its replay: the log-det partial rows plus the L*K
+        data-independent constants H*W*(sum(scale) + log|det W|), and the Split log-prob rows (``None``: not requested)."""
+        ld_part, R_ld, lp_part, R_lp = parts
+        if log_det_jac is not None:
+            dev = ld_part.device
+            N.accumulate(log_det_jac, ld_part, R_ld, log_det_jac.shape[0], self._slots(dev), self._multipliers(H, W, dev),
+                         self.L * self.K)
+        if logp is not None and R_lp > 0:
+            N.accumulate(logp, lp_part, R_lp, logp.shape[0])
+
+    def _transform_walk(self, x: Tensor, with_logp: bool, ready: bool):
+        """x -> (latents, (ld_part, R_ld, lp_part, R_lp)): the levels in forward order.  Each level squeezes its input, runs
+        its K StepFlows with the kernels of its `_level_mode` (every level unfused for a model that is not ready or under
+        NFDPM_FUSED_BOUNDARY=0) and splits off its latent."""
         B, c, H, W = x.shape
         dev = x.device
-        if ready and self._fast_ok(H, W):
-            return self._transform_fast(x, with_logp, levels, slots, steps)
+        fused = ready and E.fused_boundary_enabled()
         if ready:
-            # one batched LU/fold launch for every StepFlow whose parameters changed since the last call
-            E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
-        # partial-sum rows: per step T_l rows of B
-        geo = []
-        h, w, ch = H, W, c
-        for li in range(self.L):
-            h, w = h // 2, w // 2
-            C = ch * 4
-            geo.append((C, h, w, N.ld_tiles(h * w)))
-            ch = C // 2
-        R_ld = sum(g[3] for g in geo) * self.K
-        R_lp = sum(g[3] for g in geo[:-1])
-        ld_part = E.WS.get("ld_part", max(R_ld, 1) * B, torch.float32, dev)
-        lp_part = E.WS.get("lp_part", max(R_lp, 1) * B, torch.float32, dev) if with_logp else None
+            self._prepare_mix(dev)
+        parts = ld_part, R_ld, lp_part, R_lp = self._density_parts(B, H, W, dev, False, fused, True, with_logp)
+        slots = self._slots(dev)
+        run = {"image": self._transform_level_image, "tiled": self._transform_level_tiled,
+               "unfused": self._transform_level_unfused}
         latents: List[Tensor] = []
-        cur, cur_bs, cur_c, cur_h, cur_w = x, c * H * W, c, H, W
-        row = lrow = si = 0
-        for li, (flows, split) in enumerate(levels):
-            C, h, w, T = geo[li]
-            P = h * w
-            a = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-            b = torch.empty_like(a)
-            N.squeeze(cur, a, B, cur_c, cur_h, cur_w, cur_bs, C * P)
-            for step in flows:
-                step._forward_views(a, C * P, b, C * P, B, h, w, ld_part[row * B:], slots[si:si + 1])
-                a, b = b, a
-                row += T
-                si += 1
+        cur, cur_bs = x, c * H * W
+        row = lrow = 0
+        for li, (flows, split, C, h, w) in enumerate(self._geometry(H, W)):
+            mode = self._level_mode(B, C, h, w) if fused else "unfused"
+            st, rows = run[mode](flows, slots[li * self.K:(li + 1) * self.K], cur, cur_bs, B, C, h, w, ld_part, row)
+            row += rows
             if split is None:
-                latents.append(a)
+                latents.append(st)
                 break
             z = torch.empty(B, C // 2, h, w, dtype=torch.float32, device=dev)
-            split._forward_views(a, C * P, B, C, h, w, z, lp_part[lrow * B:] if lp_part is not None else None)
-            lrow += T
+            split._forward_views(st, C * h * w, B, C, h, w, z, lp_part[lrow * B:] if lp_part is not None else None)
+            lrow += N.ld_tiles(h * w)
             latents.append(z)
-            cur, cur_bs, cur_c, cur_h, cur_w = a, C * P, C // 2, h, w
-        return latents, ld_part, R_ld, lp_part, R_lp
+            cur, cur_bs = st, C * h * w
+        assert (row, lrow) == (R_ld, R_lp), f"wrote {row} / {lrow} partial rows, allotted {R_ld} / {R_lp}"
+        return latents, parts
+
+    def _transform_level_image(self, flows, slots, src, src_bs: int, B: int, C: int, h: int, w: int, ld_part, row: int):
+        """K forward StepFlows with one CTA per image, in place on the level's state: the level entry (squeeze + K-A of
+        step 0 + im2col), then per step GEMM1, GEMM2 and [GEMM3 +] the step boundary.  Returns (state, log-det partial rows
+        written from `row` on)."""
+        P, dev = h * w, src.device
+        st = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
+        first = flows[0]
+        A1, K1p = E.coupling_a1(first.affcoupling, B, C, h, w, dev)
+        N.flow_boundary(src, src_bs, True, None, 0, None, None, None, first._mix.fwd_mt, first._mix.fwd_beta, st, C * P,
+                        A1, K1p, B, C, h, w, False)
+        for k, step in enumerate(flows):
+            cp = step.affcoupling
+            nxt = flows[k + 1] if k + 1 < len(flows) else None
+            part = ld_part[(row + k) * B:]
+            if nxt is not None:
+                A1n, K1p = E.coupling_a1(nxt.affcoupling, B, C, h, w, dev)     # same scratch buffer as A1
+                E.coupling_boundary(cp, A1, B, C, h, w, st, C * P, part, nxt._mix.fwd_mt, nxt._mix.fwd_beta, st, C * P,
+                                    A1n, K1p, False)
+                A1 = A1n
+            else:
+                E.coupling_boundary(cp, A1, B, C, h, w, st, C * P, part, None, None, st, C * P, None, 0, False)
+        return st, len(flows)
+
+    def _transform_level_tiled(self, flows, slots, src, src_bs: int, B: int, C: int, h: int, w: int, ld_part, row: int):
+        """K forward StepFlows of one level with the row-band boundary kernel.  A band reads halo rows that a neighbouring
+        band writes, so the flow state ping-pongs between two buffers.  Returns (state, log-det partial rows written)."""
+        P, dev = h * w, src.device
+        bufs = [torch.empty(B, C, h, w, dtype=torch.float32, device=dev) for _ in range(2)]
+        first = flows[0]
+        A1, K1p = E.coupling_a1(first.affcoupling, B, C, h, w, dev)
+        N.flow_boundary_tiled(src, src_bs, True, None, 0, None, None, None, first._mix.fwd_mt, first._mix.fwd_beta,
+                              bufs[0], C * P, None, 0, A1, K1p, B, C, h, w, False,
+                              N.flow_boundary_tiles(B, C, h, w, 0, 1, 1))       # level entry: squeeze + K-A + im2col
+        cur, rows = 0, 0
+        for k, step in enumerate(flows):
+            nxt = flows[k + 1] if k + 1 < len(flows) else None
+            T = N.flow_boundary_tiles(B, C, h, w, 1, int(nxt is not None), int(nxt is not None))
+            if nxt is not None:
+                A1n, K1p = E.coupling_a1(nxt.affcoupling, B, C, h, w, dev)
+                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, bufs[cur], C * P, ld_part[(row + rows) * B:],
+                                    nxt._mix.fwd_mt, nxt._mix.fwd_beta, bufs[1 - cur], C * P, A1n, K1p, False, tiles=T)
+                A1 = A1n
+            else:
+                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, bufs[cur], C * P, ld_part[(row + rows) * B:],
+                                    None, None, bufs[1 - cur], C * P, None, 0, False, tiles=T)
+            cur = 1 - cur
+            rows += T
+        return bufs[cur], rows
+
+    def _transform_level_unfused(self, flows, slots, src, src_bs: int, B: int, C: int, h: int, w: int, ld_part,
+                                 row: int):
+        """Squeeze, then per StepFlow the separate K-A / im2col / GEMMs / coupling kernels.  A step of a model that is not
+        ready initialises its ActNorm from this batch first, then runs its LU/fold into its log-det slot (``slots[k]``).
+        Returns (state, log-det partial rows written)."""
+        P, T = h * w, N.ld_tiles(h * w)
+        a = torch.empty(B, C, h, w, dtype=torch.float32, device=src.device)
+        b = torch.empty_like(a)
+        N.squeeze(src, a, B, C // 4, 2 * h, 2 * w, src_bs, C * P)
+        for k, step in enumerate(flows):
+            step._forward_views(a, C * P, b, C * P, B, h, w, ld_part[(row + k * T) * B:], slots[k:k + 1])
+            a, b = b, a
+        return a, len(flows) * T
 
     # ---- inverse: latents -> x
     def invert(self, latents: list, temperature: float = 1.0, log_det_jac: Optional[Tensor] = None,
@@ -510,267 +512,110 @@ class Glow(Transform):
                                   log_det_jac, logp)
             return _NoBackward.apply(out, "Glow.invert", False, *deps)
         with_ld, with_lp = log_det_jac is not None, logp is not None
-        dev = z_last.device
-        levels = self._levels()
-        slots = self._slots(dev)
-        steps = [s for flows, _ in levels for s in flows]
-        ready = all(s._ready() for s in steps)
+        ready = self._ready()
         H, W = h << self.L, w << self.L
         if self._use_graph(ready) and 1 <= len(latents) <= self.L and all(isinstance(t, Tensor) for t in latents):
             # decoding (all L latents supplied) and sampling (fewer: every Split without a latent draws its half from the
             # learned conditional prior, transforms.py:305-307) replay one captured chain; the normal draws inside a
             # captured chain come from torch's default CUDA generator, whose Philox offset advances on every replay
             lat_in = [E.check_input(t, "latent") for t in latents]
-            if self._params_changed():
-                self._refresh_caches(steps, slots)
             sampling = len(latents) < self.L
-            key = ("inv", B, h, w, E.precision(), dev.index)
+            key = ("inv", B, h, w, E.precision(), z_last.device.index)
             if sampling:
                 key += (len(latents), float(temperature))
             if with_ld or with_lp:                    # a chain that also writes the density partials
                 key += ((with_ld, with_lp),)
-            ent = self._graphs.get(key)
-            if ent is None and sampling:
+            if key not in self._graphs and sampling:
                 # the temperature is baked into a sampling graph: keep at most four of them (a temperature sweep would
                 # otherwise pin one captured chain and its workspace per value)
                 old = [k for k in self._graphs if k[0] == "inv" and len(k) >= 8]
                 for k in old[:max(0, len(old) - 3)]:
                     E.WS.drop_scope(("glow", id(self), k))
                     del self._graphs[k]
-            statics = ent["lat"] if ent is not None else [torch.empty_like(t) for t in lat_in]
-            for s_, t in zip(statics, lat_in):
-                if s_.shape != t.shape:
-                    raise ValueError(f"latent has shape {tuple(t.shape)}, expected {tuple(s_.shape)}")
-                s_.copy_(t)
-
-            nsub = self._n_sub(B)
-            Bs = B // nsub
-
-            def build():
-                outs = self._fork_join(nsub, lambda i: self._invert_core(
-                    [t[i * Bs:(i + 1) * Bs] for t in statics], temperature, levels, slots, steps, True, with_ld, with_lp))
-                return {"lat": statics, "outs": outs}
-            ent = self._graph_entry(key, build)
-            if ent["lat"] is not statics:
-                for s_, t in zip(ent["lat"], lat_in):
-                    s_.copy_(t)
-            ent["graph"].replay()
-            N.launch_count += ent["n_launch"]
-            outs = ent["outs"]
-            for i, (_, ld_part, R_ld, lp_part, R_lp) in enumerate(outs):     # after the replay, into the caller's tensors
-                sl = slice(i * Bs, (i + 1) * Bs)
-                self._add_density(log_det_jac[sl] if with_ld else None, logp[sl] if with_lp else None, ld_part, R_ld,
-                                  lp_part, R_lp, Bs, H, W, slots)
-            return torch.cat([o[0] for o in outs]) if nsub > 1 else outs[0][0].clone()
-        x, ld_part, R_ld, lp_part, R_lp = self._invert_core(latents, temperature, levels, slots, steps, ready, with_ld,
-                                                            with_lp)
-        self._add_density(log_det_jac, logp, ld_part, R_ld, lp_part, R_lp, B, H, W, slots)
+            x, parts = self._replay(key, lat_in, lambda lat: self._invert_walk(lat, temperature, True, with_ld, with_lp))
+            self._add_density(log_det_jac, logp, parts, H, W)     # after the replay, into the caller's tensors
+            return x.clone()
+        x, parts = self._invert_walk(latents, temperature, ready, with_ld, with_lp)
+        self._add_density(log_det_jac, logp, parts, H, W)
         return x
 
-    def _add_density(self, log_det_jac, logp, ld_part, R_ld: int, lp_part, R_lp: int, B: int, H: int, W: int,
-                     slots: Tensor) -> None:
-        """The final accumulates of an inverse, as ``transform`` runs them: the log-det partial rows plus the L*K
-        data-independent constants, and the Split log-prob rows."""
-        if log_det_jac is not None:
-            N.accumulate(log_det_jac, ld_part, R_ld, B, slots, self._multipliers(H, W, slots.device), self.L * self.K)
-        if logp is not None and R_lp > 0:
-            N.accumulate(logp, lp_part, R_lp, B)
-
-    def _part_rows(self, B: int, H: int, W: int, inverse: bool = False, fused: bool = True) -> Tuple[int, int]:
-        """Rows of B per-image partials that one call writes for [B, c, H, W] images: (log-det rows, Split log-prob rows).
-        Log-det: one per step at "image" levels, ld_tiles(P) per step at unfused ones, one per band at "tiled" levels, where
-        K-1 boundaries carry an im2col sink and the level's last one does not (and has a mix in the inverse only, which can
-        change the band height).  ``fused=False``: every level unfused (NFDPM_FUSED_BOUNDARY=0, or a model not ready)."""
-        R_ld = R_lp = 0
-        hh, ww, cc = H, W, self.in_channel
-        for li in range(self.L):
-            hh, ww, CC = hh // 2, ww // 2, cc * 4
-            mode = self._level_mode(B, CC, hh, ww) if fused else "unfused"
-            if mode == "tiled":
-                R_ld += (self.K - 1) * N.flow_boundary_tiles(B, CC, hh, ww, 1, 1, 1) + \
-                    N.flow_boundary_tiles(B, CC, hh, ww, 1, int(inverse), 0)
-            else:
-                R_ld += self.K * (1 if mode == "image" else N.ld_tiles(hh * ww))
-            if li < self.L - 1:
-                R_lp += N.ld_tiles(hh * ww)
-            cc = CC // 2
-        return R_ld, R_lp
-
-    def _transform_fast(self, x: Tensor, with_logp: bool, levels, slots, steps):
-        """Forward with the fused step-boundary kernel: 4 launches per StepFlow (boundary + 3 GEMMs)."""
-        B, c, H, W = x.shape
-        dev = x.device
-        E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
-        R_ld, R_lp = self._part_rows(B, H, W)
-        ld_part = E.WS.get("ld_part", R_ld * B, torch.float32, dev)
-        lp_part = E.WS.get("lp_part", max(R_lp, 1) * B, torch.float32, dev) if with_logp else None
-        latents: List[Tensor] = []
-        cur, cur_bs = x, c * H * W
-        h, w, ch = H, W, c
-        row = lrow = 0
-        for li, (flows, split) in enumerate(levels):
-            h, w, C = h // 2, w // 2, ch * 4
-            P = h * w
-            mode = self._level_mode(B, C, h, w)
-            if mode == "tiled":
-                st, rows = self._transform_level_tiled(flows, cur, cur_bs, B, C, h, w, ld_part, row, dev)
-                row += rows
-                if split is None:
-                    latents.append(st)
-                    break
-                z = torch.empty(B, C // 2, h, w, dtype=torch.float32, device=dev)
-                split._forward_views(st, C * P, B, C, h, w, z, lp_part[lrow * B:] if lp_part is not None else None)
-                lrow += N.ld_tiles(P)
-                latents.append(z)
-                cur, cur_bs, ch = st, C * P, C // 2
-                continue
-            if mode == "unfused":
-                # NFDPM_TILED=0: squeeze + unfused K-A / im2col / GEMMs / coupling per step
-                T = N.ld_tiles(P)
-                a = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-                b = torch.empty_like(a)
-                N.squeeze(cur, a, B, ch, 2 * h, 2 * w, cur_bs, C * P)
-                for step in flows:
-                    step._forward_views(a, C * P, b, C * P, B, h, w, ld_part[row * B:], None)
-                    a, b = b, a
-                    row += T
-                st = a
-                if split is None:
-                    latents.append(st)
-                    break
-                z = torch.empty(B, C // 2, h, w, dtype=torch.float32, device=dev)
-                split._forward_views(st, C * P, B, C, h, w, z, lp_part[lrow * B:] if lp_part is not None else None)
-                lrow += T
-                latents.append(z)
-                cur, cur_bs, ch = st, C * P, C // 2
-                continue
-            st = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)     # flow state of this level (in place)
-            nsub = self._deep_sub(B, h, w) if torch.cuda.is_current_stream_capturing() else 1
-            Bs = B // nsub
-            row0 = row
-
-            def level_chain(i, cur=cur, cur_bs=cur_bs, st=st, flows=flows, C=C, h=h, w=w, P=P, Bs=Bs, row0=row0):
-                """The K StepFlows of this level for images [i*Bs, (i+1)*Bs): views of the level's tensors."""
-                src_i, st_i = cur[i * Bs:(i + 1) * Bs], st[i * Bs:(i + 1) * Bs]
-                first = flows[0]
-                A1, K1p = E.coupling_a1(first.affcoupling, Bs, C, h, w, dev)
-                # level entry: squeeze + K-A of step 0 + im2col
-                N.flow_boundary(src_i, cur_bs, True, None, 0, None, None, None, first._mix.fwd_mt, first._mix.fwd_beta,
-                                st_i, C * P, A1, K1p, Bs, C, h, w, False)
-                r = row0
-                for k, step in enumerate(flows):
-                    cp = step.affcoupling
-                    nxt = flows[k + 1] if k + 1 < len(flows) else None
-                    part = ld_part[r * B + i * Bs:]
-                    if nxt is not None:
-                        A1n, K1p = E.coupling_a1(nxt.affcoupling, Bs, C, h, w, dev)     # same scratch buffer as A1
-                        E.coupling_boundary(cp, A1, Bs, C, h, w, st_i, C * P, part, nxt._mix.fwd_mt,
-                                            nxt._mix.fwd_beta, st_i, C * P, A1n, K1p, False)
-                        A1 = A1n
-                    else:
-                        E.coupling_boundary(cp, A1, Bs, C, h, w, st_i, C * P, part, None, None, st_i, C * P,
-                                            None, 0, False)
-                    r += 1
-            self._fork_join(nsub, level_chain, pool="_deep_streams")
-            row += len(flows)
-            if split is None:
-                latents.append(st)
-                break
-            z = torch.empty(B, C // 2, h, w, dtype=torch.float32, device=dev)
-            split._forward_views(st, C * P, B, C, h, w, z, lp_part[lrow * B:] if lp_part is not None else None)
-            lrow += N.ld_tiles(P)
-            latents.append(z)
-            cur, cur_bs, ch = st, C * P, C // 2
-        return latents, ld_part, R_ld, lp_part, (R_lp if with_logp else 0)
-
-    def _density_parts(self, B: int, H: int, W: int, dev, with_ld: bool, with_lp: bool, fused: bool):
-        """Partial buffers of one inverse that also returns its density (None where not requested), with their row
-        counts: the rows the forward writes (`_part_rows`)."""
-        R_ld, R_lp = self._part_rows(B, H, W, inverse=True, fused=fused)
-        ld_part = E.WS.get("ld_part", R_ld * B, torch.float32, dev) if with_ld else None
-        lp_part = E.WS.get("lp_part", max(R_lp, 1) * B, torch.float32, dev) if with_lp else None
-        return ld_part, R_ld, lp_part, R_lp
-
-    def _invert_fast(self, latents, temperature, levels, slots, steps, with_ld: bool = False, with_lp: bool = False):
-        """Inverse with the fused step-boundary kernel -> (x, ld_part, R_ld, lp_part, R_lp); the partials are written
-        only when requested (``with_ld`` / ``with_lp``), in level order from the deepest level."""
-        z_last = latents[-1]
-        B, C, h, w = z_last.shape
+    def _invert_walk(self, latents, temperature: float, ready: bool, with_ld: bool = False, with_lp: bool = False,
+                     level=None, eps_sink: Optional[list] = None):
+        """latents -> (x, (ld_part, R_ld, lp_part, R_lp)): the levels deepest first.  Each level runs its K inverse
+        StepFlows with the kernels of its `_level_mode` (as `_transform_walk`) and unsqueezes into the first half of the
+        previous level's state, whose Split fills the second half with the supplied latent or a draw from its conditional
+        prior.  The partials are written only when requested (``with_ld`` / ``with_lp``).
+        ``level(mode, flows, src, B, C, h, w) -> state`` replaces the no-grad kernels of a level (the recorded inverse keeps
+        the operands of every step); ``eps_sink`` receives (assembled Split state, eps of its draw or None) per Split."""
+        z_last = E.check_input(latents[-1], "latents[-1]")
+        B, _, h, w = z_last.shape
+        H, W = h << self.L, w << self.L
         dev = z_last.device
-        E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
-        ld_part, R_ld, lp_part, R_lp = self._density_parts(B, h << self.L, w << self.L, dev, with_ld, with_lp, True)
-        src = z_last                                   # caller memory: read only
+        fused = ready and E.fused_boundary_enabled()
+        if ready or with_ld:
+            # (the inverse initialises no StepFlow ActNorm, so the log-det constants of a model that is not ready are
+            # final here too)
+            self._prepare_mix(dev)
+        parts = ld_part, R_ld, lp_part, R_lp = self._density_parts(B, H, W, dev, True, fused, with_ld, with_lp)
+        run = {"image": self._invert_level_image, "tiled": self._invert_level_tiled,
+               "unfused": self._invert_level_unfused}
+        geo = self._geometry(H, W)
+        st = z_last
         row = lrow = 0
         for li in range(self.L - 1, -1, -1):
-            flows, _ = levels[li]
-            P = h * w
-            mode = self._level_mode(B, C, h, w)
-            if mode == "tiled":
-                st, rows = self._invert_level_tiled(flows, src, B, C, h, w, dev, ld_part, row)
+            flows, _, C, h, w = geo[li]
+            mode = self._level_mode(B, C, h, w) if fused else "unfused"
+            if level is None:          # (the deepest level's input is caller memory: `own` False, only read)
+                st, rows = run[mode](flows, st, li < self.L - 1, B, C, h, w, ld_part, row)
                 row += rows
-            elif mode == "unfused":
-                # NFDPM_TILED=0: unfused inverse steps (coupling^-1 in place, then K-A^-1)
-                cur, own = src, li < self.L - 1        # the deepest level reads caller memory
-                other = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-                for step in reversed(flows):
-                    part = ld_part[row * B:] if ld_part is not None else None
-                    if own:
-                        step._inverse_views(cur, C * P, cur, C * P, other, C * P, B, h, w, part)
-                        cur, other = other, cur
-                    else:
-                        tmp = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-                        step._inverse_views(cur, C * P, tmp, C * P, other, C * P, B, h, w, part)
-                        cur, other, own = other, tmp, True
-                    row += N.ld_tiles(P)
-                st = cur
             else:
-                st = self._invert_level_fast(flows, src, li < self.L - 1, B, C, h, w, dev, ld_part, row)
-                row += len(flows)
-            if li == 0:
-                out = torch.empty(B, C // 4, h * 2, w * 2, dtype=torch.float32, device=dev)
-                N.unsqueeze(st, out, B, C, h, w, C * P, (C // 4) * P * 4)
-                return out, ld_part, R_ld, lp_part, R_lp
-            Cn, hn, wn = 2 * (C // 4), h * 2, w * 2
-            nxt = torch.empty(B, Cn, hn, wn, dtype=torch.float32, device=dev)
-            N.unsqueeze(st, nxt, B, C, h, w, C * P, Cn * hn * wn)
-            latent = get_item(latents, -(self.L - li + 1))
-            levels[li - 1][1]._fill_second_half(nxt, Cn * hn * wn, B, Cn, hn, wn, latent, temperature,
-                                                logp_part=lp_part[lrow * B:] if lp_part is not None else None)
-            lrow += N.ld_tiles(hn * wn)
-            src, C, h, w = nxt, Cn, hn, wn
-        raise AssertionError("unreachable")
+                st = level(mode, flows, st, B, C, h, w)
+            # undo the squeeze of this level into the first half of the previous level's state (the image at level 0)
+            Cn = C // 4 if li == 0 else C // 2
+            nxt = torch.empty(B, Cn, 2 * h, 2 * w, dtype=torch.float32, device=dev)
+            N.unsqueeze(st, nxt, B, C, h, w, C * h * w, Cn * 4 * h * w)
+            st = nxt
+            if li > 0:
+                drawn = [] if eps_sink is not None else None
+                geo[li - 1][1]._fill_second_half(nxt, Cn * 4 * h * w, B, Cn, 2 * h, 2 * w,
+                                                 get_item(latents, li - self.L - 1), temperature, eps_sink=drawn,
+                                                 logp_part=lp_part[lrow * B:] if lp_part is not None else None)
+                lrow += N.ld_tiles(4 * h * w)
+                if eps_sink is not None:
+                    eps_sink.append((nxt, drawn[0] if drawn else None))
+        assert lrow == R_lp and (row == R_ld or level is not None), \
+            f"wrote {row} / {lrow} partial rows, allotted {R_ld} / {R_lp}"
+        return st, parts
 
-    def _transform_level_tiled(self, flows, cur, cur_bs: int, B: int, C: int, h: int, w: int, ld_part, row: int, dev):
-        """K forward StepFlows of one level with the row-band boundary kernel.  A band reads halo rows that a neighbouring
-        band writes, so the flow state ping-pongs between two buffers.  Returns (state, log-det partial rows used)."""
-        P = h * w
-        bufs = [torch.empty(B, C, h, w, dtype=torch.float32, device=dev) for _ in range(2)]
-        first = flows[0]
-        A1, K1p = E.coupling_a1(first.affcoupling, B, C, h, w, dev)
-        N.flow_boundary_tiled(cur, cur_bs, True, None, 0, None, None, None, first._mix.fwd_mt, first._mix.fwd_beta,
-                              bufs[0], C * P, None, 0, A1, K1p, B, C, h, w, False,
-                              N.flow_boundary_tiles(B, C, h, w, 0, 1, 1))       # level entry: squeeze + K-A + im2col
-        src, rows = 0, 0
-        for k, step in enumerate(flows):
-            nxt = flows[k + 1] if k + 1 < len(flows) else None
-            T = N.flow_boundary_tiles(B, C, h, w, 1, int(nxt is not None), int(nxt is not None))
-            if nxt is not None:
-                A1n, K1p = E.coupling_a1(nxt.affcoupling, B, C, h, w, dev)
-                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, bufs[src], C * P, ld_part[(row + rows) * B:],
-                                    nxt._mix.fwd_mt, nxt._mix.fwd_beta, bufs[1 - src], C * P, A1n, K1p, False, tiles=T)
+    def _invert_level_image(self, flows, src, own: bool, B: int, C: int, h: int, w: int, ld_part, row: int):
+        """K inverse StepFlows with one CTA per image, in place on the level's state (on a copy when `src` is caller memory,
+        ``own`` False).  Step k writes its log-det partial to row `row + k` of `ld_part` when given.  Returns (state,
+        rows)."""
+        P, dev = h * w, src.device
+        st = src if own else torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
+        last = flows[-1]
+        A1, K1p = E.coupling_a1(last.affcoupling, B, C, h, w, dev)
+        N.flow_boundary(src, C * P, False, None, 0, None, None, None, None, None, None, 0, A1, K1p, B, C, h, w,
+                        False)                         # im2col of the level's entry state
+        for k in range(len(flows) - 1, -1, -1):
+            step = flows[k]
+            cp = step.affcoupling
+            part = ld_part[(row + k) * B:] if ld_part is not None else None
+            if k > 0:
+                A1n, K1p = E.coupling_a1(flows[k - 1].affcoupling, B, C, h, w, dev)
+                E.coupling_boundary(cp, A1, B, C, h, w, src, C * P, part, step._mix.inv_mt, step._mix.inv_beta,
+                                    st, C * P, A1n, K1p, True)
                 A1 = A1n
             else:
-                E.coupling_boundary(step.affcoupling, A1, B, C, h, w, bufs[src], C * P, ld_part[(row + rows) * B:],
-                                    None, None, bufs[1 - src], C * P, None, 0, False, tiles=T)
-            src = 1 - src
-            rows += T
-        return bufs[src], rows
+                E.coupling_boundary(cp, A1, B, C, h, w, src, C * P, part, step._mix.inv_mt, step._mix.inv_beta,
+                                    st, C * P, None, 0, True)
+            src = st
+        return st, len(flows)
 
-    def _invert_level_tiled(self, flows, src, B: int, C: int, h: int, w: int, dev, ld_part=None, row: int = 0):
+    def _invert_level_tiled(self, flows, src, own: bool, B: int, C: int, h: int, w: int, ld_part, row: int):
         """K inverse StepFlows of one level with the row-band boundary kernel (state ping-pongs between two buffers;
-        `src` — caller memory or the previous level's output — is only read).  Returns (state, log-det partial rows used
-        from `row` on; written only when `ld_part` is given)."""
-        P = h * w
+        `src` is only read).  Returns (state, log-det partial rows from `row` on; written only when `ld_part` is given)."""
+        P, dev = h * w, src.device
         rows = 0
         bufs = [torch.empty(B, C, h, w, dtype=torch.float32, device=dev) for _ in range(2)]
         A1, K1p = E.coupling_a1(flows[-1].affcoupling, B, C, h, w, dev)
@@ -793,83 +638,21 @@ class Glow(Transform):
             rows += T
         return cur, rows
 
-    def _invert_level_fast(self, flows, src, own: bool, B: int, C: int, h: int, w: int, dev, ld_part=None,
-                           row: int = 0) -> Tensor:
-        """K inverse StepFlows of one level with the fused kernels; returns the level's input state.  Deep levels run as
-        concurrent sub-batches inside a captured graph (`_deep_sub`).  Step k writes its log-det partial to row `row + k`
-        of `ld_part` when given."""
-        P = h * w
-        st = src if own else torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-        nsub = self._deep_sub(B, h, w) if torch.cuda.is_current_stream_capturing() else 1
-        Bs = B // nsub
-
-        def level_chain(i):
-            src_i, st_i = src[i * Bs:(i + 1) * Bs], st[i * Bs:(i + 1) * Bs]
-            last = flows[-1]
-            A1, K1p = E.coupling_a1(last.affcoupling, Bs, C, h, w, dev)
-            N.flow_boundary(src_i, C * P, False, None, 0, None, None, None, None, None, None, 0, A1, K1p, Bs, C, h, w,
-                            False)                     # im2col of the level's entry state
-            for k in range(len(flows) - 1, -1, -1):
-                step = flows[k]
-                cp = step.affcoupling
-                part = ld_part[(row + k) * B + i * Bs:] if ld_part is not None else None
-                if k > 0:
-                    A1n, K1p = E.coupling_a1(flows[k - 1].affcoupling, Bs, C, h, w, dev)
-                    E.coupling_boundary(cp, A1, Bs, C, h, w, src_i, C * P, part, step._mix.inv_mt, step._mix.inv_beta,
-                                        st_i, C * P, A1n, K1p, True)
-                    A1 = A1n
-                else:
-                    E.coupling_boundary(cp, A1, Bs, C, h, w, src_i, C * P, part, step._mix.inv_mt, step._mix.inv_beta,
-                                        st_i, C * P, None, 0, True)
-                src_i = st_i
-        self._fork_join(nsub, level_chain, pool="_deep_streams")
-        return st
-
-    def _invert_core(self, latents, temperature, levels, slots, steps, ready: bool, with_ld: bool = False,
-                     with_lp: bool = False):
-        """-> (x, ld_part, R_ld, lp_part, R_lp), as `_invert_fast`."""
-        z_last = E.check_input(latents[-1], "latents[-1]")
-        B, Cf, h, w = z_last.shape
-        dev = z_last.device
-        if ready and self._fast_ok(h * 2 ** self.L, w * 2 ** self.L):
-            return self._invert_fast([z_last] if len(latents) == 1 else list(latents), temperature, levels, slots, steps,
-                                     with_ld, with_lp)
-        if ready or with_ld:
-            # (the inverse initialises no StepFlow ActNorm, so the log-det constants of a model that is not ready are
-            # final here too)
-            E.prepare_mix([s._mix_entry(slots[i:i + 1]) for i, s in enumerate(steps)])
-        ld_part, R_ld, lp_part, R_lp = self._density_parts(B, h << self.L, w << self.L, dev, with_ld, with_lp, False)
-        C, P = Cf, h * w
-        cur = z_last
-        own = False          # `cur` is caller memory until the first step has produced a copy
-        row = lrow = 0
-        for li in range(self.L - 1, -1, -1):
-            flows, _ = levels[li]
-            other = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-            for step in reversed(flows):
-                part = ld_part[row * B:] if ld_part is not None else None
-                if own:
-                    step._inverse_views(cur, C * P, cur, C * P, other, C * P, B, h, w, part)
-                    cur, other = other, cur
-                else:
-                    tmp = torch.empty(B, C, h, w, dtype=torch.float32, device=dev)
-                    step._inverse_views(cur, C * P, tmp, C * P, other, C * P, B, h, w, part)
-                    cur, other, own = other, tmp, True
-                row += N.ld_tiles(P)
-            # undo the squeeze of this level into the first half of the previous level's tensor
-            if li == 0:
-                out = torch.empty(B, C // 4, h * 2, w * 2, dtype=torch.float32, device=dev)
-                N.unsqueeze(cur, out, B, C, h, w, C * P, (C // 4) * P * 4)
-                return out, ld_part, R_ld, lp_part, R_lp
-            Cn, hn, wn = 2 * (C // 4), h * 2, w * 2
-            nxt = torch.empty(B, Cn, hn, wn, dtype=torch.float32, device=dev)
-            N.unsqueeze(cur, nxt, B, C, h, w, C * P, Cn * hn * wn)
-            latent = get_item(latents, -(self.L - li + 1))   # None -> draw from the conditional prior
-            levels[li - 1][1]._fill_second_half(nxt, Cn * hn * wn, B, Cn, hn, wn, latent, temperature,
-                                                logp_part=lp_part[lrow * B:] if lp_part is not None else None)
-            lrow += N.ld_tiles(hn * wn)
-            cur, own, C, h, w, P = nxt, True, Cn, hn, wn, hn * wn
-        raise AssertionError("unreachable")
+    def _invert_level_unfused(self, flows, src, own: bool, B: int, C: int, h: int, w: int, ld_part, row: int):
+        """K inverse StepFlows with the separate kernels: coupling^-1 in place, then K-A^-1 into the other buffer (caller
+        memory, ``own`` False, is only read).  Returns (state, log-det partial rows from `row` on)."""
+        P, T = h * w, N.ld_tiles(h * w)
+        cur, other = src, torch.empty(B, C, h, w, dtype=torch.float32, device=src.device)
+        for k, step in enumerate(reversed(flows)):
+            part = ld_part[(row + k * T) * B:] if ld_part is not None else None
+            if own:
+                step._inverse_views(cur, C * P, cur, C * P, other, C * P, B, h, w, part)
+                cur, other = other, cur
+            else:
+                tmp = torch.empty(B, C, h, w, dtype=torch.float32, device=src.device)
+                step._inverse_views(cur, C * P, tmp, C * P, other, C * P, B, h, w, part)
+                cur, other, own = other, tmp, True
+        return cur, len(flows) * T
 
     @torch.no_grad()
     def sample(self, latents: list, postprocess_func=None, temperature: float = 1.0,

@@ -5,7 +5,7 @@ Kernel level: every inverse-mode step boundary writes the forward's log-det part
 half) and its other outputs do not change with the sink.  Model level, against the CPU oracle's transform of the oracle's
 inverse (north-star bar: log-det / log-p relative <= 1e-4, bits/dim |d| <= 1e-3) and against this package's own transform:
 decoding at config 2 with the weight sets of test_gpu_benchmarked_path.py, sampling at three temperatures, every inverse
-path (one CTA per image, row bands, unfused, eager, replayed graphs, sub-batch streams, a model that is not ready), the
+path (one CTA per image, row bands, unfused, eager, replayed graphs, a model that is not ready), the
 bf16 mode at its stated tolerance, and the call contract."""
 import numpy as np
 import pytest
@@ -23,7 +23,7 @@ DEV = torch.device("cuda")
 
 @pytest.fixture(autouse=True)
 def _no_grad_default_mode(monkeypatch):
-    for k in ("NFDPM_PRECISION", "NFDPM_TILED", "NFDPM_STREAMS", "NFDPM_DEEP_STREAMS", "NFDPM_INVERT_GRAD"):
+    for k in ("NFDPM_PRECISION", "NFDPM_TILED", "NFDPM_INVERT_GRAD"):
         monkeypatch.delenv(k, raising=False)
     monkeypatch.setenv("NFDPM_GRAPHS", "1")
     monkeypatch.setenv("NFDPM_FUSED_BOUNDARY", "1")
@@ -239,15 +239,13 @@ def _paths_model(B):
     return bench_style_model(3, 3, 16, B, 32, 5e-3)
 
 
-@pytest.mark.parametrize("path", ["graph", "eager", "unfused", "unfused_eager", "tiled", "streams"])
+@pytest.mark.parametrize("path", ["graph", "eager", "unfused", "unfused_eager", "tiled"])
 def test_every_inverse_path_agrees(path, monkeypatch):
     """Config-2 geometry through each inverse path: captured and replayed (image mode), eager (NFDPM_GRAPHS=0), unfused
-    (NFDPM_FUSED_BOUNDARY=0 and NFDPM_TILED=0, captured and eager), row bands (a small batch), and concurrent sub-batches
-    (NFDPM_STREAMS=2, NFDPM_DEEP_STREAMS=2:2)."""
+    (NFDPM_FUSED_BOUNDARY=0 and NFDPM_TILED=0, captured and eager) and row bands (a small batch)."""
     B = 16 if path == "tiled" else 128
     env = {"eager": {"NFDPM_GRAPHS": "0"}, "unfused": {"NFDPM_FUSED_BOUNDARY": "0", "NFDPM_TILED": "0"},
-           "unfused_eager": {"NFDPM_FUSED_BOUNDARY": "0", "NFDPM_TILED": "0", "NFDPM_GRAPHS": "0"},
-           "streams": {"NFDPM_STREAMS": "2", "NFDPM_DEEP_STREAMS": "2:2"}}.get(path, {})
+           "unfused_eager": {"NFDPM_FUSED_BOUNDARY": "0", "NFDPM_TILED": "0", "NFDPM_GRAPHS": "0"}}.get(path, {})
     flow, prior, sd, psd, x = _paths_model(B)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
@@ -286,7 +284,7 @@ def test_config4_row_bands_and_image_mode(monkeypatch):
 
 
 def test_not_ready_model_eager_path():
-    """A model whose StepFlow ActNorms are not initialised inverts through the eager unfused chain (`_invert_core`); the
+    """A model whose StepFlow ActNorms are not initialised inverts through the eager unfused chain (`_invert_walk`); the
     density it returns is that of the model as it stands (the inverse initialises no StepFlow ActNorm)."""
     c, L, K, B, S = 3, 3, 2, 4, 32
     sd, psd = O.seeded_state(c, L, K, 3)

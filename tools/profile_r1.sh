@@ -1,7 +1,6 @@
 #!/bin/bash
 # Round-1 profiling recipe (run under gpurun): plain runs first, then the ncu launch lists and --set full captures.
 set -x
-export NFDPM_STREAMS=1
 OUT=gpurun_out
 python tools/train_steps.py 3 > $OUT/plain_train.log 2>&1 || exit 1
 NFDPM_GRAPHS=0 python bench.py --steps 2 --warmup 3 --no-train --no-cpu-baseline > $OUT/plain_bench_eager.log 2>&1 || exit 1
