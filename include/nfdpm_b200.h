@@ -202,6 +202,13 @@ int nfdpm_flow_boundary_inv_stash(const float* in, int64_t in_bs, const float* p
                                   const float* logs3, const float* mt, const float* beta, float* y, int64_t y_bs, float* xs,
                                   int64_t xs_bs, void* a1, int a1_dtype, int64_t lda1, int B, int C, int H, int W,
                                   nfdpm_stream_t stream);
+/* nfdpm_flow_boundary_inv_stash with a log-det sink: ld_part [B] (may be NULL) receives each image's sum of log(s + 1e-6),
+ * the partial nfdpm_flow_boundary writes in inverse mode (same arithmetic and reduction order).  The density of a
+ * recorded Glow.invert. */
+int nfdpm_flow_boundary_inv_stash_ld(const float* in, int64_t in_bs, const float* pm, int64_t ldp, const float* bias3,
+                                     const float* logs3, float* ld_part, const float* mt, const float* beta, float* y,
+                                     int64_t y_bs, float* xs, int64_t xs_bs, void* a1, int a1_dtype, int64_t lda1, int B,
+                                     int C, int H, int W, nfdpm_stream_t stream);
 
 /* ZeroConv GEMM + step boundary in ONE launch (tensor-core mode): pm = h2[M,K] * w3p[ldp,K]^T is accumulated in tensor
  * memory, staged in shared memory and consumed by the arithmetic of nfdpm_flow_boundary (coupling source), so the
@@ -255,6 +262,12 @@ int nfdpm_coupling_inv_bwd(const float* dx, int64_t dx_bs, const float* y, int64
                            const float* bias3, const float* logs3, float* dy, int64_t dy_bs, void* dpm, int dpm_dtype,
                            int64_t ld_dpm, float* dpar, float* dbias, float* dlogs, int32_t* counter, float* dp_scratch,
                            int B, int C, int H, int W, nfdpm_stream_t stream);
+/* nfdpm_coupling_inv_bwd plus the gradient of the log-det the inverse accumulates, sum log(s+1e-6): dld [B] (may be NULL:
+ * identical to nfdpm_coupling_inv_bwd) adds dld/(s+1e-6) to ds, the forward's term of nfdpm_coupling_bwd. */
+int nfdpm_coupling_inv_bwd_ld(const float* dx, int64_t dx_bs, const float* dld, const float* y, int64_t y_bs,
+                              const float* pm, int64_t ldp, const float* bias3, const float* logs3, float* dy, int64_t dy_bs,
+                              void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias, float* dlogs,
+                              int32_t* counter, float* dp_scratch, int B, int C, int H, int W, nfdpm_stream_t stream);
 /* ActNorm+ReLU backward on rows (utils.py:69,84-87): dpre = dh*(h>0)*exp(scale); part[cta][2N] partial d(scale), d(bias);
  * ctas = ceil(M/rows_per_cta).  dtypes: any mix of F32 / BF16, or the fp32-faithful form (F32 dh, BF16X2 h) -> BF16X2 dpre. */
 int nfdpm_actnorm_relu_bwd(const void* dh, int dh_dtype, int64_t ld_dh, const void* h, int h_dtype, int64_t ld_h,
@@ -284,7 +297,9 @@ int nfdpm_mix_param_grad(const nfdpm_mix_grad_item* items_host, int n, nfdpm_str
 /* Parameter gradients of the INVERSE mix x = M u - b, M = diag(e^-s) W^-1 (transforms.py:92-94,142-145), from the
  * partials of an nfdpm_mix_bwd run with mt = inv_mt (its x = the inverse input u, its du = grad wrt the output x):
  * d_bias = -g, d_scale_c = -sum_j G_cj M_cj, d_weight = -W^-T diag(e^-s) G W^-T.  weight may be NULL; winv is W^-1 (the
- * identity for a lone ActNorm); dld_sum and P are unused; any of d_weight / d_scale / d_bias may be NULL. */
+ * identity for a lone ActNorm); any of d_weight / d_scale / d_bias may be NULL.  dld_sum (may be NULL: no log-det term)
+ * is sum_b d(ld)[b] for the constant P*(sum s + log|det W|) the inverse accumulates: it adds P*dld_sum*W^-T to d_weight
+ * and P*dld_sum to d_scale. */
 int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items_host, int n, nfdpm_stream_t stream);
 /* Weight gradients: D[N1,N2] (+)= sum_m A[m,N1]*B[m,N2] (A, B row-major, F32, BF16 or both BF16X2; D fp32 with ldd == N2).
  * Split pairs (needs counters): the tensor-core accumulator holds hi*hi, hi*lo, lo*hi, lo*lo of every logical element and the
@@ -316,6 +331,12 @@ int nfdpm_gauss_const_bwd(const float* dl, const float* z, const float* bias, co
 int nfdpm_split_sample_bwd(const float* dz, int64_t dz_bs, const float* eps, float temperature, const float* h, int64_t ldh,
                            const float* bias, const float* logs, float* dh, float* dpar, int B, int C, int H, int W,
                            nfdpm_stream_t stream);
+/* nfdpm_split_sample_bwd plus the gradient of the draw's log-density sum -(log 2pi + 2 lg + T^2 eps^2)/2 (the logp term of
+ * a sampled Split in Glow.invert): d lg -= dlp[b] per element, nothing on the mean.  dlp [B] may be NULL (identical to
+ * nfdpm_split_sample_bwd). */
+int nfdpm_split_sample_bwd_lp(const float* dz, int64_t dz_bs, const float* dlp, const float* eps, float temperature,
+                              const float* h, int64_t ldh, const float* bias, const float* logs, float* dh, float* dpar,
+                              int B, int C, int H, int W, nfdpm_stream_t stream);
 /* dstate[b,c,p] += col2im(da)[b,c,p] for c < Cin (input gradient of a 3x3 "same" conv expressed as im2col rows). */
 int nfdpm_col2im_add(const float* da, int64_t lda, float* dstate, int64_t dbs, int B, int Cin, int H, int W,
                      nfdpm_stream_t stream);

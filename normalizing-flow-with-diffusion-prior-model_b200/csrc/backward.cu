@@ -106,8 +106,9 @@ __host__ __device__ __forceinline__ size_t coupling_bwd_floats(int C, int H, int
 // One CTA per image.  Same structure as the forward step boundary (boundary_body.cuh): the image's pm block arrives by
 // bulk copy while the gradients are staged; index divisions are multiply-high; the dpm rows (the transposed-conv scatter
 // dpm[p, tap*C+co] = dP[co][p - shift(tap)]) are gathered from a zero-bordered copy of dP through a column table.
-// INV: backward of the inverse x_b = y_b/(s+1e-6) - t (a.u = the inverse's input y, a.dy = grad wrt its output x; no
-// log-det term): du_b = dx_b/(s+eps), ds = -dx_b*y_b/(s+eps)^2, dt = -dx_b.
+// INV: backward of the inverse x_b = y_b/(s+1e-6) - t (a.u = the inverse's input y, a.dy = grad wrt its output x):
+// du_b = dx_b/(s+eps), ds = -dx_b*y_b/(s+eps)^2 (+ dld/(s+eps) when dld is given: the inverse accumulates the same
+// sum log(s+eps) as the forward), dt = -dx_b.
 template <typename TD, bool INV>
 __global__ void __launch_bounds__(1024) coupling_bwd_kernel(const CouplingBwdArgs a) {
   extern __shared__ __align__(128) float sm_raw[];
@@ -203,6 +204,7 @@ __global__ void __launch_bounds__(1024) coupling_bwd_kernel(const CouplingBwdArg
       const float r = 1.f / (s + 1e-6f);
       dub = dyv * r;
       ds = -dub * ub_s[j * PS + p] * r;
+      if (a.dld != nullptr) ds += gld / (s + 1e-6f);   // the inverse's log-det term: the forward's, from the same s
       dt = -dyv;
     } else {
       ds = dyv * (ub_s[j * PS + p] + t) + gld / (s + 1e-6f);
@@ -370,6 +372,7 @@ __global__ void __launch_bounds__(256) coupling_bwd_tiled_kernel(const CouplingB
       const float r = 1.f / (s + 1e-6f);
       duv = dyv * r;
       ds = -duv * ub[(int64_t)(Ch + j) * P + p] * r;
+      if (a.dld != nullptr) ds += gld / (s + 1e-6f);
       dt = -dyv;
     } else {
       ds = dyv * (ub[(int64_t)(Ch + j) * P + p] + tv) + gld / (s + 1e-6f);
@@ -711,8 +714,9 @@ __global__ void __launch_bounds__(256) mix_param_grad_kernel(const MixParamBatch
 }
 
 // The inverse mix x = M u - b, M = diag(e^-s) W^-1, from the partials of a mix_bwd run with mt = inv_mt (G = sum dx u^T,
-// g = sum dx):  db = -g,  ds_c = -sum_j G_cj M_cj,  dW = -W^-T (diag(e^-s) G) W^-T.  One CTA per StepFlow; shared memory
-// holds diag(e^-s) G W^-T [C][C].
+// g = sum dx):  db = -g,  ds_c = -sum_j G_cj M_cj,  dW = -W^-T (diag(e^-s) G) W^-T.  With dld_sum, the log-det constant
+// P*(sum s + log|det W|) that the inverse accumulates adds P*dld_sum to ds and P*dld_sum*W^-T to dW.  One CTA per
+// StepFlow; shared memory holds diag(e^-s) G W^-T [C][C].
 __global__ void __launch_bounds__(256) mix_inv_param_grad_kernel(const MixParamBatch batch) {
   extern __shared__ float t_s[];
   const MixParamItem it = batch.it[blockIdx.x];
@@ -721,12 +725,15 @@ __global__ void __launch_bounds__(256) mix_inv_param_grad_kernel(const MixParamB
   __syncthreads();
   const float* G = it.scratch;
   const float* g = it.scratch + C * C;
+  const float Gld = (it.dld_sum != nullptr) ? it.dld_sum[0] * it.P : 0.f;
   for (int c = tid; c < C; c += 256) {
     if (it.db) it.db[c] = -g[c];
     if (it.ds) {
       float acc = 0.f;
       for (int j = 0; j < C; ++j) acc = fmaf(G[c * C + j], it.winv[c * C + j], acc);
-      it.ds[c] = -expf(-it.s[c]) * acc;
+      float v = -expf(-it.s[c]) * acc;
+      if (it.dld_sum != nullptr) v += Gld;
+      it.ds[c] = v;
     }
   }
   if (it.dW == nullptr) return;
@@ -741,7 +748,9 @@ __global__ void __launch_bounds__(256) mix_inv_param_grad_kernel(const MixParamB
     const int a = e / C, k = e - a * C;
     float acc = 0.f;
     for (int c = 0; c < C; ++c) acc = fmaf(it.winv[c * C + a], t_s[c * C + k], acc);
-    it.dW[e] = -acc;
+    float v = -acc;
+    if (it.dld_sum != nullptr) v += Gld * it.winv[k * C + a];
+    it.dW[e] = v;
   }
 }
 
@@ -914,7 +923,10 @@ __global__ void __launch_bounds__(256) gauss_const_bwd_kernel(const float* __res
 // 256: thread t owns channel j0 + t % cw and every rg-th pixel (rg = 256 / cw row groups), so the dh / h rows are read and
 // written along consecutive channels; per-channel partials are combined over the row groups in a fixed order
 // (deterministic).  Writes dh rows [M, ldh] (columns C..ldh zero) when h is given, and dpar [B][2C] (dbias[C], dlogs[C]).
+// dlp (may be null): gradient of the draw's log-density sum -(log(2 pi) + 2 lg + T^2 eps^2)/2 at fixed eps, which is
+// -dlp[b] on every lg and nothing on the mean.
 __global__ void __launch_bounds__(256) split_sample_bwd_kernel(const float* __restrict__ dz, int64_t dz_bs,
+                                                               const float* __restrict__ dlp,
                                                                const float* __restrict__ eps, float temperature,
                                                                const float* __restrict__ h, int64_t ldh,
                                                                const float* __restrict__ bias, const float* __restrict__ logs,
@@ -933,7 +945,8 @@ __global__ void __launch_bounds__(256) split_sample_bwd_kernel(const float* __re
         const float hm = (h != nullptr) ? h[m * ldh + j] : 0.f, hl = (h != nullptr) ? h[m * ldh + Ch + j] : 0.f;
         const float mean = (hm + bm) * em, lg = (hl + bl) * el;
         const float g = dz[b * dz_bs + (int64_t)j * P + p];
-        const float dlg = g * expf(lg) * temperature * eps[((int64_t)b * Ch + j) * P + p];
+        float dlg = g * expf(lg) * temperature * eps[((int64_t)b * Ch + j) * P + p];
+        if (dlp != nullptr) dlg -= dlp[b];
         const float dhm = g * em, dhl = dlg * el;
         if (h != nullptr) {
           dh[m * ldh + j] = dhm;
@@ -1011,12 +1024,11 @@ extern "C" int nfdpm_coupling_bwd_tiles(int C, int H, int W) {
 }
 
 template <bool INV>
-static int coupling_bwd_launch(const float* dy, int64_t dy_bs, const float* dld, const float* u, int64_t u_bs,
-                               const float* pm, int64_t ldp, const float* bias3, const float* logs3, float* du,
-                               int64_t du_bs, void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias,
-                               float* dlogs, int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
+static int coupling_bwd_launch(const char* name, const float* dy, int64_t dy_bs, const float* dld, const float* u,
+                               int64_t u_bs, const float* pm, int64_t ldp, const float* bias3, const float* logs3,
+                               float* du, int64_t du_bs, void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar,
+                               float* dbias, float* dlogs, int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
                                cudaStream_t st) {
-  const char* name = INV ? "nfdpm_coupling_inv_bwd" : "nfdpm_coupling_bwd";
   NFDPM_REQUIRE(dy && u && pm && bias3 && logs3 && du && dpm && dpar, "%s: null pointer", name);
   NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0 && ldp >= 9 * (int64_t)C && ld_dpm >= 9 * (int64_t)C,
                 "%s: bad shape", name);
@@ -1075,8 +1087,18 @@ extern "C" int nfdpm_coupling_bwd(const float* dy, int64_t dy_bs, const float* d
                                   int64_t du_bs, void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias,
                                   float* dlogs, int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
                                   nfdpm_stream_t stream) {
-  return coupling_bwd_launch<false>(dy, dy_bs, dld, u, u_bs, pm, ldp, bias3, logs3, du, du_bs, dpm, dpm_dtype, ld_dpm, dpar,
+  return coupling_bwd_launch<false>("nfdpm_coupling_bwd", dy, dy_bs, dld, u, u_bs, pm, ldp, bias3, logs3, du, du_bs, dpm, dpm_dtype, ld_dpm, dpar,
                                     dbias, dlogs, counter, dp_scratch, B, C, H, W, as_stream(stream));
+}
+
+extern "C" int nfdpm_coupling_inv_bwd_ld(const float* dx, int64_t dx_bs, const float* dld, const float* y, int64_t y_bs,
+                                         const float* pm, int64_t ldp, const float* bias3, const float* logs3, float* dy,
+                                         int64_t dyo_bs, void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias,
+                                         float* dlogs, int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
+                                         nfdpm_stream_t stream) {
+  return coupling_bwd_launch<true>("nfdpm_coupling_inv_bwd_ld", dx, dx_bs, dld, y, y_bs, pm, ldp, bias3, logs3, dy, dyo_bs,
+                                   dpm, dpm_dtype, ld_dpm, dpar, dbias, dlogs, counter, dp_scratch, B, C, H, W,
+                                   as_stream(stream));
 }
 
 extern "C" int nfdpm_coupling_inv_bwd(const float* dx, int64_t dx_bs, const float* y, int64_t y_bs, const float* pm,
@@ -1084,8 +1106,9 @@ extern "C" int nfdpm_coupling_inv_bwd(const float* dx, int64_t dx_bs, const floa
                                       void* dpm, int dpm_dtype, int64_t ld_dpm, float* dpar, float* dbias, float* dlogs,
                                       int32_t* counter, float* dp_scratch, int B, int C, int H, int W,
                                       nfdpm_stream_t stream) {
-  return coupling_bwd_launch<true>(dx, dx_bs, nullptr, y, y_bs, pm, ldp, bias3, logs3, dy, dyo_bs, dpm, dpm_dtype, ld_dpm,
-                                   dpar, dbias, dlogs, counter, dp_scratch, B, C, H, W, as_stream(stream));
+  return coupling_bwd_launch<true>("nfdpm_coupling_inv_bwd", dx, dx_bs, nullptr, y, y_bs, pm, ldp, bias3, logs3, dy, dyo_bs,
+                                   dpm, dpm_dtype, ld_dpm, dpar, dbias, dlogs, counter, dp_scratch, B, C, H, W,
+                                   as_stream(stream));
 }
 
 extern "C" int nfdpm_actnorm_relu_bwd(const void* dh, int dh_dtype, int64_t ld_dh, const void* h, int h_dtype, int64_t ld_h,
@@ -1225,7 +1248,7 @@ extern "C" int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items, int n,
     int cmax = 0;
     for (int i = 0; i < cnt; ++i) {
       const nfdpm_mix_grad_item& s = items[base + i];
-      pb.it[i] = MixParamItem{s.part, s.B, s.weight, s.scale, s.bias, s.winv, nullptr, s.P, s.d_weight, s.d_scale,
+      pb.it[i] = MixParamItem{s.part, s.B, s.weight, s.scale, s.bias, s.winv, s.dld_sum, s.P, s.d_weight, s.d_scale,
                               s.d_bias, s.scratch, s.C};
       if (s.C > cmax) cmax = s.C;
     }
@@ -1323,16 +1346,26 @@ extern "C" int nfdpm_gauss_const_bwd(const float* dl, const float* z, const floa
   return 0;
 }
 
+extern "C" int nfdpm_split_sample_bwd_lp(const float* dz, int64_t dz_bs, const float* dlp, const float* eps,
+                                         float temperature, const float* h, int64_t ldh, const float* bias,
+                                         const float* logs, float* dh, float* dpar, int B, int C, int H, int W,
+                                         nfdpm_stream_t stream) {
+  NFDPM_REQUIRE(dz && eps && bias && logs && dpar, "nfdpm_split_sample_bwd_lp: null pointer");
+  NFDPM_REQUIRE(h == nullptr || (dh && ldh >= C), "nfdpm_split_sample_bwd_lp: the conditional form needs dh with ldh >= C");
+  NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_sample_bwd_lp: bad shape");
+  split_sample_bwd_kernel<<<B, 256, 0, as_stream(stream)>>>(dz, dz_bs, dlp, eps, temperature, h, ldh, bias, logs, dh, dpar,
+                                                            C, H * W);
+  NFDPM_CHECK_LAUNCH("split_sample_bwd_kernel");
+  return 0;
+}
+
 extern "C" int nfdpm_split_sample_bwd(const float* dz, int64_t dz_bs, const float* eps, float temperature, const float* h,
                                       int64_t ldh, const float* bias, const float* logs, float* dh, float* dpar, int B, int C,
                                       int H, int W, nfdpm_stream_t stream) {
   NFDPM_REQUIRE(dz && eps && bias && logs && dpar, "nfdpm_split_sample_bwd: null pointer");
   NFDPM_REQUIRE(h == nullptr || (dh && ldh >= C), "nfdpm_split_sample_bwd: the conditional form needs dh with ldh >= C");
   NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_sample_bwd: bad shape");
-  split_sample_bwd_kernel<<<B, 256, 0, as_stream(stream)>>>(dz, dz_bs, eps, temperature, h, ldh, bias,
-                                                                                 logs, dh, dpar, C, H * W);
-  NFDPM_CHECK_LAUNCH("split_sample_bwd_kernel");
-  return 0;
+  return nfdpm_split_sample_bwd_lp(dz, dz_bs, nullptr, eps, temperature, h, ldh, bias, logs, dh, dpar, B, C, H, W, stream);
 }
 
 extern "C" int nfdpm_col2im_add(const float* da, int64_t lda, float* dstate, int64_t dbs, int B, int Cin, int H, int W,

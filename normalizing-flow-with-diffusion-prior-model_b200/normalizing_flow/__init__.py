@@ -56,6 +56,12 @@ class NFBackbone(nn.Module):
         would add it (the Split priors are not evaluated, as in ``transform``)."""
         return self.model.invert(latents, log_det_jac=log_det_jac)
 
+    def invert_with_density(self, latents: list, log_det_jac: Tensor) -> Tuple[Tensor, Tensor]:
+        """Glow.invert_with_density without the Split priors (as ``transform``): ``(x, log_det_jac)``, differentiable in
+        both; a frozen flow still passes gradients to the latents."""
+        x, log_det_jac, _ = self.model.invert_with_density(latents, log_det_jac=log_det_jac)
+        return x, log_det_jac
+
     @torch.no_grad()
     def sample(self, latents: list, postprocess_func=None, log_det_jac: Optional[Tensor] = None) -> Tensor:
         """Glow.sample; ``log_det_jac`` as in ``invert``, at the sample before ``postprocess_func``."""

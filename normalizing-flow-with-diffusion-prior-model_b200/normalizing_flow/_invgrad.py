@@ -48,24 +48,33 @@ def _a1(cp, M: int, dt: torch.dtype, dev) -> Tensor:
     return torch.empty(M * cp._cache.K1p, dtype=dt, device=dev)
 
 
-def _level_stash(flows, src: Tensor, mode: str, B: int, C: int, h: int, w: int):
-    """The K inverse StepFlows of one level (input ``src``, only read) with the operands of every step kept.
-    Returns (level output, [(y_k, stash_k, u_k) for k = 0..K-1])."""
+def _level_stash(flows, src: Tensor, mode: str, B: int, C: int, h: int, w: int, ld_part: Optional[Tensor] = None,
+                 row: int = 0):
+    """The K inverse StepFlows of one level (input ``src``, only read) with the operands of every step kept.  The log-det
+    partials go to the rows of ``ld_part`` from ``row`` on that the no-grad level function of ``mode`` writes (none when
+    ``ld_part`` is None).  Returns (level output, [(y_k, stash_k, u_k) for k = 0..K-1], partial rows)."""
     dev = src.device
     P, M = h * w, B * h * w
     K = len(flows)
     recs = [None] * K
     cur = src
+    rows = 0
+
+    def part():
+        return ld_part[(row + rows) * B:] if ld_part is not None else None
+
     if mode == "unfused":
+        T = N.ld_tiles(P)
         for k in range(K - 1, -1, -1):
             step = flows[k]
             E.prepare_mix([step._mix_entry(None)])
-            u, st = MG.coupling_invert_stash(step.affcoupling, cur)
+            u, st = MG.coupling_invert_stash(step.affcoupling, cur, part())
             x = torch.empty_like(u)
             N.channel_mix(u, x, step._mix.inv_mt, step._mix.inv_beta, B, C, P, C * P, C * P)
             recs[k] = (cur, st, u)
             cur = x
-        return cur, recs
+            rows += T
+        return cur, recs, rows
     dt = E.coupling_dtype()
     A1 = _a1(flows[-1].affcoupling, M, dt, dev)
     K1p = flows[-1].affcoupling._cache.K1p
@@ -87,52 +96,64 @@ def _level_stash(flows, src: Tensor, mode: str, B: int, C: int, h: int, w: int):
         K1n = flows[k - 1].affcoupling._cache.K1p if k > 0 else 0
         mt, beta = step._mix.inv_mt, step._mix.inv_beta
         if mode == "tiled":
+            T = N.flow_boundary_tiles(B, C, h, w, 1, 1, int(k > 0))
             N.gemm_nt(h2, F, cp._cache.at(dt).w3, F, pm, ldp, M, ldp, F)
-            N.flow_boundary_tiled(cur, C * P, False, pm, ldp, zc.bias, zc.logs, None, mt, beta, x, C * P, u, C * P, A1n, K1n,
-                                  B, C, h, w, True, N.flow_boundary_tiles(B, C, h, w, 1, 1, int(k > 0)))
+            N.flow_boundary_tiled(cur, C * P, False, pm, ldp, zc.bias, zc.logs, part(), mt, beta, x, C * P, u, C * P, A1n,
+                                  K1n, B, C, h, w, True, T)
         elif E.fused_g3_ok(B, C, h, w, F, ldp, dt):
-            N.gemm3_boundary(h2, F, cp._cache.at(dt).w3, pm, ldp, cur, C * P, zc.bias, zc.logs, None, mt, beta, x, C * P, u,
-                             C * P, A1n, K1n, B, C, h, w, F, ldp, True)
+            T = 1
+            N.gemm3_boundary(h2, F, cp._cache.at(dt).w3, pm, ldp, cur, C * P, zc.bias, zc.logs, part(), mt, beta, x, C * P,
+                             u, C * P, A1n, K1n, B, C, h, w, F, ldp, True)
         else:
+            T = 1
             N.gemm_nt(h2, F, cp._cache.at(dt).w3, F, pm, ldp, M, ldp, F)
-            N.flow_boundary_inv_stash(cur, C * P, pm, ldp, zc.bias, zc.logs, mt, beta, x, C * P, u, C * P, A1n, K1n, B, C, h,
-                                      w)
+            N.flow_boundary_inv_stash_ld(cur, C * P, pm, ldp, zc.bias, zc.logs, part(), mt, beta, x, C * P, u, C * P, A1n,
+                                         K1n, B, C, h, w)
         recs[k] = (cur, SimpleNamespace(A1=A1, h1=h1, h2=h2, pm=pm, dt=dt, K1p=K1p, ldp=ldp), u)
         cur, A1 = x, A1n
-    return cur, recs
+        rows += T
+    return cur, recs, rows
 
 
-def invert_stash(glow, latents, temperature: float):
-    """Glow.invert returning (x, per-level step records, per-Split (input, eps)).  The walk and the kernels are those of the
-    no-grad inverse (uncaptured, ``Glow._invert_walk``), with `_level_stash` for each level's StepFlows; an uninitialised
-    model takes the unfused chain, which initialises the coupling networks' ActNorms on the way (without gradient), as the
-    no-grad inverse does."""
+def invert_stash(glow, latents, temperature: float, with_ld: bool = False, with_lp: bool = False):
+    """Glow.invert returning (x, per-level step records, per-Split (input, eps), density partials as `_invert_walk`
+    returns them).  The walk and the kernels are those of the no-grad inverse (uncaptured, ``Glow._invert_walk``), with
+    `_level_stash` for each level's StepFlows; an uninitialised model takes the unfused chain, which initialises the
+    coupling networks' ActNorms on the way (without gradient), as the no-grad inverse does."""
     steps_rec, split_rec = [], []
 
-    def level(mode, flows, src, B, C, h, w):
-        x, recs = _level_stash(flows, src, mode, B, C, h, w)
+    def level(mode, flows, src, B, C, h, w, ld_part, row):
+        x, recs, rows = _level_stash(flows, src, mode, B, C, h, w, ld_part, row)
         steps_rec.insert(0, recs)                       # the walk runs deepest first
-        return x
+        return x, rows
 
-    x, _ = glow._invert_walk(latents, temperature, glow._ready(), level=level, eps_sink=split_rec)
-    return x, steps_rec, split_rec[::-1]
+    x, parts = glow._invert_walk(latents, temperature, glow._ready(), with_ld, with_lp, level=level, eps_sink=split_rec)
+    return x, steps_rec, split_rec[::-1], parts
 
 
 class GlowInvertFn(torch.autograd.Function):
-    """(glow, temperature, n_latents, *latents, *parameters) -> x."""
+    """(glow, temperature, n_latents, log_det_jac | None, logp | None, *latents, *parameters) -> x, or (x, log_det_jac?,
+    logp?) when an accumulator is given: the accumulators receive the density of x in place (``Glow._add_density``, as
+    the no-grad inverse) and are marked dirty; their gradients reach the log-det and Split log-p terms."""
 
     @staticmethod
-    def forward(ctx, glow, temperature, n_lat, *args):
+    def forward(ctx, glow, temperature, n_lat, ld, lp, *args):
         latents = [t.detach() if isinstance(t, Tensor) else t for t in args[:n_lat]]
         ctx.glow, ctx.temperature, ctx.n_lat, ctx.params = glow, temperature, n_lat, args[n_lat:]
-        x, steps_rec, split_rec = invert_stash(glow, latents, temperature)
+        ctx.have_ld, ctx.have_lp = ld is not None, lp is not None
+        x, steps_rec, split_rec, parts = invert_stash(glow, latents, temperature, ld is not None, lp is not None)
         ctx.rec = (steps_rec, split_rec)
         # the deepest level's first step keeps the caller's last latent: saved so that an in-place change is detected
         ctx.save_for_backward(*[t for t in args[:n_lat] if isinstance(t, Tensor)])
-        return x
+        accs = [a for a in (ld, lp) if a is not None]
+        if not accs:
+            return x
+        glow._add_density(ld, lp, parts, x.shape[2], x.shape[3])
+        ctx.mark_dirty(*accs)
+        return (x,) + tuple(accs)
 
     @staticmethod
-    def backward(ctx, dx):
+    def backward(ctx, dx, *g_acc):
         if ctx.rec is None:
             raise RuntimeError("Glow.invert: the stash of this call was released by an earlier backward")
         ctx.saved_tensors                               # raises if a latent was modified in place since the forward
@@ -142,6 +163,10 @@ class GlowInvertFn(torch.autograd.Function):
         L = glow.L
         dy = dx.to(torch.float32).contiguous()
         B, _, H, W = dy.shape
+        g_acc = list(g_acc)
+        dld = g_acc.pop(0).to(torch.float32).contiguous() if ctx.have_ld else None
+        dlp = g_acc.pop(0).to(torch.float32).contiguous() if ctx.have_lp else None
+        dld_sum = MG._dld_sum(dld) if dld is not None else None
         g = {}
         d_lat: List[Optional[Tensor]] = [None] * n_lat
         for li, (flows, split, C, h, w) in enumerate(glow._geometry(H, W)):
@@ -152,9 +177,9 @@ class GlowInvertFn(torch.autograd.Function):
             for step, (y_k, st_k, u_k) in zip(flows, steps_rec[li]):
                 an, ic = step.actnorm, step.invconv2d
                 du, dW, dS, dB = MG._mix_inv_backward(step._mix, u_k, d, ic.weight, an.scale, an.bias,
-                                                      MG._wants_grad(an) or MG._wants_grad(ic), da1, lda1)
+                                                      MG._wants_grad(an) or MG._wants_grad(ic), da1, lda1, dld_sum)
                 g[ic.weight], g[an.scale], g[an.bias] = dW, dS, dB
-                d, gc, da1 = MG._coupling_backward(step.affcoupling, st_k, y_k, du, None, inverse=True,
+                d, gc, da1 = MG._coupling_backward(step.affcoupling, st_k, y_k, du, dld, inverse=True,
                                                    wgrad=MG._wants_grad(step.affcoupling), col2im=False)
                 lda1 = st_k.K1p
                 g.update(gc)
@@ -163,18 +188,27 @@ class GlowInvertFn(torch.autograd.Function):
                 d_lat[n_lat - 1] = d
                 break
             nxt, eps = split_rec[li]
-            dy, dz, gs = MG._split_sample_backward(split, nxt, eps, T, d, MG._wants_grad(split))
+            dy, dz, gs = MG._split_sample_backward(split, nxt, eps, T, d, MG._wants_grad(split), dlp)
             g.update(gs)
             if dz is not None:
                 d_lat[n_lat - (L - li)] = dz
-        lat_g = [gl if ctx.needs_input_grad[3 + i] else None for i, gl in enumerate(d_lat)]
+        lat_g = [gl if ctx.needs_input_grad[5 + i] else None for i, gl in enumerate(d_lat)]
         par_g = [g.get(p) if p.requires_grad else None for p in ctx.params]
-        return (None, None, None) + tuple(lat_g) + tuple(par_g)
+        return (None, None, None, None, None) + tuple(lat_g) + tuple(par_g)
 
 
-def glow_invert(glow, latents: list, temperature: float) -> Tensor:
+def glow_invert(glow, latents: list, temperature: float, log_det_jac: Optional[Tensor] = None,
+                logp: Optional[Tensor] = None):
+    """The recorded Glow.invert: x, or (x, log_det_jac, logp) when an accumulator is given (``None`` stays ``None``)."""
     lat = [E.check_input(t, "latent") if isinstance(t, Tensor) else t for t in latents]
-    return GlowInvertFn.apply(glow, float(temperature), len(lat), *lat, *glow.parameters())
+    out = GlowInvertFn.apply(glow, float(temperature), len(lat), log_det_jac, logp, *lat, *glow.parameters())
+    if log_det_jac is None and logp is None:
+        return out
+    out = list(out)
+    x = out.pop(0)
+    ld = out.pop(0) if log_det_jac is not None else None
+    lp = out.pop(0) if logp is not None else None
+    return x, ld, lp
 
 
 # ------------------------------------------------------------------------------------------- priors

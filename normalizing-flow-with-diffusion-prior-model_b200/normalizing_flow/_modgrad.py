@@ -66,10 +66,11 @@ def _mix_backward(mod, x: Tensor, dy: Tensor, dld32: Tensor, weight, scale, bias
 
 
 def _mix_inv_backward(mix, u: Tensor, dx: Tensor, weight, scale, bias, wgrad: bool = True, da1: Optional[Tensor] = None,
-                      lda1: int = 0):
+                      lda1: int = 0, dld_sum: Optional[Tensor] = None):
     """Backward of the inverse mix x = diag(e^-s) W^-1 u - b: du (nfdpm_mix_bwd with inv_mt) and, with ``wgrad``, the
     parameter gradients (nfdpm_mix_inv_param_grad).  ``da1``: im2col-row gradient of a coupling network that read ``x``;
-    its col2im is added to ``dx`` inside mix_bwd."""
+    its col2im is added to ``dx`` inside mix_bwd.  ``dld_sum`` ([1], sum over the batch of d(log_det_jac)): the gradient of
+    the constant H*W*(sum s + log|det W|) the inverse accumulates is folded into the parameter gradients."""
     B, C, H, W = u.shape
     P = H * W
     f32 = dict(dtype=torch.float32, device=u.device)
@@ -86,29 +87,54 @@ def _mix_inv_backward(mix, u: Tensor, dx: Tensor, weight, scale, bias, wgrad: bo
     dB = torch.empty_like(bias) if bias is not None else None
     scratch = torch.empty(C * C + C, **f32)
     item = N.MixGradItem(part=part.data_ptr(), B=B * T_m, C=C, weight=N._p(weight), scale=N._p(scale), bias=N._p(bias),
-                         winv=mix.winv.data_ptr() if weight is not None else eye.data_ptr(), dld_sum=None, P=0.0, pad_=0,
+                         winv=mix.winv.data_ptr() if weight is not None else eye.data_ptr(), dld_sum=N._p(dld_sum),
+                         P=float(P) if dld_sum is not None else 0.0, pad_=0,
                          d_weight=N._p(dW), d_scale=N._p(dS), d_bias=N._p(dB), scratch=scratch.data_ptr())
     N.mix_inv_param_grad([item])
     return du, dW, dS, dB
 
 
-def _split_sample_backward(sp, out: Tensor, eps: Optional[Tensor], temperature: float, d_out: Tensor, wgrad: bool = True):
+def _split_sample_backward(sp, out: Tensor, eps: Optional[Tensor], temperature: float, d_out: Tensor, wgrad: bool = True,
+                           dlp: Optional[Tensor] = None):
     """Backward of Split.invert: ``out`` = (y | z) [B,C,H,W], ``d_out`` its gradient.  Returns (dy, d_latent, grads).  A
     sampled half (``eps`` given) z = mean(y) + exp(lg(y))*T*eps back-propagates into y and the prior conv's parameters
-    (nfdpm_split_sample_bwd + the conv's fp32 wgrad / dgrad GEMMs); a supplied latent receives the second half."""
+    (nfdpm_split_sample_bwd + the conv's fp32 wgrad / dgrad GEMMs); a supplied latent receives the second half.
+    ``dlp`` ([B] fp32): gradient of the log-density log N(z; mean(y), exp(lg(y))) the inverse accumulated for this Split.
+    A sampled half takes it inside nfdpm_split_sample_bwd_lp (-dlp on lg); a supplied one through nfdpm_split_prior_bwd on
+    the assembled ``out``, into the latent and, through the prior conv, into y and the conv's parameters (it adds to the
+    second half of ``d_out`` in place)."""
     B, C, H, W = out.shape
-    Ch, P, M = C // 2, H * W, B * H * W
+    Ch, P = C // 2, H * W
     f32 = dict(dtype=torch.float32, device=out.device)
     dy = torch.empty(B, Ch, H, W, **f32)
     N.copy_channels(d_out, dy, B, Ch, P, C * P, Ch * P)
     g = {}
+    conv = sp.conv
     if eps is None:
+        if dlp is not None and conv is None:            # the standard-normal prior ignores y: only the latent's term
+            N.split_prior_bwd(dlp, None, 0, None, None, out, C * P, d_out, C * P, None, None, B, C, H, W)
+        elif dlp is not None:
+            _prior_conv_backward(sp, out, dy, Ch * P, wgrad, g, lambda hs, ldh, dh, dpar: N.split_prior_bwd(
+                dlp, hs, ldh, conv.bias, conv.logs, out, C * P, d_out, C * P, dh, dpar, B, C, H, W))
         dz = torch.empty(B, Ch, H, W, **f32)
         N.copy_channels(d_out.view(-1)[Ch * P:], dz, B, Ch, P, C * P, Ch * P)
         return dy, dz, g
-    conv = sp.conv
     if conv is None:                                    # the standard-normal prior has no parameters and ignores y
         return dy, None, g
+    _prior_conv_backward(sp, out, dy, Ch * P, wgrad, g, lambda hs, ldh, dh, dpar: N.split_sample_bwd_lp(
+        d_out.view(-1)[Ch * P:], C * P, dlp, eps, temperature, hs, ldh, conv.bias, conv.logs, dh, dpar, B, C, H, W))
+    return dy, None, g
+
+
+def _prior_conv_backward(sp, out: Tensor, dy: Tensor, dy_bs: int, wgrad: bool, g: dict, prior_bwd) -> None:
+    """The Split prior conv's part of a Split backward: recompute its rows hs from the first half of ``out`` [B,C,H,W]
+    (im2col + fp32 GEMM), run ``prior_bwd(hs, ldh, dh, dpar)`` (the prior kernel's backward, which writes dh and the
+    per-image bias / logs partials), then the conv's wgrad (with ``wgrad``, into ``g``) and dgrad + col2im into the first
+    C/2 channels of ``dy`` (batch stride ``dy_bs``)."""
+    B, C, H, W = out.shape
+    Ch, P, M = C // 2, H * W, B * H * W
+    f32 = dict(dtype=torch.float32, device=out.device)
+    conv = sp.conv
     Ks, Kp, ldh = Ch * 9, E.round_up(Ch * 9, 16), E.round_up(C, 16)
     wp = torch.empty(ldh * Kp, **f32)
     N.pack_matrix(conv.weight, wp, 1, C, Ks, 0, Ks, 1, Kp, ldh)
@@ -120,7 +146,7 @@ def _split_sample_backward(sp, out: Tensor, eps: Optional[Tensor], temperature: 
     N.gemm_nt(As, Kp, wp, Kp, hs, ldh, M, C, Kp)
     dh = torch.empty(M * ldh, **f32)
     dpar = torch.empty(B * 2 * C, **f32)
-    N.split_sample_bwd(d_out.view(-1)[Ch * P:], C * P, eps, temperature, hs, ldh, conv.bias, conv.logs, dh, dpar, B, C, H, W)
+    prior_bwd(hs, ldh, dh, dpar)
     if wgrad:
         g[conv.bias], g[conv.logs] = torch.empty_like(conv.bias), torch.empty_like(conv.logs)
         N.reduce_rows2(dpar, g[conv.bias], g[conv.logs], B, C, C, 2 * C)
@@ -131,8 +157,7 @@ def _split_sample_backward(sp, out: Tensor, eps: Optional[Tensor], temperature: 
         N.pack_matrix(dws, g[conv.weight], C, 1, Ks, Kp, 0, 1, Ks, C)        # drop the K padding
     dAs = torch.empty(M * Kp, **f32)
     N.gemm_nt(dh, ldh, wst, ldh, dAs, Kp, M, Kp, ldh)
-    N.col2im_add(dAs, Kp, dy, Ch * P, B, Ch, H, W)
-    return dy, None, g
+    N.col2im_add(dAs, Kp, dy, dy_bs, B, Ch, H, W)
 
 
 def _wants_grad(mod) -> bool:
@@ -157,7 +182,8 @@ def _coupling_forward(cp, x: Tensor, ld: Optional[Tensor]):
 def _coupling_backward(cp, st: SimpleNamespace, x: Tensor, dy: Tensor, dld32: Optional[Tensor], inverse: bool = False,
                        wgrad: bool = True, col2im: bool = True):
     """Backward of AffineCoupling.transform (``x`` its input) or, with ``inverse``, of AffineCoupling.invert (``x`` the
-    inverse's input y, ``dy`` the gradient of its output; no log-det): coupling_bwd / coupling_inv_bwd, then the coupling
+    inverse's input y, ``dy`` the gradient of its output; ``dld32`` None or the gradient of the log-det the inverse
+    accumulated): coupling_bwd / coupling_inv_bwd_ld, then the coupling
     network (``_net_backward``).  ``wgrad=False`` skips every parameter gradient (frozen network).  With
     ``col2im=False`` the network's im2col-row gradient dA1 is returned as a third value instead of being added to du (the
     caller fuses it into the next mix_bwd)."""
@@ -176,8 +202,8 @@ def _coupling_backward(cp, st: SimpleNamespace, x: Tensor, dy: Tensor, dld32: Op
     fused = dict(dbias=g[zc.bias], dlogs=g[zc.logs]) if wgrad and T_c == 1 else {}
     tiled = dict(dp_scratch=torch.empty(M * C, **f32)) if T_c > 1 else {}
     if inverse:
-        N.coupling_inv_bwd(dy, C * P, x, C * P, st.pm, st.ldp, zc.bias, zc.logs, du, C * P, dpm, Kp3, dpar3, B, C, H, W,
-                           **fused, **tiled)
+        N.coupling_inv_bwd_ld(dy, C * P, dld32, x, C * P, st.pm, st.ldp, zc.bias, zc.logs, du, C * P, dpm, Kp3, dpar3, B, C,
+                              H, W, **fused, **tiled)
     else:
         N.coupling_bwd(dy, C * P, dld32, x, C * P, st.pm, st.ldp, zc.bias, zc.logs, du, C * P, dpm, Kp3, dpar3, B, C, H, W,
                        **fused, **tiled)
@@ -257,8 +283,7 @@ def _net_backward(cp, st: SimpleNamespace, dpm: Tensor, dstate: Optional[Tensor]
 def _split_backward(sp, x: Tensor, dy_kept: Optional[Tensor], dz: Optional[Tensor], dlp32: Optional[Tensor]):
     """Backward of (y, z) = chunk(x), logp += N(z; mean(y), exp(logs(y))) (transforms.py:285-289)."""
     B, C, H, W = x.shape
-    Ch, P, M = C // 2, H * W, B * H * W
-    f32 = dict(dtype=torch.float32, device=x.device)
+    Ch, P = C // 2, H * W
     dx = torch.zeros_like(x)
     if dy_kept is not None:
         N.copy_channels(dy_kept.to(torch.float32).contiguous(), dx, B, Ch, P, Ch * P, C * P)
@@ -271,28 +296,8 @@ def _split_backward(sp, x: Tensor, dy_kept: Optional[Tensor], dz: Optional[Tenso
     if conv is None:
         N.split_prior_bwd(dlp32, None, 0, None, None, x, C * P, dx, C * P, None, None, B, C, H, W)
         return dx, g
-    Ks, Kp, ldh = Ch * 9, E.round_up(Ch * 9, 16), E.round_up(C, 16)
-    wp = torch.empty(ldh * Kp, **f32)
-    N.pack_matrix(conv.weight, wp, 1, C, Ks, 0, Ks, 1, Kp, ldh)
-    wst = torch.empty(Kp * ldh, **f32)
-    N.pack_matrix(conv.weight, wst, Ks, 1, C, 1, 0, Ks, ldh, Kp)
-    As = torch.empty(M * Kp, **f32)
-    N.im2col3x3(x, As, B, Ch, H, W, C * P, Kp)
-    hs = torch.empty(M * ldh, **f32)
-    N.gemm_nt(As, Kp, wp, Kp, hs, ldh, M, C, Kp)
-    dh = torch.empty(M * ldh, **f32)
-    dpar = torch.empty(B * 2 * C, **f32)
-    N.split_prior_bwd(dlp32, hs, ldh, conv.bias, conv.logs, x, C * P, dx, C * P, dh, dpar, B, C, H, W)
-    g[conv.bias], g[conv.logs] = torch.empty_like(conv.bias), torch.empty_like(conv.logs)
-    N.reduce_rows2(dpar, g[conv.bias], g[conv.logs], B, C, C, 2 * C)
-    dws = torch.empty(C * Kp, **f32)
-    ws = torch.empty(N.gemm_tn_workspace(M, C, Kp), **f32)
-    N.gemm_tn(dh, ldh, As, Kp, dws, M, C, Kp, ws, fused_reduce=False)
-    g[conv.weight] = torch.empty_like(conv.weight)
-    N.pack_matrix(dws, g[conv.weight], C, 1, Ks, Kp, 0, 1, Ks, C)        # drop the K padding
-    dAs = torch.empty(M * Kp, **f32)
-    N.gemm_nt(dh, ldh, wst, ldh, dAs, Kp, M, Kp, ldh)
-    N.col2im_add(dAs, Kp, dx, C * P, B, Ch, H, W)
+    _prior_conv_backward(sp, x, dx, C * P, True, g, lambda hs, ldh, dh, dpar: N.split_prior_bwd(
+        dlp32, hs, ldh, conv.bias, conv.logs, x, C * P, dx, C * P, dh, dpar, B, C, H, W))
     return dx, g
 
 
@@ -382,8 +387,9 @@ def transform(mod, what: str, raw_forward, x: Tensor, ld: Optional[Tensor], lp: 
 
 
 # ------------------------------------------------------------------------------------------- invert (NFDPM_INVERT_GRAD=1)
-def coupling_invert_stash(cp, y: Tensor):
-    """AffineCoupling.invert keeping the coupling network's operands, in the operand format of the no-grad inverse."""
+def coupling_invert_stash(cp, y: Tensor, ld_part: Optional[Tensor] = None):
+    """AffineCoupling.invert keeping the coupling network's operands, in the operand format of the no-grad inverse.
+    ``ld_part``: the log-det partial rows, as the no-grad inverse writes them."""
     B, C, H, W = y.shape
     E.last_coupling_stash = None
     E.coupling_rows(cp, y, C * H * W, B, C, H, W, init=True, stash=True, fmt=E.coupling_dtype())
@@ -391,7 +397,7 @@ def coupling_invert_stash(cp, y: Tensor):
     E.last_coupling_stash = None
     x = torch.empty_like(y)
     zc = cp._parts()[4]
-    N.coupling_apply(st.pm, st.ldp, zc.bias, zc.logs, y, x, None, B, C, H, W, C * H * W, C * H * W, True)
+    N.coupling_apply(st.pm, st.ldp, zc.bias, zc.logs, y, x, ld_part, B, C, H, W, C * H * W, C * H * W, True)
     return x, st
 
 

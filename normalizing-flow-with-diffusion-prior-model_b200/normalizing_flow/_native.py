@@ -80,12 +80,16 @@ def _load() -> C.CDLL:
                                 i32, i32, vp], C.c_int),
         "nfdpm_coupling_inv_bwd": ([vp, i64, vp, i64, vp, i64, vp, vp, vp, i64, vp, i32, i64, vp, vp, vp, vp, vp, i32, i32,
                                     i32, i32, vp], C.c_int),
+        "nfdpm_coupling_inv_bwd_ld": ([vp, i64, vp, vp, i64, vp, i64, vp, vp, vp, i64, vp, i32, i64, vp, vp, vp, vp, vp, i32,
+                                       i32, i32, i32, vp], C.c_int),
         "nfdpm_coupling_bwd_tiles": ([i32, i32, i32], C.c_int),
         "nfdpm_mix_bwd_tiles": ([i32, i32, i32], C.c_int),
         "nfdpm_flow_boundary_stash": ([vp, i64, i32, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp, i64, vp, i32, i64, i32, i32,
                                        i32, i32, vp], C.c_int),
         "nfdpm_flow_boundary_inv_stash": ([vp, i64, vp, i64, vp, vp, vp, vp, vp, i64, vp, i64, vp, i32, i64, i32, i32, i32, i32,
                                            vp], C.c_int),
+        "nfdpm_flow_boundary_inv_stash_ld": ([vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp, i64, vp, i32, i64, i32, i32,
+                                              i32, i32, vp], C.c_int),
         "nfdpm_actnorm_relu_bwd": ([vp, i32, i64, vp, i32, i64, vp, vp, i32, i64, vp, i32, i32, i32, vp], C.c_int),
         "nfdpm_reduce_rows2": ([vp, vp, vp, i32, i32, i32, i64, vp], C.c_int),
         "nfdpm_gemm3_boundary_ok": ([i32, i32, i32, i32, i32, i64], C.c_int),
@@ -107,6 +111,7 @@ def _load() -> C.CDLL:
         "nfdpm_split_prior_bwd": ([vp, vp, i64, vp, vp, vp, i64, vp, i64, vp, vp, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_gauss_const_bwd": ([vp, vp, vp, vp, vp, vp, i32, i32, i32, vp], C.c_int),
         "nfdpm_split_sample_bwd": ([vp, i64, vp, f32, vp, i64, vp, vp, vp, vp, i32, i32, i32, i32, vp], C.c_int),
+        "nfdpm_split_sample_bwd_lp": ([vp, i64, vp, vp, f32, vp, i64, vp, vp, vp, vp, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_col2im_add": ([vp, i64, vp, i64, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_accumulate": ([vp, i32, vp, i32, i32, vp, vp, i32, vp], C.c_int),
         "nfdpm_flow_boundary_tiles": ([i32, i32, i32, i32, i32, i32, i32], C.c_int),
@@ -185,7 +190,8 @@ EXPORTS = ["nfdpm_version", "nfdpm_last_error_string", "nfdpm_sm_count", "nfdpm_
            "nfdpm_gemm3_boundary_ok", "nfdpm_gemm3_boundary", "nfdpm_coupling_bwd_tiles", "nfdpm_mix_bwd_tiles", "nfdpm_gemm_debug", "nfdpm_flow_boundary_debug",
            "nfdpm_latent_format", "nfdpm_postprocess_u8", "nfdpm_preprocess",
            "nfdpm_flow_boundary_tiles", "nfdpm_flow_boundary_tiled",
-           "nfdpm_coupling_inv_bwd", "nfdpm_mix_inv_param_grad", "nfdpm_split_sample_bwd", "nfdpm_flow_boundary_inv_stash"]
+           "nfdpm_coupling_inv_bwd", "nfdpm_mix_inv_param_grad", "nfdpm_split_sample_bwd", "nfdpm_flow_boundary_inv_stash",
+           "nfdpm_coupling_inv_bwd_ld", "nfdpm_flow_boundary_inv_stash_ld", "nfdpm_split_sample_bwd_lp"]
 
 #: number of kernels launched through this binding (bench.py reports it as ``gpu_launches``)
 launch_count = 0
@@ -348,6 +354,15 @@ def coupling_inv_bwd(dx, dx_bs, y, y_bs, pm, ldp, bias3, logs3, dy, dy_bs, dpm, 
                                    _st()), 1 if dp_scratch is None else 2)
 
 
+def coupling_inv_bwd_ld(dx, dx_bs, dld, y, y_bs, pm, ldp, bias3, logs3, dy, dy_bs, dpm, ld_dpm, dpar, B, Cc, H, W,
+                        dbias=None, dlogs=None, dp_scratch=None) -> None:
+    """``coupling_inv_bwd`` plus the gradient ``dld`` [B] (None: none) of the log-det the inverse accumulates."""
+    cnt = _tn_counters(dx.device)[1023:] if dbias is not None else None
+    _ok(lib.nfdpm_coupling_inv_bwd_ld(_p(dx), dx_bs, _p(dld), _p(y), y_bs, _p(pm), ldp, _p(bias3), _p(logs3), _p(dy), dy_bs,
+                                      _p(dpm), _dt(dpm), ld_dpm, _p(dpar), _p(dbias), _p(dlogs), _p(cnt), _p(dp_scratch), B,
+                                      Cc, H, W, _st()), 1 if dp_scratch is None else 2)
+
+
 def flow_boundary_stash(src, src_bs, squeeze_in, pm, ldp, bias3, logs3, ld_part, mt, beta, y, y_bs, xs, xs_bs, a1, lda1,
                         B, Cc, H, W) -> None:
     _ok(lib.nfdpm_flow_boundary_stash(_p(src), src_bs, int(squeeze_in), _p(pm), ldp, _p(bias3), _p(logs3), _p(ld_part),
@@ -359,6 +374,13 @@ def flow_boundary_inv_stash(src, src_bs, pm, ldp, bias3, logs3, mt, beta, y, y_b
     _ok(lib.nfdpm_flow_boundary_inv_stash(_p(src), src_bs, _p(pm), ldp, _p(bias3), _p(logs3), _p(mt), _p(beta), _p(y), y_bs,
                                           _p(xs), xs_bs, _p(a1), _dt(a1) if a1 is not None else F32, lda1, B, Cc, H, W,
                                           _st()))
+
+
+def flow_boundary_inv_stash_ld(src, src_bs, pm, ldp, bias3, logs3, ld_part, mt, beta, y, y_bs, xs, xs_bs, a1, lda1, B, Cc,
+                               H, W) -> None:
+    _ok(lib.nfdpm_flow_boundary_inv_stash_ld(_p(src), src_bs, _p(pm), ldp, _p(bias3), _p(logs3), _p(ld_part), _p(mt),
+                                             _p(beta), _p(y), y_bs, _p(xs), xs_bs, _p(a1), _dt(a1) if a1 is not None else F32,
+                                             lda1, B, Cc, H, W, _st()))
 
 
 def actnorm_relu_bwd(dh, ld_dh, h, ld_h, scale, dpre, ld_o, part, M, Nn, rows_per_cta) -> None:
@@ -425,6 +447,11 @@ def gauss_const_bwd(dl, z, bias, logs, dz, dpar, B, Cc, P) -> None:
 def split_sample_bwd(dz, dz_bs, eps, temperature, h, ldh, bias, logs, dh, dpar, B, Cc, H, W) -> None:
     _ok(lib.nfdpm_split_sample_bwd(_p(dz), dz_bs, _p(eps), float(temperature), _p(h), ldh, _p(bias), _p(logs), _p(dh),
                                    _p(dpar), B, Cc, H, W, _st()))
+
+
+def split_sample_bwd_lp(dz, dz_bs, dlp, eps, temperature, h, ldh, bias, logs, dh, dpar, B, Cc, H, W) -> None:
+    _ok(lib.nfdpm_split_sample_bwd_lp(_p(dz), dz_bs, _p(dlp), _p(eps), float(temperature), _p(h), ldh, _p(bias), _p(logs),
+                                      _p(dh), _p(dpar), B, Cc, H, W, _st()))
 
 
 def col2im_add(da, lda, dstate, dbs, B, Cin, H, W) -> None:

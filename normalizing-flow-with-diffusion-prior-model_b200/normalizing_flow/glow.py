@@ -485,22 +485,18 @@ class Glow(Transform):
           logp        += sum over the L-1 Split halves of log N(z_l; mean_l, exp(logs_l)), supplied or drawn; the final
                          latent's prior is not included, as in ``transform``.
         Under a temperature this is the model's density at the returned sample, not the tempered one.  The accumulated
-        density is not differentiable: a call that NFDPM_INVERT_GRAD=1 would record raises NotImplementedError."""
-        z_last = E.check_input(latents[-1], "latents[-1]")
-        B, Cf, h, w = z_last.shape
-        if Cf != 2 ** (self.L + 1) * self.in_channel:
-            raise ValueError(f"final latent has {Cf} channels, expected {2 ** (self.L + 1) * self.in_channel}")
-        E.check_acc(log_det_jac, B, "log_det_jac")
-        E.check_acc(logp, B, "logp")
+        density is not differentiable here: a call that NFDPM_INVERT_GRAD=1 would record raises NotImplementedError.
+        ``invert_with_density`` returns the same values and back-propagates through them."""
+        z_last, recorded = self._check_invert_args(latents, log_det_jac, logp)
         accs = [a for a in (log_det_jac, logp) if a is not None]
-        if torch.is_grad_enabled() and any(a.requires_grad for a in accs):
-            raise RuntimeError("log_det_jac / logp are updated in place and must not require grad on entry")
-        if E.autograd_needed(z_last, self) or any(isinstance(t, Tensor) and t.requires_grad for t in latents):
+        B, _, h, w = z_last.shape
+        if recorded:
             if E.invert_grad_enabled():
                 if accs:
                     raise NotImplementedError(
                         "Glow.invert: the accumulated log_det_jac / logp are not differentiable; a recorded invert "
-                        "(NFDPM_INVERT_GRAD=1) takes no accumulators.  Call it under torch.no_grad() for the density.")
+                        "(NFDPM_INVERT_GRAD=1) takes no accumulators.  Call it under torch.no_grad() for the density, "
+                        "or Glow.invert_with_density to back-propagate through it.")
                 from ._invgrad import glow_invert
                 return glow_invert(self, latents, temperature)
             # without NFDPM_INVERT_GRAD: compute it without recording and fail loudly on back-propagation
@@ -539,14 +535,50 @@ class Glow(Transform):
         self._add_density(log_det_jac, logp, parts, H, W)
         return x
 
+    def _check_invert_args(self, latents: list, log_det_jac: Optional[Tensor], logp: Optional[Tensor]):
+        """The argument checks of `invert` / `invert_with_density`, before any launch.  Returns (final latent, whether the
+        call is to be recorded by autograd: a latent or a parameter requires grad)."""
+        z_last = E.check_input(latents[-1], "latents[-1]")
+        B, Cf, h, w = z_last.shape
+        if Cf != 2 ** (self.L + 1) * self.in_channel:
+            raise ValueError(f"final latent has {Cf} channels, expected {2 ** (self.L + 1) * self.in_channel}")
+        E.check_acc(log_det_jac, B, "log_det_jac")
+        E.check_acc(logp, B, "logp")
+        accs = [a for a in (log_det_jac, logp) if a is not None]
+        if torch.is_grad_enabled() and any(a.requires_grad for a in accs):
+            raise RuntimeError("log_det_jac / logp are updated in place and must not require grad on entry")
+        return z_last, E.autograd_needed(z_last, self) or any(isinstance(t, Tensor) and t.requires_grad for t in latents)
+
+    def invert_with_density(self, latents: list, temperature: float = 1.0, log_det_jac: Optional[Tensor] = None,
+                            logp: Optional[Tensor] = None) -> Tuple[Tensor, Optional[Tensor], Optional[Tensor]]:
+        """``invert(latents, temperature, log_det_jac, logp)`` returning ``(x, log_det_jac, logp)``, differentiable in all
+        three: the density of generated images as a function of the latents and the weights (reverse-KL / variational
+        training, entropy terms, distillation through the flow).  The arguments and the accumulated values are exactly
+        those of ``invert``; at least one accumulator is required (``None`` stays ``None``), and both are updated in place.
+
+        Without autograd (no latent and no parameter requires grad, or under ``torch.no_grad()``) this is ``invert``, with
+        the same captured chain.  Otherwise it records ONE autograd node whose outputs are x and the accumulators (marked
+        dirty, like ``transform``'s): gradients reach the latents, every StepFlow parameter and every Split prior conv,
+        at sampled Splits (through the draw and its log-density) and at supplied ones (through the log-density).  It
+        records whether or not NFDPM_INVERT_GRAD is set: that knob guards ``invert``, ``sample`` and the granular inverses,
+        whose callers did not ask for a graph.  The recorded call is not captured in a CUDA graph."""
+        if log_det_jac is None and logp is None:
+            raise ValueError("Glow.invert_with_density needs log_det_jac and/or logp; Glow.invert returns the images alone")
+        _, recorded = self._check_invert_args(latents, log_det_jac, logp)
+        if recorded:
+            from ._invgrad import glow_invert
+            return glow_invert(self, latents, temperature, log_det_jac, logp)
+        return self.invert(latents, temperature, log_det_jac, logp), log_det_jac, logp
+
     def _invert_walk(self, latents, temperature: float, ready: bool, with_ld: bool = False, with_lp: bool = False,
                      level=None, eps_sink: Optional[list] = None):
         """latents -> (x, (ld_part, R_ld, lp_part, R_lp)): the levels deepest first.  Each level runs its K inverse
         StepFlows with the kernels of its `_level_mode` (as `_transform_walk`) and unsqueezes into the first half of the
         previous level's state, whose Split fills the second half with the supplied latent or a draw from its conditional
         prior.  The partials are written only when requested (``with_ld`` / ``with_lp``).
-        ``level(mode, flows, src, B, C, h, w) -> state`` replaces the no-grad kernels of a level (the recorded inverse keeps
-        the operands of every step); ``eps_sink`` receives (assembled Split state, eps of its draw or None) per Split."""
+        ``level(mode, flows, src, B, C, h, w, ld_part, row) -> (state, rows)`` replaces the no-grad kernels of a level (the
+        recorded inverse keeps the operands of every step) and writes the log-det partial rows the no-grad level function
+        of ``mode`` writes; ``eps_sink`` receives (assembled Split state, eps of its draw or None) per Split."""
         z_last = E.check_input(latents[-1], "latents[-1]")
         B, _, h, w = z_last.shape
         H, W = h << self.L, w << self.L
@@ -567,9 +599,9 @@ class Glow(Transform):
             mode = self._level_mode(B, C, h, w) if fused else "unfused"
             if level is None:          # (the deepest level's input is caller memory: `own` False, only read)
                 st, rows = run[mode](flows, st, li < self.L - 1, B, C, h, w, ld_part, row)
-                row += rows
             else:
-                st = level(mode, flows, st, B, C, h, w)
+                st, rows = level(mode, flows, st, B, C, h, w, ld_part, row)
+            row += rows
             # undo the squeeze of this level into the first half of the previous level's state (the image at level 0)
             Cn = C // 4 if li == 0 else C // 2
             nxt = torch.empty(B, Cn, 2 * h, 2 * w, dtype=torch.float32, device=dev)
@@ -583,8 +615,7 @@ class Glow(Transform):
                 lrow += N.ld_tiles(4 * h * w)
                 if eps_sink is not None:
                     eps_sink.append((nxt, drawn[0] if drawn else None))
-        assert lrow == R_lp and (row == R_ld or level is not None), \
-            f"wrote {row} / {lrow} partial rows, allotted {R_ld} / {R_lp}"
+        assert (row, lrow) == (R_ld, R_lp), f"wrote {row} / {lrow} partial rows, allotted {R_ld} / {R_lp}"
         return st, parts
 
     def _invert_level_image(self, flows, src, own: bool, B: int, C: int, h: int, w: int, ld_part, row: int):
