@@ -166,6 +166,23 @@ int nfdpm_split_prior_logp(const float* h, int64_t ldh, const float* bias, const
 int nfdpm_split_prior_sample(const float* h, int64_t ldh, const float* bias, const float* logs, const float* eps,
                              float temperature, float* y, int64_t y_bstride, int B, int C, int H, int W,
                              nfdpm_stream_t stream);
+/* nfdpm_split_prior_sample with per-image temperatures and seeded draws.  Exactly one of eps / seeds is given.
+ *   temp_b   fp32 [B]: the temperature of image b (NULL: `temperature` for every image)
+ *   seeds    int64 [B]: the draw of image b is a pure function of (seeds[b], stream_id, element index), independent of the
+ *            batch, the image's position in it and any earlier draw (contract below); NULL: read eps as above
+ *   stream_id the draw site (Glow: the level of the Split; a stand-alone Split or GlowBlock: 0; GaussianPrior: 0xFFFFFFFF);
+ *            must be 0 without seeds
+ *   eps_out  [B,C/2,P] contiguous (may be NULL; needs seeds): receives the drawn standard normals
+ * Draw contract (Philox4x32-10 of <curand_philox4x32_x.h>, full-precision logf / sincospif):
+ *   key = (lo32(s), hi32(s)) with s = seeds[b] as uint64;  counter = (e >> 2, stream_id, 0, 0), e = c*P + p the element's
+ *   index in the image's drawn tensor [C_draw, H, W];  u_i = fp32((w_i >> 8) + 0.5) * 2^-24 for the four output words
+ *   (in (0, 1]: the +0.5 rounds to even from 2^23 on);  r = sqrtf(-2 logf(u_even)), sincospif(2 u_odd):
+ *   n_even = r*cos, n_odd = r*sin for the pairs (w0, w1), (w2, w3);  element e takes n[e & 3].
+ * With NULL new arguments the result is nfdpm_split_prior_sample's bit for bit. */
+int nfdpm_split_prior_sample_ex(const float* h, int64_t ldh, const float* bias, const float* logs, const float* eps,
+                                const int64_t* seeds, uint32_t stream_id, float temperature, const float* temp_b,
+                                float* eps_out, float* y, int64_t y_bstride, int B, int C, int H, int W,
+                                nfdpm_stream_t stream);
 
 /* GaussianPrior (prior.py:70-99): the reference convolves an all-zero map, so mean/logs are the
  * per-channel constants (bias*exp(3*logs))[0:C] and [C:2C] of the 2C-channel ZeroConv2d.
@@ -174,6 +191,11 @@ int nfdpm_gauss_logp_const(const float* z, const float* bias, const float* logs,
                            int P, nfdpm_stream_t stream);
 int nfdpm_gauss_sample_const(const float* eps, const float* bias, const float* logs, float temperature, float* out,
                              int B, int C, int P, nfdpm_stream_t stream);
+/* nfdpm_gauss_sample_const with temp_b / seeds / stream_id / eps_out as in nfdpm_split_prior_sample_ex (the drawn tensor
+ * of image b is out[b], [C, P]; GaussianPrior.sample draws with stream_id 0xFFFFFFFF).  NULL new arguments: the old bits. */
+int nfdpm_gauss_sample_const_ex(const float* eps, const int64_t* seeds, uint32_t stream_id, const float* bias,
+                                const float* logs, float temperature, const float* temp_b, float* eps_out, float* out, int B,
+                                int C, int P, nfdpm_stream_t stream);
 
 /* Fused step boundary (one CTA per image; P = H*W <= 256 and the image must fit in shared memory, see
  * nfdpm_flow_boundary_smem): source -> [affine coupling with pm] -> [channel mix] -> NCHW state and/or im2col rows.
@@ -337,6 +359,11 @@ int nfdpm_split_sample_bwd(const float* dz, int64_t dz_bs, const float* eps, flo
 int nfdpm_split_sample_bwd_lp(const float* dz, int64_t dz_bs, const float* dlp, const float* eps, float temperature,
                               const float* h, int64_t ldh, const float* bias, const float* logs, float* dh, float* dpar,
                               int B, int C, int H, int W, nfdpm_stream_t stream);
+/* nfdpm_split_sample_bwd_lp with a per-image temperature: temp_b fp32 [B] (may be NULL: `temperature` for every image, the
+ * old bits).  eps is the draw the forward used (eps_out of a seeded draw). */
+int nfdpm_split_sample_bwd_ex(const float* dz, int64_t dz_bs, const float* eps, float temperature, const float* temp_b,
+                              const float* dlp, const float* h, int64_t ldh, const float* bias, const float* logs, float* dh,
+                              float* dpar, int B, int C, int H, int W, nfdpm_stream_t stream);
 /* dstate[b,c,p] += col2im(da)[b,c,p] for c < Cin (input gradient of a 3x3 "same" conv expressed as im2col rows). */
 int nfdpm_col2im_add(const float* da, int64_t lda, float* dstate, int64_t dbs, int B, int Cin, int H, int W,
                      nfdpm_stream_t stream);

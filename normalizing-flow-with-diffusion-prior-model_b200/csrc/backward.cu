@@ -924,15 +924,18 @@ __global__ void __launch_bounds__(256) gauss_const_bwd_kernel(const float* __res
 // written along consecutive channels; per-channel partials are combined over the row groups in a fixed order
 // (deterministic).  Writes dh rows [M, ldh] (columns C..ldh zero) when h is given, and dpar [B][2C] (dbias[C], dlogs[C]).
 // dlp (may be null): gradient of the draw's log-density sum -(log(2 pi) + 2 lg + T^2 eps^2)/2 at fixed eps, which is
-// -dlp[b] on every lg and nothing on the mean.
+// -dlp[b] on every lg and nothing on the mean.  temp_b (may be null): per-image temperature T = temp_b[b] instead of
+// `temperature`.
 __global__ void __launch_bounds__(256) split_sample_bwd_kernel(const float* __restrict__ dz, int64_t dz_bs,
                                                                const float* __restrict__ dlp,
                                                                const float* __restrict__ eps, float temperature,
+                                                               const float* __restrict__ temp_b,
                                                                const float* __restrict__ h, int64_t ldh,
                                                                const float* __restrict__ bias, const float* __restrict__ logs,
                                                                float* __restrict__ dh, float* __restrict__ dpar, int C, int P) {
   __shared__ float red[4][256];
   const int Ch = C >> 1, b = blockIdx.x, tid = threadIdx.x;
+  const float T = (temp_b != nullptr) ? temp_b[b] : temperature;
   for (int j0 = 0; j0 < Ch; j0 += 256) {
     const int cw = min(256, Ch - j0), rg = 256 / cw;
     const int jl = tid % cw, r = tid / cw, j = j0 + jl;
@@ -945,7 +948,7 @@ __global__ void __launch_bounds__(256) split_sample_bwd_kernel(const float* __re
         const float hm = (h != nullptr) ? h[m * ldh + j] : 0.f, hl = (h != nullptr) ? h[m * ldh + Ch + j] : 0.f;
         const float mean = (hm + bm) * em, lg = (hl + bl) * el;
         const float g = dz[b * dz_bs + (int64_t)j * P + p];
-        float dlg = g * expf(lg) * temperature * eps[((int64_t)b * Ch + j) * P + p];
+        float dlg = g * expf(lg) * T * eps[((int64_t)b * Ch + j) * P + p];
         if (dlp != nullptr) dlg -= dlp[b];
         const float dhm = g * em, dhl = dlg * el;
         if (h != nullptr) {
@@ -1346,6 +1349,19 @@ extern "C" int nfdpm_gauss_const_bwd(const float* dl, const float* z, const floa
   return 0;
 }
 
+extern "C" int nfdpm_split_sample_bwd_ex(const float* dz, int64_t dz_bs, const float* eps, float temperature,
+                                         const float* temp_b, const float* dlp, const float* h, int64_t ldh,
+                                         const float* bias, const float* logs, float* dh, float* dpar, int B, int C, int H,
+                                         int W, nfdpm_stream_t stream) {
+  NFDPM_REQUIRE(dz && eps && bias && logs && dpar, "nfdpm_split_sample_bwd_ex: null pointer");
+  NFDPM_REQUIRE(h == nullptr || (dh && ldh >= C), "nfdpm_split_sample_bwd_ex: the conditional form needs dh with ldh >= C");
+  NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_sample_bwd_ex: bad shape");
+  split_sample_bwd_kernel<<<B, 256, 0, as_stream(stream)>>>(dz, dz_bs, dlp, eps, temperature, temp_b, h, ldh, bias, logs, dh,
+                                                            dpar, C, H * W);
+  NFDPM_CHECK_LAUNCH("split_sample_bwd_kernel");
+  return 0;
+}
+
 extern "C" int nfdpm_split_sample_bwd_lp(const float* dz, int64_t dz_bs, const float* dlp, const float* eps,
                                          float temperature, const float* h, int64_t ldh, const float* bias,
                                          const float* logs, float* dh, float* dpar, int B, int C, int H, int W,
@@ -1353,10 +1369,7 @@ extern "C" int nfdpm_split_sample_bwd_lp(const float* dz, int64_t dz_bs, const f
   NFDPM_REQUIRE(dz && eps && bias && logs && dpar, "nfdpm_split_sample_bwd_lp: null pointer");
   NFDPM_REQUIRE(h == nullptr || (dh && ldh >= C), "nfdpm_split_sample_bwd_lp: the conditional form needs dh with ldh >= C");
   NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_sample_bwd_lp: bad shape");
-  split_sample_bwd_kernel<<<B, 256, 0, as_stream(stream)>>>(dz, dz_bs, dlp, eps, temperature, h, ldh, bias, logs, dh, dpar,
-                                                            C, H * W);
-  NFDPM_CHECK_LAUNCH("split_sample_bwd_kernel");
-  return 0;
+  return nfdpm_split_sample_bwd_ex(dz, dz_bs, eps, temperature, nullptr, dlp, h, ldh, bias, logs, dh, dpar, B, C, H, W, stream);
 }
 
 extern "C" int nfdpm_split_sample_bwd(const float* dz, int64_t dz_bs, const float* eps, float temperature, const float* h,
@@ -1365,7 +1378,8 @@ extern "C" int nfdpm_split_sample_bwd(const float* dz, int64_t dz_bs, const floa
   NFDPM_REQUIRE(dz && eps && bias && logs && dpar, "nfdpm_split_sample_bwd: null pointer");
   NFDPM_REQUIRE(h == nullptr || (dh && ldh >= C), "nfdpm_split_sample_bwd: the conditional form needs dh with ldh >= C");
   NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_sample_bwd: bad shape");
-  return nfdpm_split_sample_bwd_lp(dz, dz_bs, nullptr, eps, temperature, h, ldh, bias, logs, dh, dpar, B, C, H, W, stream);
+  return nfdpm_split_sample_bwd_ex(dz, dz_bs, eps, temperature, nullptr, nullptr, h, ldh, bias, logs, dh, dpar, B, C, H, W,
+                                   stream);
 }
 
 extern "C" int nfdpm_col2im_add(const float* da, int64_t lda, float* dstate, int64_t dbs, int B, int Cin, int H, int W,

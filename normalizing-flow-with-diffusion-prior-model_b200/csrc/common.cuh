@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
+#include <curand_philox4x32_x.h>   // header-only device code: no libcurand link
 
 #include "../../include/nfdpm_b200.h"
 
@@ -128,6 +129,29 @@ static inline FastDiv make_fastdiv(int d) {
   return f;
 }
 __device__ __forceinline__ int fdiv(int n, const FastDiv f) { return f.m ? (int)__umulhi((uint32_t)n, f.m) : n; }
+
+// Counter-based standard normal draw: a pure function of (seed of the image, draw site, element index), so a sample does not
+// depend on its batch, its position in it, earlier draws or graph replays.  The contract (include/nfdpm_b200.h, DESIGN §4;
+// tests/test_seeded_sampling_cpu.py holds a numpy oracle of it):
+//   key     = (lo32(seed), hi32(seed)), seed = the image's int64 seed reinterpreted as uint64
+//   counter = (e >> 2, stream, 0, 0), e = c*P + p the element's index in the image's drawn tensor [C_draw, H, W]
+//   w0..w3  = Philox4x32-10(counter, key)
+//   u_i     = fp32((w_i >> 8) + 0.5) * 2^-24: in (0, 1]; the +0.5 is exact below 2^23 and rounds to even above, so
+//             u = 1 is possible (probability 2^-24) and gives a zero normal, never a NaN or an infinity
+//   r = sqrtf(-2 logf(u_even)); sincospif(2 u_odd) -> n_even = r*cos, n_odd = r*sin, for (w0, w1) and (w2, w3)
+//   element e takes n[e & 3]
+__device__ __forceinline__ float philox_normal(uint64_t seed, uint32_t stream, uint32_t e) {
+  const uint4 w = curand_Philox4x32_10(make_uint4(e >> 2, stream, 0u, 0u),
+                                       make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+  const bool hi = (e & 2u) != 0u;
+  const uint32_t we = hi ? w.z : w.x, wo = hi ? w.w : w.y;
+  const float ue = ((float)(we >> 8) + 0.5f) * 0x1p-24f;
+  const float uo = ((float)(wo >> 8) + 0.5f) * 0x1p-24f;
+  const float r = sqrtf(-2.f * logf(ue));
+  float s, c;
+  sincospif(2.f * uo, &s, &c);
+  return (e & 1u) ? r * s : r * c;
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -231,6 +231,8 @@ __global__ void __launch_bounds__(TPB) coupling_apply_kernel(const float* __rest
 }
 
 // Split prior: mean/logs from the raw ZeroConv GEMM rows h [M, ldh] (column = co), z = x[:, C/2:].
+// SAMPLE: y[:, C/2:] = mean + exp(lg)*T*eps with T = temp_b[b] (temp_b != NULL) or `temperature`, and eps read from `eps`
+// or, with `seeds`, drawn by philox_normal(seeds[b], stream_id, j*P + p) and copied to eps_out (may be NULL).
 template <bool SAMPLE>
 __global__ void __launch_bounds__(TPB) split_prior_kernel(const float* __restrict__ h, int64_t ldh,
                                                           const float* __restrict__ bias,
@@ -238,6 +240,9 @@ __global__ void __launch_bounds__(TPB) split_prior_kernel(const float* __restric
                                                           const float* __restrict__ x, int64_t xbs,
                                                           float* __restrict__ z_out, float* __restrict__ logp_part,
                                                           const float* __restrict__ eps, float temperature,
+                                                          const float* __restrict__ temp_b,
+                                                          const int64_t* __restrict__ seeds, uint32_t stream_id,
+                                                          float* __restrict__ eps_out,
                                                           float* __restrict__ y, int64_t ybs, int B, int C, int P) {
   __shared__ float sh[TPB];
   extern __shared__ __align__(16) float s_par[];  // [2*C]
@@ -264,8 +269,25 @@ __global__ void __launch_bounds__(TPB) split_prior_kernel(const float* __restric
         lg = (hr[Ch + j] + s_par[Ch + j]) * s_par[C + Ch + j];
       }
       if (SAMPLE) {
-        const float e = eps[(b * Ch + j) * (int64_t)P + p];
-        y[b * ybs + (int64_t)(Ch + j) * P + p] = mean + (expf(lg) * temperature) * e;
+        const int64_t ie = (b * Ch + j) * (int64_t)P + p;
+        float e;
+        if (seeds != nullptr) {
+          e = philox_normal((uint64_t)seeds[b], stream_id, (uint32_t)(j * P + p));
+          if (eps_out != nullptr) eps_out[ie] = e;
+        } else {
+          e = eps[ie];
+        }
+        const float T = (temp_b != nullptr) ? temp_b[b] : temperature;
+        // mean + exp(lg)*T*e with the roundings spelled out, so that the register draw and the loaded eps give the same
+        // bits (left to contraction, the two branches fused different products): fma(h + bias, exp(3 logs), exp(lg)*T*e)
+        float v;
+        if (hr != nullptr) {
+          const float lgr = __fmul_rn(__fadd_rn(hr[Ch + j], s_par[Ch + j]), s_par[C + Ch + j]);
+          v = __fmaf_rn(__fadd_rn(hr[j], s_par[j]), s_par[C + j], __fmul_rn(__fmul_rn(expf(lgr), T), e));
+        } else {
+          v = __fmaf_rn(__fmul_rn(expf(0.f), T), e, 0.f);
+        }
+        y[b * ybs + (int64_t)(Ch + j) * P + p] = v;
       } else {
         const float z = x[b * xbs + (int64_t)(Ch + j) * P + p];
         if (z_out != nullptr) z_out[(b * Ch + j) * (int64_t)P + p] = z;
@@ -395,8 +417,26 @@ extern "C" int nfdpm_split_prior_logp(const float* h, int64_t ldh, const float* 
   NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_prior_logp: bad shape");
   const int P = H * W;
   split_prior_kernel<false><<<pix_grid(B, P), TPB, sizeof(float) * 2 * C, as_stream(stream)>>>(
-      h, ldh, bias, logs, x, xbs, z_out, logp_part, nullptr, 0.f, nullptr, 0, B, C, P);
+      h, ldh, bias, logs, x, xbs, z_out, logp_part, nullptr, 0.f, nullptr, nullptr, 0u, nullptr, nullptr, 0, B, C, P);
   NFDPM_CHECK_LAUNCH("split_prior_kernel<logp>");
+  return 0;
+}
+
+extern "C" int nfdpm_split_prior_sample_ex(const float* h, int64_t ldh, const float* bias, const float* logs,
+                                           const float* eps, const int64_t* seeds, uint32_t stream_id, float temperature,
+                                           const float* temp_b, float* eps_out, float* y, int64_t ybs, int B, int C,
+                                           int H, int W, nfdpm_stream_t stream) {
+  NFDPM_REQUIRE(y, "nfdpm_split_prior_sample_ex: null pointer");
+  NFDPM_REQUIRE((eps == nullptr) != (seeds == nullptr), "nfdpm_split_prior_sample_ex: give exactly one of eps / seeds");
+  NFDPM_REQUIRE(seeds != nullptr || (stream_id == 0 && eps_out == nullptr),
+                "nfdpm_split_prior_sample_ex: stream_id / eps_out need seeds");
+  NFDPM_REQUIRE(h == nullptr || (bias && logs && ldh >= C), "nfdpm_split_prior_sample_ex: learned prior needs bias/logs/ldh");
+  NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_prior_sample_ex: bad shape");
+  NFDPM_REQUIRE((int64_t)(C / 2) * H * W <= 0xFFFFFFFFll, "nfdpm_split_prior_sample_ex: more than 2^32 drawn elements per image");
+  const int P = H * W;
+  split_prior_kernel<true><<<pix_grid(B, P), TPB, sizeof(float) * 2 * C, as_stream(stream)>>>(
+      h, ldh, bias, logs, nullptr, 0, nullptr, nullptr, eps, temperature, temp_b, seeds, stream_id, eps_out, y, ybs, B, C, P);
+  NFDPM_CHECK_LAUNCH("split_prior_kernel<sample>");
   return 0;
 }
 
@@ -404,13 +444,8 @@ extern "C" int nfdpm_split_prior_sample(const float* h, int64_t ldh, const float
                                         const float* eps, float temperature, float* y, int64_t ybs, int B, int C,
                                         int H, int W, nfdpm_stream_t stream) {
   NFDPM_REQUIRE(eps && y, "nfdpm_split_prior_sample: null pointer");
-  NFDPM_REQUIRE(h == nullptr || (bias && logs && ldh >= C), "nfdpm_split_prior_sample: learned prior needs bias/logs/ldh");
-  NFDPM_REQUIRE(B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0, "nfdpm_split_prior_sample: bad shape");
-  const int P = H * W;
-  split_prior_kernel<true><<<pix_grid(B, P), TPB, sizeof(float) * 2 * C, as_stream(stream)>>>(
-      h, ldh, bias, logs, nullptr, 0, nullptr, nullptr, eps, temperature, y, ybs, B, C, P);
-  NFDPM_CHECK_LAUNCH("split_prior_kernel<sample>");
-  return 0;
+  return nfdpm_split_prior_sample_ex(h, ldh, bias, logs, eps, nullptr, 0u, temperature, nullptr, nullptr, y, ybs, B, C, H, W,
+                                     stream);
 }
 
 extern "C" int nfdpm_rows_to_nchw(const float* h, int64_t ldh, int mode, const float* p1, const float* p2, float* out,

@@ -284,9 +284,14 @@ __global__ void __launch_bounds__(256) gauss_logp_const_kernel(const float* __re
   if (threadIdx.x == 0) out[b] = sh[0];
 }
 
-__global__ void gauss_sample_const_kernel(const float* __restrict__ eps, const float* __restrict__ bias,
+// out = mean + exp(lg)*T*eps per channel; T = temp_b[b] or `temperature`; eps from `eps` or, with `seeds`, drawn by
+// philox_normal(seeds[b], stream_id, c*P + p) and copied to eps_out (may be NULL)
+__global__ void gauss_sample_const_kernel(const float* __restrict__ eps, const int64_t* __restrict__ seeds,
+                                          uint32_t stream_id, const float* __restrict__ bias,
                                           const float* __restrict__ logs, float temperature,
+                                          const float* __restrict__ temp_b, float* __restrict__ eps_out,
                                           float* __restrict__ out, int C, int P, int64_t n) {
+  const int64_t CP = (int64_t)C * P;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const int c = (int)((i / P) % C);
     float mean = 0.f, lg = 0.f;
@@ -294,7 +299,20 @@ __global__ void gauss_sample_const_kernel(const float* __restrict__ eps, const f
       mean = __ldg(bias + c) * expf(3.f * __ldg(logs + c));
       lg = __ldg(bias + C + c) * expf(3.f * __ldg(logs + C + c));
     }
-    out[i] = mean + (expf(lg) * temperature) * eps[i];
+    float e, T = temperature;
+    if (seeds != nullptr || temp_b != nullptr) {
+      const int64_t b = i / CP;
+      if (temp_b != nullptr) T = temp_b[b];
+      if (seeds != nullptr) {
+        e = philox_normal((uint64_t)seeds[b], stream_id, (uint32_t)(i - b * CP));
+        if (eps_out != nullptr) eps_out[i] = e;
+      } else {
+        e = eps[i];
+      }
+    } else {
+      e = eps[i];
+    }
+    out[i] = __fmaf_rn(__fmul_rn(expf(lg), T), e, mean);   // the roundings spelled out: the same bits in every branch
   }
 }
 
@@ -428,15 +446,27 @@ extern "C" int nfdpm_gauss_logp_const(const float* z, const float* bias, const f
   return 0;
 }
 
+extern "C" int nfdpm_gauss_sample_const_ex(const float* eps, const int64_t* seeds, uint32_t stream_id, const float* bias,
+                                           const float* logs, float temperature, const float* temp_b, float* eps_out,
+                                           float* out, int B, int C, int P, nfdpm_stream_t stream) {
+  NFDPM_REQUIRE(out, "nfdpm_gauss_sample_const_ex: null pointer");
+  NFDPM_REQUIRE((eps == nullptr) != (seeds == nullptr), "nfdpm_gauss_sample_const_ex: give exactly one of eps / seeds");
+  NFDPM_REQUIRE(seeds != nullptr || (stream_id == 0 && eps_out == nullptr),
+                "nfdpm_gauss_sample_const_ex: stream_id / eps_out need seeds");
+  NFDPM_REQUIRE((bias == nullptr) == (logs == nullptr), "nfdpm_gauss_sample_const_ex: bias/logs must both be set or both NULL");
+  NFDPM_REQUIRE(B > 0 && C > 0 && P > 0, "nfdpm_gauss_sample_const_ex: bad shape");
+  NFDPM_REQUIRE((int64_t)C * P <= 0xFFFFFFFFll, "nfdpm_gauss_sample_const_ex: more than 2^32 drawn elements per image");
+  const int64_t n = (int64_t)B * C * P;
+  gauss_sample_const_kernel<<<grid_for(n, 256), 256, 0, as_stream(stream)>>>(eps, seeds, stream_id, bias, logs, temperature,
+                                                                              temp_b, eps_out, out, C, P, n);
+  NFDPM_CHECK_LAUNCH("gauss_sample_const_kernel");
+  return 0;
+}
+
 extern "C" int nfdpm_gauss_sample_const(const float* eps, const float* bias, const float* logs, float temperature,
                                         float* out, int B, int C, int P, nfdpm_stream_t stream) {
   NFDPM_REQUIRE(eps && out, "nfdpm_gauss_sample_const: null pointer");
-  NFDPM_REQUIRE((bias == nullptr) == (logs == nullptr), "nfdpm_gauss_sample_const: bias/logs must both be set or both NULL");
-  NFDPM_REQUIRE(B > 0 && C > 0 && P > 0, "nfdpm_gauss_sample_const: bad shape");
-  const int64_t n = (int64_t)B * C * P;
-  gauss_sample_const_kernel<<<grid_for(n, 256), 256, 0, as_stream(stream)>>>(eps, bias, logs, temperature, out, C, P, n);
-  NFDPM_CHECK_LAUNCH("gauss_sample_const_kernel");
-  return 0;
+  return nfdpm_gauss_sample_const_ex(eps, nullptr, 0u, bias, logs, temperature, nullptr, nullptr, out, B, C, P, stream);
 }
 
 extern "C" int nfdpm_accumulate(void* acc, int acc_dtype, const float* part, int R, int B, const float* cval,

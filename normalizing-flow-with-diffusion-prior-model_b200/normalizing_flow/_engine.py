@@ -145,6 +145,39 @@ def check_acc(a: Optional[torch.Tensor], B: int, what: str) -> None:
                          f"(got {a.dtype}, shape {tuple(a.shape)})")
 
 
+def sampling_inputs(temperature, seeds: Optional[torch.Tensor], B: int, device: torch.device):
+    """The checks of the sampling keywords of a call that draws B images, before any launch.  ``temperature``: a Python
+    number, or a contiguous float32 CUDA vector [B] (one per image, no gradient); ``seeds``: None or a contiguous int64
+    CUDA vector [B].  Returns (temperature, seeds): the number unchanged when neither is a tensor (the torch-generator
+    draw with a scalar temperature), else a [B] float32 device vector (a number is broadcast) and the seeds."""
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    if seeds is not None:
+        if not isinstance(seeds, torch.Tensor):
+            raise TypeError(f"seeds must be an int64 CUDA tensor [B] (got {type(seeds).__name__})")
+        N.require_cuda(seeds, "seeds")
+        if seeds.dtype != torch.int64 or seeds.dim() != 1 or seeds.shape[0] != B or not seeds.is_contiguous():
+            raise ValueError(f"seeds must be a contiguous int64 vector of length {B} (got {seeds.dtype}, shape "
+                             f"{tuple(seeds.shape)})")
+        if seeds.device != device:
+            raise ValueError(f"seeds live on {seeds.device}, the call runs on {device}")
+    if isinstance(temperature, torch.Tensor):
+        N.require_cuda(temperature, "temperature")
+        if temperature.dtype != torch.float32 or temperature.dim() != 1 or temperature.shape[0] != B or \
+                not temperature.is_contiguous():
+            raise ValueError(f"a tensor temperature must be a contiguous float32 vector of length {B} (got "
+                             f"{temperature.dtype}, shape {tuple(temperature.shape)})")
+        if temperature.device != device:
+            raise ValueError(f"temperature lives on {temperature.device}, the call runs on {device}")
+        if temperature.requires_grad:
+            raise ValueError("temperature requires grad: sampling has no gradient with respect to the temperature")
+        return temperature, seeds
+    if seeds is None:
+        return temperature, None
+    return torch.full((B,), float(temperature), dtype=torch.float32, device=device), seeds
+
+
 def autograd_needed(x: torch.Tensor, module: torch.nn.Module) -> bool:
     if not torch.is_grad_enabled():
         return False

@@ -115,7 +115,8 @@ def _level_stash(flows, src: Tensor, mode: str, B: int, C: int, h: int, w: int, 
     return cur, recs, rows
 
 
-def invert_stash(glow, latents, temperature: float, with_ld: bool = False, with_lp: bool = False):
+def invert_stash(glow, latents, temperature, with_ld: bool = False, with_lp: bool = False,
+                 seeds: Optional[Tensor] = None):
     """Glow.invert returning (x, per-level step records, per-Split (input, eps), density partials as `_invert_walk`
     returns them).  The walk and the kernels are those of the no-grad inverse (uncaptured, ``Glow._invert_walk``), with
     `_level_stash` for each level's StepFlows; an uninitialised model takes the unfused chain, which initialises the
@@ -127,21 +128,25 @@ def invert_stash(glow, latents, temperature: float, with_ld: bool = False, with_
         steps_rec.insert(0, recs)                       # the walk runs deepest first
         return x, rows
 
-    x, parts = glow._invert_walk(latents, temperature, glow._ready(), with_ld, with_lp, level=level, eps_sink=split_rec)
+    x, parts = glow._invert_walk(latents, temperature, glow._ready(), with_ld, with_lp, level=level, eps_sink=split_rec,
+                                 seeds=seeds)
     return x, steps_rec, split_rec[::-1], parts
 
 
 class GlowInvertFn(torch.autograd.Function):
-    """(glow, temperature, n_latents, log_det_jac | None, logp | None, *latents, *parameters) -> x, or (x, log_det_jac?,
-    logp?) when an accumulator is given: the accumulators receive the density of x in place (``Glow._add_density``, as
-    the no-grad inverse) and are marked dirty; their gradients reach the log-det and Split log-p terms."""
+    """(glow, (temperature, seeds), n_latents, log_det_jac | None, logp | None, *latents, *parameters) -> x, or (x,
+    log_det_jac?, logp?) when an accumulator is given: the accumulators receive the density of x in place
+    (``Glow._add_density``, as the no-grad inverse) and are marked dirty; their gradients reach the log-det and Split log-p
+    terms.  The temperature is a number or a per-image [B] vector; with seeds the draws come from the kernels' counter-based
+    generator and are kept for the backward like torch's."""
 
     @staticmethod
-    def forward(ctx, glow, temperature, n_lat, ld, lp, *args):
+    def forward(ctx, glow, draw, n_lat, ld, lp, *args):
+        temperature, seeds = draw
         latents = [t.detach() if isinstance(t, Tensor) else t for t in args[:n_lat]]
         ctx.glow, ctx.temperature, ctx.n_lat, ctx.params = glow, temperature, n_lat, args[n_lat:]
         ctx.have_ld, ctx.have_lp = ld is not None, lp is not None
-        x, steps_rec, split_rec, parts = invert_stash(glow, latents, temperature, ld is not None, lp is not None)
+        x, steps_rec, split_rec, parts = invert_stash(glow, latents, temperature, ld is not None, lp is not None, seeds)
         ctx.rec = (steps_rec, split_rec)
         # the deepest level's first step keeps the caller's last latent: saved so that an in-place change is detected
         ctx.save_for_backward(*[t for t in args[:n_lat] if isinstance(t, Tensor)])
@@ -197,11 +202,13 @@ class GlowInvertFn(torch.autograd.Function):
         return (None, None, None, None, None) + tuple(lat_g) + tuple(par_g)
 
 
-def glow_invert(glow, latents: list, temperature: float, log_det_jac: Optional[Tensor] = None,
-                logp: Optional[Tensor] = None):
-    """The recorded Glow.invert: x, or (x, log_det_jac, logp) when an accumulator is given (``None`` stays ``None``)."""
+def glow_invert(glow, latents: list, temperature, log_det_jac: Optional[Tensor] = None,
+                logp: Optional[Tensor] = None, seeds: Optional[Tensor] = None):
+    """The recorded Glow.invert: x, or (x, log_det_jac, logp) when an accumulator is given (``None`` stays ``None``).
+    ``temperature`` / ``seeds`` as ``E.sampling_inputs`` returns them."""
     lat = [E.check_input(t, "latent") if isinstance(t, Tensor) else t for t in latents]
-    out = GlowInvertFn.apply(glow, float(temperature), len(lat), log_det_jac, logp, *lat, *glow.parameters())
+    draw = (temperature if isinstance(temperature, Tensor) else float(temperature), seeds)
+    out = GlowInvertFn.apply(glow, draw, len(lat), log_det_jac, logp, *lat, *glow.parameters())
     if log_det_jac is None and logp is None:
         return out
     out = list(out)
@@ -213,14 +220,21 @@ def glow_invert(glow, latents: list, temperature: float, log_det_jac: Optional[T
 
 # ------------------------------------------------------------------------------------------- priors
 class GaussianSampleFn(torch.autograd.Function):
-    """GaussianPrior.sample: z = bias*e^(3 logs) (mean half) + exp(log-sd half)*T*eps, per channel."""
+    """GaussianPrior.sample: z = bias*e^(3 logs) (mean half) + exp(log-sd half)*T*eps, per channel.  ``draw``: (temperature,
+    seeds) as ``E.sampling_inputs`` returns them."""
 
     @staticmethod
-    def forward(ctx, shape, temperature, bias, logs):
+    def forward(ctx, shape, draw, bias, logs):
+        temperature, seeds = draw
         B, C, H, W = shape
-        eps = torch.empty(B, C, H, W, dtype=torch.float32, device=bias.device).normal_()
+        eps = torch.empty(B, C, H, W, dtype=torch.float32, device=bias.device)
         out = torch.empty_like(eps)
-        N.gauss_sample_const(eps, bias, logs, temperature, out, B, C, H * W)
+        if seeds is None and not isinstance(temperature, Tensor):
+            N.gauss_sample_const(eps.normal_(), bias, logs, temperature, out, B, C, H * W)
+        elif seeds is None:
+            N.gauss_sample_const_ex(eps.normal_(), None, 0, bias, logs, 1.0, temperature, None, out, B, C, H * W)
+        else:
+            N.gauss_sample_const_ex(None, seeds, N.PRIOR_STREAM, bias, logs, 1.0, temperature, eps, out, B, C, H * W)
         ctx.temperature = temperature
         ctx.save_for_backward(eps, bias, logs)
         return out
@@ -231,7 +245,11 @@ class GaussianSampleFn(torch.autograd.Function):
         B, C, H, W = eps.shape
         dz = dz.to(torch.float32).contiguous()
         dpar = torch.empty(B * 4 * C, dtype=torch.float32, device=dz.device)
-        N.split_sample_bwd(dz, C * H * W, eps, ctx.temperature, None, 0, bias, logs, None, dpar, B, 2 * C, H, W)
+        if isinstance(ctx.temperature, Tensor):
+            N.split_sample_bwd_ex(dz, C * H * W, eps, 1.0, ctx.temperature, None, None, 0, bias, logs, None, dpar, B, 2 * C,
+                                  H, W)
+        else:
+            N.split_sample_bwd(dz, C * H * W, eps, ctx.temperature, None, 0, bias, logs, None, dpar, B, 2 * C, H, W)
         db, dl = torch.empty_like(bias), torch.empty_like(logs)
         N.reduce_rows2(dpar, db, dl, B, 2 * C, 2 * C, 4 * C)
         return None, None, db if ctx.needs_input_grad[2] else None, dl if ctx.needs_input_grad[3] else None

@@ -94,12 +94,12 @@ def _mix_inv_backward(mix, u: Tensor, dx: Tensor, weight, scale, bias, wgrad: bo
     return du, dW, dS, dB
 
 
-def _split_sample_backward(sp, out: Tensor, eps: Optional[Tensor], temperature: float, d_out: Tensor, wgrad: bool = True,
+def _split_sample_backward(sp, out: Tensor, eps: Optional[Tensor], temperature, d_out: Tensor, wgrad: bool = True,
                            dlp: Optional[Tensor] = None):
     """Backward of Split.invert: ``out`` = (y | z) [B,C,H,W], ``d_out`` its gradient.  Returns (dy, d_latent, grads).  A
     sampled half (``eps`` given) z = mean(y) + exp(lg(y))*T*eps back-propagates into y and the prior conv's parameters
     (nfdpm_split_sample_bwd + the conv's fp32 wgrad / dgrad GEMMs); a supplied latent receives the second half.
-    ``dlp`` ([B] fp32): gradient of the log-density log N(z; mean(y), exp(lg(y))) the inverse accumulated for this Split.
+    ``temperature``: the draw's number or per-image [B] vector.  ``dlp`` ([B] fp32): gradient of the log-density log N(z; mean(y), exp(lg(y))) the inverse accumulated for this Split.
     A sampled half takes it inside nfdpm_split_sample_bwd_lp (-dlp on lg); a supplied one through nfdpm_split_prior_bwd on
     the assembled ``out``, into the latent and, through the prior conv, into y and the conv's parameters (it adds to the
     second half of ``d_out`` in place)."""
@@ -121,8 +121,12 @@ def _split_sample_backward(sp, out: Tensor, eps: Optional[Tensor], temperature: 
         return dy, dz, g
     if conv is None:                                    # the standard-normal prior has no parameters and ignores y
         return dy, None, g
-    _prior_conv_backward(sp, out, dy, Ch * P, wgrad, g, lambda hs, ldh, dh, dpar: N.split_sample_bwd_lp(
-        d_out.view(-1)[Ch * P:], C * P, dlp, eps, temperature, hs, ldh, conv.bias, conv.logs, dh, dpar, B, C, H, W))
+    if isinstance(temperature, Tensor):                 # per-image temperatures [B]
+        _prior_conv_backward(sp, out, dy, Ch * P, wgrad, g, lambda hs, ldh, dh, dpar: N.split_sample_bwd_ex(
+            d_out.view(-1)[Ch * P:], C * P, eps, 1.0, temperature, dlp, hs, ldh, conv.bias, conv.logs, dh, dpar, B, C, H, W))
+    else:
+        _prior_conv_backward(sp, out, dy, Ch * P, wgrad, g, lambda hs, ldh, dh, dpar: N.split_sample_bwd_lp(
+            d_out.view(-1)[Ch * P:], C * P, dlp, eps, temperature, hs, ldh, conv.bias, conv.logs, dh, dpar, B, C, H, W))
     return dy, None, g
 
 
@@ -402,10 +406,12 @@ def coupling_invert_stash(cp, y: Tensor, ld_part: Optional[Tensor] = None):
 
 
 class ModuleInvertFn(torch.autograd.Function):
-    """(y, latent | None, *parameters) -> x for one granular ``invert``."""
+    """(y, latent | None, *parameters) -> x for one granular ``invert``.  ``draw``: (temperature, seeds) of a Split, as
+    ``E.sampling_inputs`` returns them."""
 
     @staticmethod
-    def forward(ctx, mod, what, raw_invert, temperature, y, latent, *params):
+    def forward(ctx, mod, what, raw_invert, draw, y, latent, *params):
+        temperature, seeds = draw
         ctx.mod, ctx.what, ctx.temperature, ctx.params = mod, what, temperature, params
         ctx.stash = ctx.eps = None
         if what == "AffineCoupling":
@@ -415,7 +421,7 @@ class ModuleInvertFn(torch.autograd.Function):
             x = torch.empty(B, 2 * Ch, H, W, dtype=torch.float32, device=y.device)
             N.copy_channels(y, x, B, Ch, H * W, Ch * H * W, 2 * Ch * H * W)
             sink = []
-            mod._fill_second_half(x, 2 * Ch * H * W, B, 2 * Ch, H, W, latent, temperature, eps_sink=sink)
+            mod._fill_second_half(x, 2 * Ch * H * W, B, 2 * Ch, H, W, latent, temperature, eps_sink=sink, seeds=seeds)
             ctx.eps = sink[0] if sink else None
             ctx.save_for_backward(y, x)
             return x
@@ -455,6 +461,12 @@ class ModuleInvertFn(torch.autograd.Function):
                 d_lat if ctx.needs_input_grad[5] else None) + tuple(pg)
 
 
-def invert(mod, what: str, raw_invert, y: Tensor, latent: Optional[Tensor] = None, temperature: float = 1.0):
+def invert(mod, what: str, raw_invert, y: Tensor, latent: Optional[Tensor] = None, temperature=1.0,
+           seeds: Optional[Tensor] = None):
     """Run ``mod.invert`` under autograd (one ModuleInvertFn node)."""
-    return ModuleInvertFn.apply(mod, what, raw_invert, float(temperature), E.check_input(y), latent, *mod.parameters())
+    y = E.check_input(y)
+    if isinstance(temperature, Tensor) or seeds is not None:
+        draw = E.sampling_inputs(temperature, seeds, y.shape[0], y.device)
+    else:
+        draw = (float(temperature), None)
+    return ModuleInvertFn.apply(mod, what, raw_invert, draw, y, latent, *mod.parameters())

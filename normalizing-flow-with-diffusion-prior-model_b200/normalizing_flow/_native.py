@@ -50,7 +50,7 @@ def _load() -> C.CDLL:
             f"libnfdpm_b200.so not found at {LIB_PATH}. Build it with `python -c 'import __graft_entry__ as g; "
             f"g.build()'` (nvcc, sm_100a). This package has no CPU or PyTorch fallback.")
     lib = C.CDLL(LIB_PATH)
-    vp, i32, i64, f32 = C.c_void_p, C.c_int, C.c_int64, C.c_float
+    vp, i32, i64, f32, u32 = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_uint32
     sig = {
         "nfdpm_version": ([], C.c_int),
         "nfdpm_last_error_string": ([], C.c_char_p),
@@ -71,6 +71,8 @@ def _load() -> C.CDLL:
         "nfdpm_split_prior_sample": ([vp, i64, vp, vp, vp, f32, vp, i64, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_gauss_logp_const": ([vp, vp, vp, vp, i32, i32, i32, vp], C.c_int),
         "nfdpm_gauss_sample_const": ([vp, vp, vp, f32, vp, i32, i32, i32, vp], C.c_int),
+        "nfdpm_split_prior_sample_ex": ([vp, i64, vp, vp, vp, vp, u32, f32, vp, vp, vp, i64, i32, i32, i32, i32, vp], C.c_int),
+        "nfdpm_gauss_sample_const_ex": ([vp, vp, u32, vp, vp, f32, vp, vp, vp, i32, i32, i32, vp], C.c_int),
         "nfdpm_rows_to_nchw": ([vp, i64, i32, vp, vp, vp, i32, i32, i32, vp], C.c_int),
         "nfdpm_nchw_to_rows": ([vp, vp, i32, i32, i32, i32, i64, i64, vp], C.c_int),
         "nfdpm_flow_boundary_smem": ([i32, i32, i32, i32, i32], C.c_size_t),
@@ -112,6 +114,7 @@ def _load() -> C.CDLL:
         "nfdpm_gauss_const_bwd": ([vp, vp, vp, vp, vp, vp, i32, i32, i32, vp], C.c_int),
         "nfdpm_split_sample_bwd": ([vp, i64, vp, f32, vp, i64, vp, vp, vp, vp, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_split_sample_bwd_lp": ([vp, i64, vp, vp, f32, vp, i64, vp, vp, vp, vp, i32, i32, i32, i32, vp], C.c_int),
+        "nfdpm_split_sample_bwd_ex": ([vp, i64, vp, f32, vp, vp, vp, i64, vp, vp, vp, vp, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_col2im_add": ([vp, i64, vp, i64, i32, i32, i32, i32, vp], C.c_int),
         "nfdpm_accumulate": ([vp, i32, vp, i32, i32, vp, vp, i32, vp], C.c_int),
         "nfdpm_flow_boundary_tiles": ([i32, i32, i32, i32, i32, i32, i32], C.c_int),
@@ -191,7 +194,8 @@ EXPORTS = ["nfdpm_version", "nfdpm_last_error_string", "nfdpm_sm_count", "nfdpm_
            "nfdpm_latent_format", "nfdpm_postprocess_u8", "nfdpm_preprocess",
            "nfdpm_flow_boundary_tiles", "nfdpm_flow_boundary_tiled",
            "nfdpm_coupling_inv_bwd", "nfdpm_mix_inv_param_grad", "nfdpm_split_sample_bwd", "nfdpm_flow_boundary_inv_stash",
-           "nfdpm_coupling_inv_bwd_ld", "nfdpm_flow_boundary_inv_stash_ld", "nfdpm_split_sample_bwd_lp"]
+           "nfdpm_coupling_inv_bwd_ld", "nfdpm_flow_boundary_inv_stash_ld", "nfdpm_split_sample_bwd_lp",
+           "nfdpm_split_prior_sample_ex", "nfdpm_gauss_sample_const_ex", "nfdpm_split_sample_bwd_ex"]
 
 #: number of kernels launched through this binding (bench.py reports it as ``gpu_launches``)
 launch_count = 0
@@ -289,6 +293,23 @@ def split_prior_logp(h, ldh, bias, logs, x, xbs, z_out, logp_part, B, Cc, H, W) 
 def split_prior_sample(h, ldh, bias, logs, eps, temperature, y, ybs, B, Cc, H, W) -> None:
     _ok(lib.nfdpm_split_prior_sample(_p(h), ldh, _p(bias), _p(logs), _p(eps), float(temperature), _p(y), ybs, B, Cc,
                                      H, W, _st()))
+
+
+#: draw site of GaussianPrior.sample in the seeded-draw contract (include/nfdpm_b200.h); a Split uses its level
+PRIOR_STREAM = 0xFFFFFFFF
+
+
+def split_prior_sample_ex(h, ldh, bias, logs, eps, seeds, stream_id, temperature, temp_b, eps_out, y, ybs, B, Cc, H,
+                          W) -> None:
+    """``split_prior_sample`` with a per-image temperature ``temp_b`` and/or seeded draws (``seeds``, ``stream_id``; the
+    draws go to ``eps_out`` when given).  Exactly one of ``eps`` / ``seeds``."""
+    _ok(lib.nfdpm_split_prior_sample_ex(_p(h), ldh, _p(bias), _p(logs), _p(eps), _p(seeds), int(stream_id),
+                                        float(temperature), _p(temp_b), _p(eps_out), _p(y), ybs, B, Cc, H, W, _st()))
+
+
+def gauss_sample_const_ex(eps, seeds, stream_id, bias, logs, temperature, temp_b, eps_out, out, B, Cc, P) -> None:
+    _ok(lib.nfdpm_gauss_sample_const_ex(_p(eps), _p(seeds), int(stream_id), _p(bias), _p(logs), float(temperature),
+                                        _p(temp_b), _p(eps_out), _p(out), B, Cc, P, _st()))
 
 
 def gauss_logp_const(z, bias, logs, part, B, Cc, P) -> None:
@@ -452,6 +473,11 @@ def split_sample_bwd(dz, dz_bs, eps, temperature, h, ldh, bias, logs, dh, dpar, 
 def split_sample_bwd_lp(dz, dz_bs, dlp, eps, temperature, h, ldh, bias, logs, dh, dpar, B, Cc, H, W) -> None:
     _ok(lib.nfdpm_split_sample_bwd_lp(_p(dz), dz_bs, _p(dlp), _p(eps), float(temperature), _p(h), ldh, _p(bias), _p(logs),
                                       _p(dh), _p(dpar), B, Cc, H, W, _st()))
+
+
+def split_sample_bwd_ex(dz, dz_bs, eps, temperature, temp_b, dlp, h, ldh, bias, logs, dh, dpar, B, Cc, H, W) -> None:
+    _ok(lib.nfdpm_split_sample_bwd_ex(_p(dz), dz_bs, _p(eps), float(temperature), _p(temp_b), _p(dlp), _p(h), ldh, _p(bias),
+                                      _p(logs), _p(dh), _p(dpar), B, Cc, H, W, _st()))
 
 
 def col2im_add(da, lda, dstate, dbs, B, Cin, H, W) -> None:

@@ -122,8 +122,10 @@ class GlowBlock(Transform):
             y, log_det_jac, logp = flow.transform(y, log_det_jac, logp)
         return self.split.transform(y, log_det_jac, logp)
 
-    def invert(self, y: Tensor, latent: Tensor = None, temperature: float = 1.0) -> Tensor:
-        inv = self.split.invert(y, latent, temperature=temperature)
+    def invert(self, y: Tensor, latent: Tensor = None, temperature: float = 1.0, *,
+               seeds: Optional[Tensor] = None) -> Tensor:
+        """``temperature`` / ``seeds`` as in ``Split.invert`` (draw site 0: the draw of ``Glow`` level 0)."""
+        inv = self.split.invert(y, latent, temperature=temperature, seeds=seeds)
         for flow in reversed(self.flows):
             inv = flow.invert(inv)
         return self.squeeze.invert(inv)
@@ -474,7 +476,7 @@ class Glow(Transform):
 
     # ---- inverse: latents -> x
     def invert(self, latents: list, temperature: float = 1.0, log_det_jac: Optional[Tensor] = None,
-               logp: Optional[Tensor] = None) -> Tensor:
+               logp: Optional[Tensor] = None, *, seeds: Optional[Tensor] = None) -> Tensor:
         """latents -> x.  ``latents`` holds all L parts (decoding) or the last ones only: every Split without a latent draws
         its half from its conditional prior at ``temperature``.
 
@@ -486,10 +488,18 @@ class Glow(Transform):
                          latent's prior is not included, as in ``transform``.
         Under a temperature this is the model's density at the returned sample, not the tempered one.  The accumulated
         density is not differentiable here: a call that NFDPM_INVERT_GRAD=1 would record raises NotImplementedError.
-        ``invert_with_density`` returns the same values and back-propagates through them."""
+        ``invert_with_density`` returns the same values and back-propagates through them.
+
+        ``temperature`` may also be a float32 CUDA vector [B], one temperature per image.  ``seeds`` (int64 CUDA [B],
+        optional) makes every draw of the call a pure function of (seeds[b], level of the Split, element): image b does
+        not depend on the batch it is drawn in, its position there, earlier draws or graph replays (the contract is in
+        include/nfdpm_b200.h).  Without seeds the draws come from torch's CUDA generator.  A call that draws nothing (all
+        L latents supplied) accepts seeds and a tensor temperature and uses neither.  With seeds or a tensor temperature
+        one captured chain serves every temperature and seed vector of its shape."""
         z_last, recorded = self._check_invert_args(latents, log_det_jac, logp)
         accs = [a for a in (log_det_jac, logp) if a is not None]
         B, _, h, w = z_last.shape
+        temperature, seeds = E.sampling_inputs(temperature, seeds, B, z_last.device)
         if recorded:
             if E.invert_grad_enabled():
                 if accs:
@@ -498,40 +508,52 @@ class Glow(Transform):
                         "(NFDPM_INVERT_GRAD=1) takes no accumulators.  Call it under torch.no_grad() for the density, "
                         "or Glow.invert_with_density to back-propagate through it.")
                 from ._invgrad import glow_invert
-                return glow_invert(self, latents, temperature)
+                return glow_invert(self, latents, temperature, seeds=seeds)
             # without NFDPM_INVERT_GRAD: compute it without recording and fail loudly on back-propagation
             from .transforms import _NoBackward
             deps = [t for t in latents if isinstance(t, Tensor) and t.requires_grad] + \
                    [p for p in self.parameters() if p.requires_grad]
             with torch.no_grad():
                 out = self.invert([t.detach() if isinstance(t, Tensor) else t for t in latents], temperature,
-                                  log_det_jac, logp)
+                                  log_det_jac, logp, seeds=seeds)
             return _NoBackward.apply(out, "Glow.invert", False, *deps)
         with_ld, with_lp = log_det_jac is not None, logp is not None
         ready = self._ready()
         H, W = h << self.L, w << self.L
         if self._use_graph(ready) and 1 <= len(latents) <= self.L and all(isinstance(t, Tensor) for t in latents):
             # decoding (all L latents supplied) and sampling (fewer: every Split without a latent draws its half from the
-            # learned conditional prior, transforms.py:305-307) replay one captured chain; the normal draws inside a
-            # captured chain come from torch's default CUDA generator, whose Philox offset advances on every replay
+            # learned conditional prior, transforms.py:305-307) replay one captured chain; without seeds the normal draws
+            # inside a captured chain come from torch's default CUDA generator, whose Philox offset advances on every
+            # replay, and with seeds the prior kernels draw from the static seed vector
             lat_in = [E.check_input(t, "latent") for t in latents]
             sampling = len(latents) < self.L
+            # seeds or per-image temperatures: the [B] vectors are static inputs of the chain, so its key has no temperature
+            ex = sampling and isinstance(temperature, Tensor)
             key = ("inv", B, h, w, E.precision(), z_last.device.index)
-            if sampling:
+            if ex:
+                key += (len(latents), "ex", seeds is not None)
+            elif sampling:
                 key += (len(latents), float(temperature))
             if with_ld or with_lp:                    # a chain that also writes the density partials
                 key += ((with_ld, with_lp),)
-            if key not in self._graphs and sampling:
+            if key not in self._graphs and sampling and not ex:
                 # the temperature is baked into a sampling graph: keep at most four of them (a temperature sweep would
                 # otherwise pin one captured chain and its workspace per value)
-                old = [k for k in self._graphs if k[0] == "inv" and len(k) >= 8]
+                old = [k for k in self._graphs if k[0] == "inv" and len(k) >= 8 and k[7] != "ex"]
                 for k in old[:max(0, len(old) - 3)]:
                     E.WS.drop_scope(("glow", id(self), k))
                     del self._graphs[k]
-            x, parts = self._replay(key, lat_in, lambda lat: self._invert_walk(lat, temperature, True, with_ld, with_lp))
+            n = len(lat_in)
+            if ex:
+                ins = lat_in + [temperature] + ([seeds] if seeds is not None else [])
+                walk = lambda st: self._invert_walk(st[:n], st[n], True, with_ld, with_lp,
+                                                    seeds=st[n + 1] if len(st) > n + 1 else None)
+            else:
+                ins, walk = lat_in, lambda lat: self._invert_walk(lat, temperature, True, with_ld, with_lp)
+            x, parts = self._replay(key, ins, walk)
             self._add_density(log_det_jac, logp, parts, H, W)     # after the replay, into the caller's tensors
             return x.clone()
-        x, parts = self._invert_walk(latents, temperature, ready, with_ld, with_lp)
+        x, parts = self._invert_walk(latents, temperature, ready, with_ld, with_lp, seeds=seeds)
         self._add_density(log_det_jac, logp, parts, H, W)
         return x
 
@@ -550,7 +572,8 @@ class Glow(Transform):
         return z_last, E.autograd_needed(z_last, self) or any(isinstance(t, Tensor) and t.requires_grad for t in latents)
 
     def invert_with_density(self, latents: list, temperature: float = 1.0, log_det_jac: Optional[Tensor] = None,
-                            logp: Optional[Tensor] = None) -> Tuple[Tensor, Optional[Tensor], Optional[Tensor]]:
+                            logp: Optional[Tensor] = None, *,
+                            seeds: Optional[Tensor] = None) -> Tuple[Tensor, Optional[Tensor], Optional[Tensor]]:
         """``invert(latents, temperature, log_det_jac, logp)`` returning ``(x, log_det_jac, logp)``, differentiable in all
         three: the density of generated images as a function of the latents and the weights (reverse-KL / variational
         training, entropy terms, distillation through the flow).  The arguments and the accumulated values are exactly
@@ -561,24 +584,27 @@ class Glow(Transform):
         dirty, like ``transform``'s): gradients reach the latents, every StepFlow parameter and every Split prior conv,
         at sampled Splits (through the draw and its log-density) and at supplied ones (through the log-density).  It
         records whether or not NFDPM_INVERT_GRAD is set: that knob guards ``invert``, ``sample`` and the granular inverses,
-        whose callers did not ask for a graph.  The recorded call is not captured in a CUDA graph."""
+        whose callers did not ask for a graph.  The recorded call is not captured in a CUDA graph.  ``temperature`` /
+        ``seeds`` as in ``invert``; the backward uses each image's temperature and the draws the forward made."""
         if log_det_jac is None and logp is None:
             raise ValueError("Glow.invert_with_density needs log_det_jac and/or logp; Glow.invert returns the images alone")
-        _, recorded = self._check_invert_args(latents, log_det_jac, logp)
+        z_last, recorded = self._check_invert_args(latents, log_det_jac, logp)
         if recorded:
+            temperature, seeds = E.sampling_inputs(temperature, seeds, z_last.shape[0], z_last.device)
             from ._invgrad import glow_invert
-            return glow_invert(self, latents, temperature, log_det_jac, logp)
-        return self.invert(latents, temperature, log_det_jac, logp), log_det_jac, logp
+            return glow_invert(self, latents, temperature, log_det_jac, logp, seeds)
+        return self.invert(latents, temperature, log_det_jac, logp, seeds=seeds), log_det_jac, logp
 
-    def _invert_walk(self, latents, temperature: float, ready: bool, with_ld: bool = False, with_lp: bool = False,
-                     level=None, eps_sink: Optional[list] = None):
+    def _invert_walk(self, latents, temperature, ready: bool, with_ld: bool = False, with_lp: bool = False,
+                     level=None, eps_sink: Optional[list] = None, seeds: Optional[Tensor] = None):
         """latents -> (x, (ld_part, R_ld, lp_part, R_lp)): the levels deepest first.  Each level runs its K inverse
         StepFlows with the kernels of its `_level_mode` (as `_transform_walk`) and unsqueezes into the first half of the
         previous level's state, whose Split fills the second half with the supplied latent or a draw from its conditional
         prior.  The partials are written only when requested (``with_ld`` / ``with_lp``).
         ``level(mode, flows, src, B, C, h, w, ld_part, row) -> (state, rows)`` replaces the no-grad kernels of a level (the
         recorded inverse keeps the operands of every step) and writes the log-det partial rows the no-grad level function
-        of ``mode`` writes; ``eps_sink`` receives (assembled Split state, eps of its draw or None) per Split."""
+        of ``mode`` writes; ``eps_sink`` receives (assembled Split state, eps of its draw or None) per Split.
+        ``temperature``: a number or a [B] device vector; ``seeds``: the Split of level l draws with draw site l."""
         z_last = E.check_input(latents[-1], "latents[-1]")
         B, _, h, w = z_last.shape
         H, W = h << self.L, w << self.L
@@ -611,7 +637,8 @@ class Glow(Transform):
                 drawn = [] if eps_sink is not None else None
                 geo[li - 1][1]._fill_second_half(nxt, Cn * 4 * h * w, B, Cn, 2 * h, 2 * w,
                                                  get_item(latents, li - self.L - 1), temperature, eps_sink=drawn,
-                                                 logp_part=lp_part[lrow * B:] if lp_part is not None else None)
+                                                 logp_part=lp_part[lrow * B:] if lp_part is not None else None,
+                                                 seeds=seeds, stream_id=li - 1)
                 lrow += N.ld_tiles(4 * h * w)
                 if eps_sink is not None:
                     eps_sink.append((nxt, drawn[0] if drawn else None))
@@ -687,12 +714,13 @@ class Glow(Transform):
 
     @torch.no_grad()
     def sample(self, latents: list, postprocess_func=None, temperature: float = 1.0,
-               log_det_jac: Optional[Tensor] = None, logp: Optional[Tensor] = None) -> Tensor:
+               log_det_jac: Optional[Tensor] = None, logp: Optional[Tensor] = None, *,
+               seeds: Optional[Tensor] = None) -> Tensor:
         """eval() -> invert -> optional postprocess -> train(), like the reference (glow.py:230-246; note the
         unconditional switch back to train mode).  ``log_det_jac`` / ``logp`` as in ``invert``: the density of the
-        continuous sample before ``postprocess_func``."""
+        continuous sample before ``postprocess_func``.  ``temperature`` / ``seeds`` as in ``invert``."""
         self.eval()
-        new_samples = self.invert(latents, temperature, log_det_jac, logp)
+        new_samples = self.invert(latents, temperature, log_det_jac, logp, seeds=seeds)
         out = postprocess_func(new_samples.float()) if postprocess_func else new_samples.float()
         self.train()
         return out

@@ -97,18 +97,29 @@ class GaussianPrior(Prior):
         N.gauss_logp_const(x, bias, logs, out, B, C, H * W)
         return out
 
-    def sample(self, shape: tuple = None, temperature: float = 1.0) -> Tensor:
+    def sample(self, shape: tuple = None, temperature: float = 1.0, *, seeds: Optional[Tensor] = None) -> Tensor:
+        """A [B, C, H, W] draw at ``temperature`` (a number, or a float32 CUDA vector [B]: one per image).  ``seeds``
+        (int64 CUDA [B], optional): image b is a pure function of seeds[b] (draw site 0xFFFFFFFF of the counter-based
+        generator, include/nfdpm_b200.h), whatever the batch; without seeds torch's CUDA generator draws."""
         B, C, H, W = shape
         if C != self._C:
             raise ValueError(f"GaussianPrior built for {self._C} channels got {C}")
         dev = self.__conv.bias.device if self.__conv is not None else self.device
+        temperature, seeds = E.sampling_inputs(temperature, seeds, B, torch.device(dev))
         bias, logs = self._params()
         if E.invert_grad_enabled() and bias is not None and E.autograd_needed(bias, self):
             from ._invgrad import GaussianSampleFn
-            return GaussianSampleFn.apply((B, C, H, W), float(temperature), bias, logs)
+            T = temperature if isinstance(temperature, Tensor) else float(temperature)
+            return GaussianSampleFn.apply((B, C, H, W), (T, seeds), bias, logs)
+        out = torch.empty(B, C, H, W, dtype=torch.float32, device=dev)
+        if seeds is not None:
+            N.gauss_sample_const_ex(None, seeds, N.PRIOR_STREAM, bias, logs, 1.0, temperature, None, out, B, C, H * W)
+            return out
         eps = torch.empty(B, C, H, W, dtype=torch.float32, device=dev).normal_()
-        out = torch.empty_like(eps)
-        N.gauss_sample_const(eps, bias, logs, temperature, out, B, C, H * W)
+        if isinstance(temperature, Tensor):
+            N.gauss_sample_const_ex(eps, None, 0, bias, logs, 1.0, temperature, None, out, B, C, H * W)
+        else:
+            N.gauss_sample_const(eps, bias, logs, temperature, out, B, C, H * W)
         return out
 
 

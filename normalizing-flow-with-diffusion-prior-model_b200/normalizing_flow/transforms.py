@@ -71,7 +71,7 @@ def _granular(what: str):
                 if what == "Split":
                     latent = args[0] if len(args) > 0 else kw.get("inv_y_split")
                     temperature = args[1] if len(args) > 1 else kw.get("temperature", 1.0)
-                    return MG.invert(self, what, fn, x, latent, temperature)
+                    return MG.invert(self, what, fn, x, latent, temperature, kw.get("seeds"))
                 return MG.invert(self, what, fn, x)
             ins = [t for t in (x,) + tuple(args) + tuple(kw.values()) if isinstance(t, Tensor)]
             deps = [t for t in ins if t.requires_grad] + [p for p in self.parameters() if p.requires_grad]
@@ -327,23 +327,29 @@ class Split(Transform):
         return y, log_det_jac, z, logp
 
     @_granular("Split")
-    def invert(self, y: Tensor, inv_y_split: Tensor = None, temperature: float = 1.0) -> Tensor:
+    def invert(self, y: Tensor, inv_y_split: Tensor = None, temperature: float = 1.0, *,
+               seeds: Optional[Tensor] = None) -> Tensor:
+        """``temperature``: a number or a float32 CUDA vector [B] (one per image).  ``seeds`` (int64 CUDA [B], optional):
+        the draw of image b is a pure function of seeds[b] and the element (draw site 0, include/nfdpm_b200.h), the same
+        draw as level 0 of a ``Glow`` with these seeds; unused when ``inv_y_split`` is given."""
         y = E.check_input(y)
         B, Ch, H, W = y.shape
+        temperature, seeds = E.sampling_inputs(temperature, seeds, B, y.device)
         C, P = 2 * Ch, H * W
         out = torch.empty(B, C, H, W, dtype=torch.float32, device=y.device)
         N.copy_channels(y, out, B, Ch, P, Ch * P, C * P)
-        self._fill_second_half(out, C * P, B, C, H, W, inv_y_split, temperature)
+        self._fill_second_half(out, C * P, B, C, H, W, inv_y_split, temperature, seeds=seeds)
         return out
 
     def _fill_second_half(self, out: Tensor, obs: int, B: int, C: int, H: int, W: int, z: Optional[Tensor],
-                          temperature: float, eps_sink: Optional[list] = None,
-                          logp_part: Optional[Tensor] = None) -> None:
+                          temperature, eps_sink: Optional[list] = None, logp_part: Optional[Tensor] = None,
+                          seeds: Optional[Tensor] = None, stream_id: int = 0) -> None:
         """Write the latent (given, or drawn from the conditional prior, reference transforms.py:305-307 and
         prior.py:49-50) into channels C/2..C of ``out`` whose first half is already in place.  ``eps_sink`` receives the
         standard-normal tensor a draw used (the inverse's backward needs it).  ``logp_part`` receives the partials of
         log N(z; mean, exp(logs)) of the written half, as ``transform`` writes them (the model's density, whatever the
-        temperature of a draw)."""
+        temperature of a draw).  ``temperature``: a number or a checked [B] device vector (``E.sampling_inputs``);
+        ``seeds``: draw in the kernel from (seeds[b], ``stream_id``, element) instead of torch's generator."""
         Ch, P = C // 2, H * W
         second = out.view(-1)[Ch * P:]
         bias = self.conv.bias if self.conv is not None else None
@@ -357,10 +363,19 @@ class Split(Transform):
                 h, ldh = E.split_rows(self, out, obs, B, C, H, W)
                 N.split_prior_logp(h, ldh, bias, logs, out, obs, None, logp_part, B, C, H, W)
             return
-        eps = torch.empty(B, Ch, H, W, dtype=torch.float32, device=out.device).normal_()
+        temp_b = temperature if isinstance(temperature, Tensor) else None
+        if seeds is None:
+            eps = torch.empty(B, Ch, H, W, dtype=torch.float32, device=out.device).normal_()
+        else:                               # the kernel draws; the draws are kept only for a backward
+            eps = torch.empty(B, Ch, H, W, dtype=torch.float32, device=out.device) if eps_sink is not None else None
         if eps_sink is not None:
             eps_sink.append(eps)
         h, ldh = E.split_rows(self, out, obs, B, C, H, W)
-        N.split_prior_sample(h, ldh, bias, logs, eps, temperature, out, obs, B, C, H, W)
+        if seeds is None and temp_b is None:
+            N.split_prior_sample(h, ldh, bias, logs, eps, temperature, out, obs, B, C, H, W)
+        elif seeds is None:
+            N.split_prior_sample_ex(h, ldh, bias, logs, eps, None, 0, 1.0, temp_b, None, out, obs, B, C, H, W)
+        else:
+            N.split_prior_sample_ex(h, ldh, bias, logs, None, seeds, stream_id, 1.0, temp_b, eps, out, obs, B, C, H, W)
         if logp_part is not None:           # the prior conv rows h of the draw serve the density too
             N.split_prior_logp(h, ldh, bias, logs, out, obs, None, logp_part, B, C, H, W)
