@@ -81,7 +81,9 @@ typedef struct {
 int nfdpm_mix_prepare(const nfdpm_mix_item* items_host, int n, nfdpm_stream_t stream);
 
 /* K-A / K-A^-1: y[b,o,p] = sum_i mt[i*C+o]*x[b,i,p] + beta[o]  (fused ActNorm + 1x1 conv,
- * transforms.py:80 + :132 forward; :144 + :93 inverse).  x,y: [B,C,P] with batch strides. */
+ * transforms.py:80 + :132 forward; :144 + :93 inverse).  x,y: [B,C,P] with batch strides.
+ * C <= 1024; above 192 the matrix streams through shared memory in chunks (same summation order) and x, y must not
+ * overlap. */
 int nfdpm_channel_mix(const float* x, float* y, const float* mt, const float* beta, int B, int C, int P,
                       int64_t x_bstride, int64_t y_bstride, nfdpm_stream_t stream);
 
@@ -302,7 +304,8 @@ int nfdpm_reduce_rows2(const float* part, float* out0, float* out1, int R, int n
                        nfdpm_stream_t stream);
 /* Fused ActNorm + 1x1 conv backward (transforms.py:80,132) incl. col2im of the im2col-row gradient da1 (may be NULL):
  * dx = W^T du; part [B][C*C + C]: per-image sum_p du[o]x[i] and sum_p du[o]. */
-/* pixel tiles per image of nfdpm_mix_bwd: `part` has B*tiles rows of C*C + C floats */
+/* pixel tiles per image of nfdpm_mix_bwd: `part` has B*tiles rows of C*C + C floats (1 for C > 192).  C <= 1024;
+ * above 192 channels dx must not overlap du. */
 int nfdpm_mix_bwd_tiles(int C, int H, int W);
 int nfdpm_mix_bwd(const float* du, int64_t du_bs, const float* da1, int64_t lda1, const float* x, int64_t x_bs,
                   const float* mt, float* dx, int64_t dx_bs, float* part, int B, int C, int H, int W,
@@ -321,7 +324,7 @@ int nfdpm_mix_param_grad(const nfdpm_mix_grad_item* items_host, int n, nfdpm_str
  * d_bias = -g, d_scale_c = -sum_j G_cj M_cj, d_weight = -W^-T diag(e^-s) G W^-T.  weight may be NULL; winv is W^-1 (the
  * identity for a lone ActNorm); any of d_weight / d_scale / d_bias may be NULL.  dld_sum (may be NULL: no log-det term)
  * is sum_b d(ld)[b] for the constant P*(sum s + log|det W|) the inverse accumulates: it adds P*dld_sum*W^-T to d_weight
- * and P*dld_sum to d_scale. */
+ * and P*dld_sum to d_scale.  C <= 1024 (scratch stays C*C + C floats). */
 int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items_host, int n, nfdpm_stream_t stream);
 /* Weight gradients: D[N1,N2] (+)= sum_m A[m,N1]*B[m,N2] (A, B row-major, F32, BF16 or both BF16X2; D fp32 with ldd == N2).
  * Split pairs (needs counters): the tensor-core accumulator holds hi*hi, hi*lo, lo*hi, lo*lo of every logical element and the

@@ -9,7 +9,10 @@
 // All reductions are two-stage with a fixed order (no float atomics): bitwise reproducible.
 #include <stdlib.h>
 
+#include <vector>
+
 #include "tc_common.cuh"
+#include "wide_mix.cuh"
 
 namespace nfdpm {
 
@@ -1185,6 +1188,7 @@ static int mix_bwd_tile(int C, int P) {
 }
 /* number of pixel tiles per image of nfdpm_mix_bwd (rows of `part` per image) */
 extern "C" int nfdpm_mix_bwd_tiles(int C, int H, int W) {
+  if (C > kWideMixMin) return 1;     // mix_bwd_wide: one partial row per image
   const int P = H * W, tp = mix_bwd_tile(C, P);
   return (P + tp - 1) / tp;
 }
@@ -1195,6 +1199,9 @@ extern "C" int nfdpm_mix_bwd(const float* du, int64_t du_bs, const float* da1, i
   NFDPM_REQUIRE(du && x && mt && dx && part, "nfdpm_mix_bwd: null pointer");
   NFDPM_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "nfdpm_mix_bwd: bad shape");
   NFDPM_REQUIRE(da1 == nullptr || (C % 2 == 0 && lda1 >= 9 * (int64_t)(C / 2)), "nfdpm_mix_bwd: bad im2col gradient");
+  NFDPM_REQUIRE(C <= kWideMixMax, "nfdpm_mix_bwd: C=%d > %d unsupported", C, kWideMixMax);
+  if (C > kWideMixMin)
+    return mix_bwd_wide(du, du_bs, da1, lda1, x, x_bs, mt, dx, dx_bs, part, B, C, H, W, as_stream(stream));
   const int P = H * W, TP = mix_bwd_tile(C, P), T = (P + TP - 1) / TP;
   const size_t smem = sizeof(float) * (2 * (size_t)C * (TP + 1) + (size_t)C * C);
   NFDPM_REQUIRE(smem <= 200 * 1024, "nfdpm_mix_bwd: %d channels do not fit shared memory (%zu bytes)", C, smem);
@@ -1238,8 +1245,22 @@ extern "C" int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items, int n,
     const nfdpm_mix_grad_item& s = items[i];
     NFDPM_REQUIRE(s.part && s.winv && s.scratch && s.C > 0 && s.B > 0 && (s.d_scale == nullptr || s.scale != nullptr),
                   "nfdpm_mix_inv_param_grad: item %d incomplete", i);
-    NFDPM_REQUIRE(sizeof(float) * (size_t)s.C * s.C <= 200 * 1024, "nfdpm_mix_inv_param_grad: %d channels do not fit", s.C);
+    NFDPM_REQUIRE(s.C <= kWideMixMax, "nfdpm_mix_inv_param_grad: item %d: C=%d > %d unsupported", i, s.C, kWideMixMax);
   }
+  // wide items (C > 192) run the multi-CTA sequence one at a time; the others keep their batched launches
+  std::vector<const nfdpm_mix_grad_item*> narrow;
+  for (int i = 0; i < n; ++i) {
+    const nfdpm_mix_grad_item& s = items[i];
+    if (s.C <= kWideMixMin) {
+      narrow.push_back(&s);
+      continue;
+    }
+    const int rc = mix_inv_param_grad_wide(s.part, s.B, s.C, s.scale, s.winv, s.dld_sum, s.P, s.d_weight, s.d_scale,
+                                           s.d_bias, s.scratch, as_stream(stream));
+    if (rc != 0) return rc;
+  }
+  if (narrow.empty()) return 0;
+  n = (int)narrow.size();
   static bool attr_set = false;
   if (!attr_set) {
     NFDPM_CUDA(cudaFuncSetAttribute(mix_inv_param_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
@@ -1250,7 +1271,7 @@ extern "C" int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items, int n,
     const int cnt = (n - base < kParamBatch) ? n - base : kParamBatch;
     int cmax = 0;
     for (int i = 0; i < cnt; ++i) {
-      const nfdpm_mix_grad_item& s = items[base + i];
+      const nfdpm_mix_grad_item& s = *narrow[base + i];
       pb.it[i] = MixParamItem{s.part, s.B, s.weight, s.scale, s.bias, s.winv, s.dld_sum, s.P, s.d_weight, s.d_scale,
                               s.d_bias, s.scratch, s.C};
       if (s.C > cmax) cmax = s.C;

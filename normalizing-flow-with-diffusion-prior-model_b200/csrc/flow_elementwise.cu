@@ -5,6 +5,7 @@
 // Roofline: all of these read x once and write y once => 8 bytes per element (fp32 in + out);
 // DESIGN.md §kernels lists the algorithmic bytes per image per StepFlow (8*C*P).
 #include "common.cuh"
+#include "wide_mix.cuh"
 
 namespace nfdpm {
 
@@ -342,8 +343,9 @@ extern "C" int nfdpm_channel_mix(const float* x, float* y, const float* mt, cons
                                  int64_t xbs, int64_t ybs, nfdpm_stream_t stream) {
   NFDPM_REQUIRE(x && y && mt && beta, "nfdpm_channel_mix: null pointer");
   NFDPM_REQUIRE(B > 0 && C > 0 && P > 0, "nfdpm_channel_mix: bad shape B=%d C=%d P=%d", B, C, P);
-  NFDPM_REQUIRE(C <= 192, "nfdpm_channel_mix: C=%d > 192 unsupported", C);
+  NFDPM_REQUIRE(C <= kWideMixMax, "nfdpm_channel_mix: C=%d > %d unsupported", C, kWideMixMax);
   cudaStream_t st = as_stream(stream);
+  if (C > kWideMixMin) return chanmix_wide(x, y, mt, beta, B, C, P, xbs, ybs, st);
   const bool vec = (P % 4 == 0) && (xbs % 4 == 0) && (ybs % 4 == 0) && (((uintptr_t)x | (uintptr_t)y) % 16 == 0);
   if (vec && (C == 4 || C == 8 || C == 12 || C == 16)) {
     const int64_t ng = (int64_t)B * (P / 4);

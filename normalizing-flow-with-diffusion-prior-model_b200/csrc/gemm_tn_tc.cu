@@ -38,6 +38,74 @@ __device__ __forceinline__ uint32_t make_idesc_mn(int M, int N) {
          ((uint32_t)(M >> 4) << 24);
 }
 
+// One item of the split reduction: logical output row n1, columns n2..n2+3 (row rr / column cc of tile (t1, t2)), summed
+// over the `splits` slabs of ws in slab order (split pairs: then hh, hl, lh, ll) and stored in the output's layout.
+__device__ __forceinline__ void tn_reduce_item(const float* __restrict__ ws, float* __restrict__ D, int n1, int n2, int t1,
+                                               int rr, int t2, int cc, int BN, int N2, int64_t slab, int splits, int x3,
+                                               int out_mode, int out_c, int N2L, int accumulate) {
+  int tap = 0, co = 0;
+  if (out_mode == NFDPM_TN_OUT_TAPS) {              // n1 = tap*out_c + co  ->  [co][n2][tap]  (ZeroConv weight)
+    tap = n1 / out_c;
+    co = n1 - tap * out_c;
+    if (tap >= 9) return;
+  } else if (out_mode == NFDPM_TN_OUT_STRIP && n2 >= out_c) {   // keep the first out_c columns
+    return;
+  }
+  // accumulator coordinates of the (hi, hi) entry; the other three components sit 32 rows / columns further
+  const int mrow = x3 ? t1 * 128 + ((rr >> 5) << 6) + (rr & 31) : n1;
+  const int mcol = x3 ? t2 * BN + ((cc >> 5) << 6) + (cc & 31) : n2;
+  const float* src = ws + (int64_t)mrow * N2 + mcol;
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (x3) {
+    for (int s2 = 0; s2 < splits; ++s2) {            // slab order, then hh, hl, lh, ll: fixed => bitwise reproducible
+      const float* p = src + s2 * slab;
+      const float4 v0 = __ldcg(reinterpret_cast<const float4*>(p));
+      const float4 v1 = __ldcg(reinterpret_cast<const float4*>(p + 32));
+      const float4 v2 = __ldcg(reinterpret_cast<const float4*>(p + 32 * (int64_t)N2));
+      const float4 v3 = __ldcg(reinterpret_cast<const float4*>(p + 32 * (int64_t)N2 + 32));
+      acc.x += ((v0.x + v1.x) + v2.x) + v3.x;
+      acc.y += ((v0.y + v1.y) + v2.y) + v3.y;
+      acc.z += ((v0.z + v1.z) + v2.z) + v3.z;
+      acc.w += ((v0.w + v1.w) + v2.w) + v3.w;
+    }
+  } else {
+    int s2 = 0;
+    for (; s2 + 4 <= splits; s2 += 4) {              // four slab loads in flight, added in slab order
+      float4 v[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) v[j] = __ldcg(reinterpret_cast<const float4*>(src + (s2 + j) * slab));
+#pragma unroll
+      for (int j = 0; j < 4; ++j) { acc.x += v[j].x; acc.y += v[j].y; acc.z += v[j].z; acc.w += v[j].w; }
+    }
+    for (; s2 < splits; ++s2) {
+      const float4 v = __ldcg(reinterpret_cast<const float4*>(src + s2 * slab));
+      acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    }
+  }
+  if (out_mode == NFDPM_TN_OUT_PLAIN) {
+    float4* d = reinterpret_cast<float4*>(D + (int64_t)n1 * N2L + n2);
+    if (accumulate) {
+      const float4 o = *d;
+      acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
+    }
+    *d = acc;
+  } else {
+    // layout-changing outputs (the weight tensors' own layouts): four scalar stores
+    const float av[4] = {acc.x, acc.y, acc.z, acc.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      int64_t o;
+      if (out_mode == NFDPM_TN_OUT_TAPS) {
+        o = ((int64_t)co * N2L + n2 + j) * 9 + tap;
+      } else {
+        if (n2 + j >= out_c) break;
+        o = (int64_t)n1 * out_c + n2 + j;
+      }
+      D[o] = accumulate ? D[o] + av[j] : av[j];
+    }
+  }
+}
+
 __global__ void __launch_bounds__(TN_THREADS, 1) gemm_tn_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                                                                    const __grid_constant__ CUtensorMap tmB,
                                                                    float* __restrict__ ws, int M, int N1, int N2, int BN,
@@ -178,68 +246,8 @@ __global__ void __launch_bounds__(TN_THREADS, 1) gemm_tn_tc_kernel(const __grid_
     for (int it = threadIdx.x; it < n_items; it += TN_THREADS) {
       const int r = it / c4, c = it - r * c4;
       const int rr = r_lo + r, cc = 4 * c;
-      const int n1 = t1 * RL + rr, n2 = t2 * CL + cc;             // logical output element (first of four columns)
-      int tap = 0, co = 0;
-      if (out_mode == NFDPM_TN_OUT_TAPS) {              // n1 = tap*out_c + co  ->  [co][n2][tap]  (ZeroConv weight)
-        tap = n1 / out_c;
-        co = n1 - tap * out_c;
-        if (tap >= 9) continue;
-      } else if (out_mode == NFDPM_TN_OUT_STRIP && n2 >= out_c) {   // keep the first out_c columns
-        continue;
-      }
-      // accumulator coordinates of the (hi, hi) entry; the other three components sit 32 rows / columns further
-      const int mrow = x3 ? t1 * 128 + ((rr >> 5) << 6) + (rr & 31) : n1;
-      const int mcol = x3 ? t2 * BN + ((cc >> 5) << 6) + (cc & 31) : n2;
-      const float* src = ws + (int64_t)mrow * N2 + mcol;
-      float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (x3) {
-        for (int s2 = 0; s2 < splits; ++s2) {            // slab order, then hh, hl, lh, ll: fixed => bitwise reproducible
-          const float* p = src + s2 * slab;
-          const float4 v0 = __ldcg(reinterpret_cast<const float4*>(p));
-          const float4 v1 = __ldcg(reinterpret_cast<const float4*>(p + 32));
-          const float4 v2 = __ldcg(reinterpret_cast<const float4*>(p + 32 * (int64_t)N2));
-          const float4 v3 = __ldcg(reinterpret_cast<const float4*>(p + 32 * (int64_t)N2 + 32));
-          acc.x += ((v0.x + v1.x) + v2.x) + v3.x;
-          acc.y += ((v0.y + v1.y) + v2.y) + v3.y;
-          acc.z += ((v0.z + v1.z) + v2.z) + v3.z;
-          acc.w += ((v0.w + v1.w) + v2.w) + v3.w;
-        }
-      } else {
-        int s2 = 0;
-        for (; s2 + 4 <= splits; s2 += 4) {              // four slab loads in flight, added in slab order
-          float4 v[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) v[j] = __ldcg(reinterpret_cast<const float4*>(src + (s2 + j) * slab));
-#pragma unroll
-          for (int j = 0; j < 4; ++j) { acc.x += v[j].x; acc.y += v[j].y; acc.z += v[j].z; acc.w += v[j].w; }
-        }
-        for (; s2 < splits; ++s2) {
-          const float4 v = __ldcg(reinterpret_cast<const float4*>(src + s2 * slab));
-          acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
-        }
-      }
-      if (out_mode == NFDPM_TN_OUT_PLAIN) {
-        float4* d = reinterpret_cast<float4*>(D + (int64_t)n1 * N2L + n2);
-        if (accumulate) {
-          const float4 o = *d;
-          acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
-        }
-        *d = acc;
-      } else {
-        // layout-changing outputs (the weight tensors' own layouts): four scalar stores
-        const float av[4] = {acc.x, acc.y, acc.z, acc.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          int64_t o;
-          if (out_mode == NFDPM_TN_OUT_TAPS) {
-            o = ((int64_t)co * N2L + n2 + j) * 9 + tap;
-          } else {
-            if (n2 + j >= out_c) break;
-            o = (int64_t)n1 * out_c + n2 + j;
-          }
-          D[o] = accumulate ? D[o] + av[j] : av[j];
-        }
-      }
+      tn_reduce_item(ws, D, t1 * RL + rr, t2 * CL + cc, t1, rr, t2, cc, BN, N2, slab, splits, x3, out_mode, out_c, N2L,
+                     accumulate);
     }
   }
   __syncthreads();
@@ -249,6 +257,22 @@ __global__ void __launch_bounds__(TN_THREADS, 1) gemm_tn_tc_kernel(const __grid_
       *done = 0;
       __threadfence();
     }
+  }
+}
+
+// The split reduction of gemm_tn_tc_kernel as a kernel of its own, for grids whose CTAs are not all co-resident (more
+// tiles x splits than SMs, e.g. the split-pair weight gradients of the ZeroConv and the first coupling conv at levels
+// wider than ~260 channels): the same items, the same slab order, hence the same bits as the in-kernel reduction.
+__global__ void __launch_bounds__(256) gemm_tn_reduce_kernel(const float* __restrict__ ws, float* __restrict__ D, int N1L,
+                                                             int N2L, int N2, int BN, int64_t slab, int splits, int x3,
+                                                             int out_mode, int out_c, int accumulate) {
+  const int RL = x3 ? 64 : 128, CL = x3 ? (BN >> 1) : BN, c4 = N2L >> 2;
+  const int64_t n_items = (int64_t)N1L * c4;
+  for (int64_t it = (int64_t)blockIdx.x * 256 + threadIdx.x; it < n_items; it += (int64_t)gridDim.x * 256) {
+    const int n1 = (int)(it / c4), n2 = (int)(it - (int64_t)n1 * c4) * 4;
+    const int t1 = n1 / RL, t2 = n2 / CL;
+    tn_reduce_item(ws, D, n1, n2, t1, n1 - t1 * RL, t2, n2 - t2 * CL, BN, N2, slab, splits, x3, out_mode, out_c, N2L,
+                   accumulate);
   }
 }
 
@@ -310,9 +334,23 @@ int gemm_tn_tc(const void* A, int64_t lda, const void* Bm, int64_t ldb, float* w
     NFDPM_CUDA(cudaFuncSetAttribute(gemm_tn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_set = true;
   }
-  if (tiles > 500 || tiles * splits > sm_count()) counters = nullptr;     // co-residency not guaranteed: reduce separately
   NFDPM_REQUIRE((out_mode == NFDPM_TN_OUT_PLAIN && !x3) || counters != nullptr,
                 "nfdpm_gemm_tn: layout-changing outputs and split-pair operands need the in-kernel reduction (counters)");
+  const bool coresident = !(tiles > 500 || tiles * splits > sm_count());
+  if (!coresident && (out_mode != NFDPM_TN_OUT_PLAIN || x3)) {
+    // slabs to ws, then the same reduction as a separate kernel (plain fp32 / bf16 outputs keep reduce_rows_kernel)
+    gemm_tn_tc_kernel<<<tiles * splits, TN_THREADS, smem, st>>>(tmA, tmB, ws, M, N1, N2, BN, num_n2, splits, per, D,
+                                                               accumulate, nullptr, out_mode, out_c, x3, N1L, N2L);
+    NFDPM_CHECK_LAUNCH("gemm_tn_tc_kernel");
+    const int64_t items = (int64_t)N1L * (N2L >> 2);
+    const int64_t g = (items + 255) / 256;
+    gemm_tn_reduce_kernel<<<(int)(g < 148 * 8 ? g : 148 * 8), 256, 0, st>>>(ws, D, N1L, N2L, N2, BN, (int64_t)N1 * N2,
+                                                                            splits, x3, out_mode, out_c, accumulate);
+    NFDPM_CHECK_LAUNCH("gemm_tn_reduce_kernel");
+    *splits_out = 0;
+    return 0;
+  }
+  if (!coresident) counters = nullptr;     // co-residency not guaranteed: reduce separately
   gemm_tn_tc_kernel<<<tiles * splits, TN_THREADS, smem, st>>>(tmA, tmB, ws, M, N1, N2, BN, num_n2, splits, per, D,
                                                              accumulate, counters, out_mode, out_c, x3, N1L, N2L);
   NFDPM_CHECK_LAUNCH("gemm_tn_tc_kernel");

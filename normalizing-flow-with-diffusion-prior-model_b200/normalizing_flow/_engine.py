@@ -127,6 +127,15 @@ def scalar_f32(device: torch.device, value: float) -> torch.Tensor:
     return t
 
 
+MAX_LEVEL_CHANNELS = 1024      # widest flow level the kernels run (nfdpm_mix_prepare, nfdpm_channel_mix, nfdpm_mix_bwd)
+
+
+def check_width(C: int, what: str) -> None:
+    """Refuses a flow level wider than MAX_LEVEL_CHANNELS, before any launch (e.g. L8 on RGB: 1536 channels)."""
+    if C > MAX_LEVEL_CHANNELS:
+        raise ValueError(f"{what}: a level of {C} channels is wider than the {MAX_LEVEL_CHANNELS} this package supports")
+
+
 def check_input(x: torch.Tensor, what: str = "input") -> torch.Tensor:
     N.require_cuda(x, what)
     if x.dtype != torch.float32:

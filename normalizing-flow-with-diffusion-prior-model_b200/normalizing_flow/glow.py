@@ -117,6 +117,7 @@ class GlowBlock(Transform):
         self.split = Split(flow_channels, learn_prior_mean_logs=learn_prior_mean_logs)
 
     def transform(self, x: Tensor, log_det_jac: Tensor, logp: Tensor) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+        E.check_width(self.flows[0]._C if len(self.flows) else 0, "GlowBlock")
         y, log_det_jac, logp = self.squeeze.transform(x, log_det_jac, logp)
         for flow in self.flows:
             y, log_det_jac, logp = flow.transform(y, log_det_jac, logp)
@@ -125,6 +126,7 @@ class GlowBlock(Transform):
     def invert(self, y: Tensor, latent: Tensor = None, temperature: float = 1.0, *,
                seeds: Optional[Tensor] = None) -> Tensor:
         """``temperature`` / ``seeds`` as in ``Split.invert`` (draw site 0: the draw of ``Glow`` level 0)."""
+        E.check_width(self.flows[0]._C if len(self.flows) else 0, "GlowBlock")
         inv = self.split.invert(y, latent, temperature=temperature, seeds=seeds)
         for flow in reversed(self.flows):
             inv = flow.invert(inv)
@@ -282,6 +284,11 @@ class Glow(Transform):
             self._cmul[key] = t
         return t
 
+    def _check_width(self) -> None:
+        """The final level is the widest (2^(L+1) * in_channel channels).  The constructor accepts any L, as the reference's
+        does (a checkpoint of such a model loads); the calls refuse one wider than the kernels run, before any launch."""
+        E.check_width(2 ** (self.L + 1) * self.in_channel, f"Glow(in_channel={self.in_channel}, L={self.L})")
+
     def _check_image(self, x: Tensor) -> Tuple[int, int, int, int]:
         B, C, H, W = x.shape
         if C != self.in_channel:
@@ -292,6 +299,7 @@ class Glow(Transform):
 
     # ---- forward: x -> ([z_0..z_{L-1}], log_det_jac, logp)
     def transform(self, x: Tensor, log_det_jac: Tensor, logp: Tensor) -> Tuple[list, Tensor, Tensor]:
+        self._check_width()
         x = E.check_input(x)
         B, c, H, W = self._check_image(x)
         if log_det_jac is None:
@@ -338,7 +346,10 @@ class Glow(Transform):
           "image"   one CTA per image (flow_boundary / gemm3_boundary): images of at most 256 pixels in batches that fill the GPU
           "tiled"   row bands with a recomputed halo (flow_boundary_tiled): larger images (the 64x64 / 32x32 levels of a
                     128x128 input) and small batches (config 4: 8 images per GPU would occupy 8 of 148 SMs)
-          "unfused" separate K-A / im2col / coupling kernels (NFDPM_TILED=0, or a single image row beyond shared memory)"""
+          "unfused" separate K-A / im2col / coupling kernels (NFDPM_TILED=0, or a single image row beyond shared memory)
+        Levels wider than 192 channels (the final levels of L6 / L7 models on RGB) take "unfused": both fused-boundary
+        queries refuse them, because their C x C mix matrix does not fit shared memory; nfdpm_channel_mix / nfdpm_mix_bwd
+        run them with their multi-CTA wide kernels."""
         tiled = os.environ.get("NFDPM_TILED", "1") != "0" and N.flow_boundary_tiles(B, C, h, w, 1, 1, 1) > 0
         if cls._level_fast(C, h, w) and (B >= 64 or not tiled):
             return "image"
@@ -560,6 +571,7 @@ class Glow(Transform):
     def _check_invert_args(self, latents: list, log_det_jac: Optional[Tensor], logp: Optional[Tensor]):
         """The argument checks of `invert` / `invert_with_density`, before any launch.  Returns (final latent, whether the
         call is to be recorded by autograd: a latent or a parameter requires grad)."""
+        self._check_width()
         z_last = E.check_input(latents[-1], "latents[-1]")
         B, Cf, h, w = z_last.shape
         if Cf != 2 ** (self.L + 1) * self.in_channel:

@@ -52,6 +52,8 @@ def _granular(what: str):
     and attaches the loud-failure node to its result."""
     def deco(fn):
         def wrapper(self, x, *args, **kw):
+            if what != "Squeeze" and isinstance(x, Tensor) and x.dim() == 4:      # (Split.invert gets the level's half)
+                E.check_width(x.shape[1] * (2 if what == "Split" and fn.__name__ == "invert" else 1), what)
             latent_grad = fn.__name__ == "invert" and E.invert_grad_enabled() and torch.is_grad_enabled() and \
                 any(isinstance(t, Tensor) and t.requires_grad for t in tuple(args) + tuple(kw.values()))
             if not E.autograd_needed(x, self) and not latent_grad:
