@@ -333,7 +333,8 @@ int nfdpm_mix_inv_param_grad(const nfdpm_mix_grad_item* items_host, int n, nfdpm
  * and private to one stream; with it the bf16 tensor-core path sums its split-M partial slabs inside the GEMM kernel
  * (the CTAs of an output tile wait for each other; fixed slab order, so the result stays bitwise reproducible) instead
  * of in a second launch.  The kernel re-arms the counters itself.  out_mode != PLAIN (needs counters + bf16 operands)
- * writes the sum directly in the weight tensor's own layout, saving the unpack launch. */
+ * writes the sum directly in the weight tensor's own layout, saving the unpack launch.  With out_mode PLAIN and either split
+ * pairs or bf16 operands with counters, the reduction stores float4 rows: D must then be 16-byte aligned. */
 int64_t nfdpm_gemm_tn_workspace(int M, int N1, int N2, int* splits_out);
 #define NFDPM_TN_OUT_PLAIN 0 /* D[n1*N2 + n2]                                                               */
 #define NFDPM_TN_OUT_TAPS 1  /* n1 = tap*out_c + co -> D[(co*N2 + n2)*9 + tap]: ZeroConv weight [out_c,N2,3,3] */

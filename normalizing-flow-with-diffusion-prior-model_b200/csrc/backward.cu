@@ -1311,6 +1311,11 @@ extern "C" int nfdpm_gemm_tn(const void* A, int a_dtype, int64_t lda, const void
                 "nfdpm_gemm_tn: bad output mode");
   cudaStream_t st = as_stream(stream);
   const int n = N1 * N2;
+  // the tensor-core reduction (tn_reduce_item) stores float4 rows into a PLAIN D
+  const bool d_vec = out_mode == NFDPM_TN_OUT_PLAIN && (a_dtype == NFDPM_BF16X2 || b_dtype == NFDPM_BF16X2 ||
+                     (counters != nullptr && a_dtype == NFDPM_BF16 && b_dtype == NFDPM_BF16 && gemm_tn_tc_ok(A, lda, Bm, ldb, N1, N2)));
+  NFDPM_REQUIRE(!d_vec || (uintptr_t)D % 16 == 0,
+                "nfdpm_gemm_tn: D must be 16-byte aligned for the tensor-core reduction of a plain output");
   if (a_dtype == NFDPM_BF16X2 || b_dtype == NFDPM_BF16X2) {
     NFDPM_REQUIRE(a_dtype == b_dtype && lda % 32 == 0 && ldb % 32 == 0 && N2 % 4 == 0 && lda >= (N1 + 31) / 32 * 32 &&
                   ldb >= (N2 + 31) / 32 * 32 && ((uintptr_t)A % 16 == 0) && ((uintptr_t)Bm % 16 == 0) && counters != nullptr,

@@ -30,13 +30,6 @@
 
 namespace nfdpm {
 
-constexpr int TC_BM = 128;
-constexpr int TC_BK = 64;            // 64 bf16 = 128 bytes = one swizzle-128B row
-constexpr int TC_STAGES = 3;           // classic layout: 3 x 48 KB ring + a whole-tile (64 KB) output staging buffer
-constexpr int TC_MAX_STAGES = 6;       // deep layout: as many (16 KB + BN x 128 B) stages as fit next to a 64-column staging buffer
-constexpr int TC_A_BYTES = TC_BM * TC_BK * 2;          // 16 KB
-constexpr int TC_B_BYTES_MAX = 256 * TC_BK * 2;        // 32 KB
-constexpr int TC_STAGE_BYTES = TC_A_BYTES + TC_B_BYTES_MAX;
 // Epilogue warps of THIS kernel: four per TMEM lane quadrant.  ncu r1 (source page): with two per quadrant the 8 epilogue
 // warps were busy ~73 % of the kernel (IPC 0.9/SM, latency-bound on tcgen05.ld -> FFMA -> F2FP -> STS chains) and the
 // tensor pipe idled at 41 % waiting for a drained accumulator stage: the kernel was EPILOGUE-bound, not operand-bound
@@ -46,21 +39,13 @@ constexpr int TCG_EPQ = TCG_EPI_WARPS / 4;            // epilogue warps per quad
 constexpr int TC_THREADS = 64 + 32 * TCG_EPI_WARPS;
 __device__ __forceinline__ void epi_barrier_g() { asm volatile("bar.sync 1, %0;" ::"n"(32 * TCG_EPI_WARPS) : "memory"); }
 constexpr int TC_ACC_COLS = 256;     // TMEM columns per accumulator stage
-constexpr int TC_CSTAGE_BYTES = 64 * 1024;   // output staging: 128 rows x 256 bf16 / 128 fp32, as 16 KB swizzled boxes
 
 // persistent tile schedule (tc_sched.h: shared with the host-side unit test)
 __device__ __forceinline__ bool tc_work(int it, int num_tiles, int num_n, int BN, int split, TcWork& w) {
   return tc_work_for((int)blockIdx.x, (int)gridDim.x, it, num_tiles, num_n, BN, split, w);
 }
 
-// Shared-memory plan chosen by the host (gemm_nt_tc):
-//   classic  n_stages = 3, stage_bytes = 48 KB, the epilogue converts the WHOLE tile into a 64 KB staging buffer (cpw = all
-//            chunks of a warp in one pass) and stores it with one burst of TMA box stores;
-//   deep     stage_bytes = 16 KB + BN x 128 B, the staging buffer holds one 64-column PASS (16 KB bf16 / 32 KB fp32, cpw = 1
-//            chunk per warp per pass) and the space goes to the operand ring: 4 x 48 KB stages at BN = 256 (r1 counters: with
-//            3 stages the MMA warp waited for TMA bytes ~25 % of its loop - two stages in flight while one is consumed is
-//            about one L2 round trip at the MMA rate).
-struct TcPlan { int n_stages, stage_bytes, cstage_bytes, cpw; };
+// Shared-memory plan chosen by the host: TcPlan (tc_sched.h)
 
 // profiling hook (nfdpm_gemm_debug): per-CTA cycle counters [grid][16] int64; NULL = off
 __device__ long long* g_tc_dbg = nullptr;
@@ -303,7 +288,7 @@ static int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUten
   static bool attr_set = false;
   if (!attr_set) {
     NFDPM_CUDA(cudaFuncSetAttribute(gemm_nt_tc_kernel<EPI, OutT, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    226 * 1024));
+                                    TC_SMEM_MAX));
     attr_set = true;
   }
   NFDPM_CUDA(launch_pdl(gemm_nt_tc_kernel<EPI, OutT, X3>, dim3(grid), dim3(TC_THREADS), smem, st, tmA, tmB, tmD, M, N, Kmem,
@@ -320,76 +305,36 @@ int gemm_nt_tc(const void* A, int64_t lda, const void* Bw, int64_t ldb, void* D,
   NFDPM_REQUIRE(((uintptr_t)A % 16 == 0) && ((uintptr_t)Bw % 16 == 0) && ((uintptr_t)D % 16 == 0),
                 "nfdpm_gemm_nt(tensor core): operands must be 16-byte aligned");
   NFDPM_REQUIRE(epilogue == NFDPM_EPI_RAW || N <= 2048, "nfdpm_gemm_nt(tensor core): fused ActNorm epilogue supports N <= 2048");
-  // N tile: multiple of 16 that splits N evenly; <= 256 columns for bf16 / split output, <= 128 for fp32 output (the
-  // classic staging tile holds 128 x 256 bf16 or 128 x 128 fp32 / split pairs)
-  static int bn_cap = -1;
+  // the plan's knobs (tc_sched.h tc_nt_plan), read once per process
+  static int bn_cap = -1, narrow_below = -1, split_on = -1, deep_on = -1, sms = 0;
   if (bn_cap < 0) {
     const char* e = getenv("NFDPM_TC_BN");
     bn_cap = e ? atoi(e) : 256;
     if (bn_cap != 64 && bn_cap != 128) bn_cap = 256;
-  }
-  int bn_max = (out_dtype == NFDPM_F32) ? 128 : 256;
-  if (bn_max > bn_cap) bn_max = bn_cap;
-  // few rows (deep levels): narrower tiles put more CTAs to work (measured at M = 2048, N = 512: 6.1 vs 7.2 us; round 2,
-  // per-StepFlow chain over the three levels with narrowing below 48 / 74 / 100 / 148 tiles: 172.3 / 170.1 / 170.9 / 175.4 us
-  // in the split-pair mode, 110.4 / 108.7 / 108.9 / 112.3 us in bf16)
-  const int m_tiles = (M + TC_BM - 1) / TC_BM;
-  static int narrow_below = -1;
-  if (narrow_below < 0) {
-    const char* e = getenv("NFDPM_TC_NARROW");
+    e = getenv("NFDPM_TC_NARROW");
     narrow_below = e ? atoi(e) : 74;
+    e = getenv("NFDPM_TC_SPLIT");                       // 0 keeps whole tiles in the last round
+    split_on = (e && atoi(e) == 0) ? 0 : 1;
+    e = getenv("NFDPM_TC_DEEP");                        // 0: classic plan everywhere, 2: deep plan for every shape
+    deep_on = e ? atoi(e) : 1;
   }
-  while (bn_max > 64 && N >= 2 * bn_max / 2 && m_tiles * ((N + bn_max - 1) / bn_max) <= narrow_below && N % (bn_max / 2) == 0) bn_max >>= 1;
-  const int cpb = (out_dtype == NFDPM_BF16) ? 64 : 32;    // logical columns per 128-byte TMA store box
-  const int nblk = (N + bn_max - 1) / bn_max;
-  // one N block: any multiple of 16 (columns >= N are clipped by the D tensor map); several N blocks: BN must be a
-  // whole number of store boxes, otherwise a tile's last box would spill into its neighbour's columns
-  const int BN = (nblk == 1) ? (N + 15) / 16 * 16 : ((N + nblk - 1) / nblk + cpb - 1) / cpb * cpb;
-  static int sms = 0;
   if (sms == 0) {
     int dev = 0;
     NFDPM_CUDA(cudaGetDevice(&dev));
     NFDPM_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   }
-  const int tiles = ((M + TC_BM - 1) / TC_BM) * ((N + BN - 1) / BN);
-  const int grid = tiles < sms ? tiles : sms;
-  // last-wave balancing (TcWork): split the tiles beyond the last full round into half-width tiles when that puts
-  // them on (almost) every SM; NFDPM_TC_SPLIT=0 keeps whole tiles
-  static int split_on = -1;
-  if (split_on < 0) {
-    const char* e = getenv("NFDPM_TC_SPLIT");
-    split_on = (e && atoi(e) == 0) ? 0 : 1;
-  }
-  const int split = (split_on && tc_split_ok(tiles, grid, BN, N)) ? 1 : 0;
   const int kmul = x3 ? 2 : 1;                           // bf16 columns per logical K
   const int Kmem = K * kmul;
+  const TcNtPlan p = tc_nt_plan(M, N, Kmem, out_dtype == NFDPM_F32, out_dtype == NFDPM_BF16, epilogue != NFDPM_EPI_RAW, sms,
+                                bn_cap, narrow_below, split_on, deep_on);
+  const int BN = p.BN, split = p.split, grid = p.grid;
+  const TcPlan plan = p.plan;
+  const size_t smem = (size_t)p.smem;
   CUtensorMap tmA, tmB, tmD;
   if (make_map(&tmA, A, M, Kmem, lda * kmul, TC_BM)) return 1;
   if (make_map(&tmB, Bw, N, Kmem, ldb * kmul, split ? BN / 2 : BN)) return 1;
   if (out_x2) { if (make_map(&tmD, D, M, 2 * (int64_t)N, 2 * ldd, TC_BM)) return 1; }
   else if (make_map(&tmD, D, M, N, ldd, TC_BM, out_dtype == NFDPM_F32)) return 1;
-  const size_t n_pad = (size_t)((N + BN - 1) / BN) * BN;
-  const size_t extra = (epilogue != NFDPM_EPI_RAW ? 2 * n_pad * 4 : 0);
-  // shared-memory plan (TcPlan): the deep ring pays when the main loop is long enough to be fed from L2 continuously;
-  // NFDPM_TC_DEEP=0 keeps the classic plan everywhere, =2 forces the deep plan for every shape
-  static int deep_on = -1;
-  if (deep_on < 0) {
-    const char* e = getenv("NFDPM_TC_DEEP");
-    deep_on = e ? atoi(e) : 1;
-  }
-  // classic: the 64 KB staging buffer holds 256 bf16 / 128 fp32 / 128 split-pair columns of the tile per pass
-  TcPlan plan = {TC_STAGES, TC_STAGE_BYTES, TC_CSTAGE_BYTES, out_dtype == NFDPM_BF16 ? 4 : 2};
-  // measured (tools/bench_gemms.py): M=32768 N=K=512 22.2 -> 21.7 us, N=112 fp32-out 11.0 -> 10.5 us; with ONE tile per CTA
-  // (deep levels) the pass-wise epilogue has no next main loop to hide behind and costs 0.5 us, so those keep the classic plan
-  if (deep_on == 2 || (deep_on == 1 && Kmem / TC_BK >= 4 && tiles > grid)) {
-    plan.stage_bytes = TC_A_BYTES + BN * TC_BK * 2;
-    plan.cstage_bytes = 128 * 64 * (out_dtype == NFDPM_BF16 ? 2 : 4);     // one 64-column pass
-    plan.cpw = 1;
-    const size_t avail = 226 * 1024 - 1024 - (size_t)plan.cstage_bytes - extra;   // 226 KB dynamic (launch_tc) + static barriers
-    plan.n_stages = (int)(avail / (size_t)plan.stage_bytes);
-    if (plan.n_stages > TC_MAX_STAGES) plan.n_stages = TC_MAX_STAGES;
-  }
-  const size_t smem = 1024 + (size_t)plan.n_stages * plan.stage_bytes + plan.cstage_bytes + extra;
 #define GO(EPI, T, X) return launch_tc<EPI, T, X>(tmA, tmB, tmD, M, N, Kmem, BN, split, plan, ep_scale, ep_bias, grid, smem, st)
   const bool raw = epilogue == NFDPM_EPI_RAW;
   if (x3) {

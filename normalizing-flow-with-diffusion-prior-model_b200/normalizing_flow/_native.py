@@ -7,6 +7,7 @@ only for memory and streams.
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import os
 from typing import Optional
 
@@ -450,10 +451,55 @@ def _tn_counters(dev: torch.device):
 TN_OUT_PLAIN, TN_OUT_TAPS, TN_OUT_STRIP = 0, 1, 2
 
 
+@functools.lru_cache(maxsize=None)
+def _tn_sms() -> int:
+    n = lib.nfdpm_sm_count()
+    return n if n > 0 else 148          # gemm_tn_tc.cu sm_count(): 148 without a device
+
+
+@functools.lru_cache(maxsize=None)
+def gemm_tn_tc_plan(M, N1, N2):
+    """gemm_tn_tc_plan (csrc/gemm_tn_tc.cu) for the kernel's dimensions (bf16 columns): (BN, tiles, splits,
+    k-blocks per split)."""
+    bn = 256 if N2 >= 256 else (N2 + 63) // 64 * 64
+    tiles = ((N1 + 127) // 128) * ((N2 + bn - 1) // bn)
+    num_kb = (M + 63) // 64
+    min_kb = max(1, int(os.environ.get("NFDPM_TN_MIN_KB", "1") or 1))
+    s = max(1, _tn_sms() // tiles)
+    s = max(1, min(s, num_kb // min_kb))
+    per = (num_kb + s - 1) // s
+    return bn, tiles, (num_kb + per - 1) // per, per
+
+
+@functools.lru_cache(maxsize=None)
+def gemm_tn_path(a_dt, b_dt, tc_ok, M, N1, N2, counters, out_mode):
+    """The kernels nfdpm_gemm_tn launches (csrc/backward.cu, gemm_tn_tc.cu): (GEMM, reduction).  GEMM: "x3" (tcgen05,
+    split pairs), "tc" (tcgen05, bf16; tc_ok = gemm_tn_tc_ok) or "simt" (gemm_tn_kernel); reduction: "in_kernel" (the
+    GEMM's CTAs sum their slabs, synchronised through the counters), "tn_reduce" (gemm_tn_reduce_kernel) or
+    "reduce_rows" (reduce_rows_kernel)."""
+    if a_dt == BF16X2 or b_dt == BF16X2:
+        gemm, n1, n2 = "x3", 2 * ((N1 + 31) // 32 * 32), 2 * ((N2 + 31) // 32 * 32)
+    elif a_dt == BF16 and b_dt == BF16 and tc_ok:
+        gemm, n1, n2 = "tc", N1, N2
+    else:
+        return "simt", "reduce_rows"
+    _, tiles, splits, _ = gemm_tn_tc_plan(M, n1, n2)
+    coresident = not (tiles > 500 or tiles * splits > _tn_sms())
+    if not coresident and (out_mode != TN_OUT_PLAIN or gemm == "x3"):
+        return gemm, "tn_reduce"
+    return gemm, "in_kernel" if coresident and counters else "reduce_rows"
+
+
+def gemm_tn_tc_ok(A, lda, Bm, ldb, N2) -> bool:
+    """gemm_tn_tc_ok (csrc/gemm_tn_tc.cu)."""
+    return lda % 8 == 0 and ldb % 8 == 0 and N2 % 16 == 0 and A.data_ptr() % 16 == 0 and Bm.data_ptr() % 16 == 0
+
+
 def gemm_tn(A, lda, Bm, ldb, D, M, N1, N2, ws, accumulate=False, fused_reduce=True, out_mode=TN_OUT_PLAIN, out_c=0) -> None:
     cnt = _tn_counters(A.device) if fused_reduce else None
+    _, red = gemm_tn_path(_dt(A), _dt(Bm), gemm_tn_tc_ok(A, lda, Bm, ldb, N2), M, N1, N2, fused_reduce, out_mode)
     _ok(lib.nfdpm_gemm_tn(_p(A), _dt(A), lda, _p(Bm), _dt(Bm), ldb, _p(D), N2, M, N1, N2, _p(ws), int(accumulate),
-                          _p(cnt), out_mode, out_c, _st()), 1 if fused_reduce else 2)
+                          _p(cnt), out_mode, out_c, _st()), 1 if red == "in_kernel" else 2)
 
 
 def split_prior_bwd(dlp, h, ldh, bias, logs, x, xbs, dstate, dbs, dh, dpar, B, Cc, H, W) -> None:

@@ -68,11 +68,11 @@ def same_bits(a, b):
 
 class Sink:
     """A device output of n elements inside a buffer with SLACK guard elements on both sides, all sentinel-filled (NaN;
-    the int32 word 7 for split pairs) or set to ``init`` (outputs the kernel adds to)."""
+    the int32 word 7 for split pairs) or set to ``init`` (outputs the kernel adds to).  ``slack`` widens the guards."""
     SLACK = 64
 
-    def __init__(self, n, dtype=torch.float32, init=None):
-        S = self.SLACK
+    def __init__(self, n, dtype=torch.float32, init=None, slack=None):
+        S = self.S = slack or self.SLACK
         fill = 7 if dtype == N.SPLIT else float("nan")
         host = torch.full((n + 2 * S,), fill, dtype=dtype)
         if init is not None:
@@ -84,7 +84,7 @@ class Sink:
     def get(self, written=None):
         """The n elements after the kernel.  The slack and the elements outside the boolean mask ``written`` must hold
         exactly what they held before."""
-        S, n = self.SLACK, self.n
+        S, n = self.S, self.n
         got = self.buf.cpu()
         assert same_bits(got[:S], self.before[:S]) and same_bits(got[S + n:], self.before[S + n:]), \
             "write outside the output"

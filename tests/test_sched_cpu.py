@@ -1,7 +1,8 @@
 """Host-side unit test of the tcgen05 GEMM's persistent tile schedule (csrc/tc_sched.h — the same functions the kernel
 calls, compiled here with g++): for every shape, every output element of the [num_m*128, N] result is produced by
 exactly one unit of work, every CTA's work list is the same for its three warp roles by construction, half tiles appear
-only in the last round and only where the host enabled them, and the last-wave split never makes the longest CTA longer."""
+only in the last round and only where the host enabled them, and the last-wave split never makes the longest CTA longer.
+The launch plan (tc_nt_plan, with the default knobs) keeps the invariants the kernel relies on over a grid of shapes."""
 import os
 import subprocess
 import sys
@@ -72,3 +73,62 @@ def test_tile_schedule_covers_every_output_exactly_once(tmp_path):
     r = subprocess.run([str(exe)], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout[-2000:]
     assert r.stdout.startswith("ok") and int(r.stdout.split()[3]) > 0, r.stdout
+
+
+PLAN_HARNESS = r"""
+#include <cstdio>
+#include "tc_sched.h"
+using namespace nfdpm;
+#define FAIL(msg) do { printf("%s: M %d N %d Kmem %d out %d actnorm %d sms %d BN %d split %d stages %d smem %d\n", msg, M, N, \
+                              Kmem, out, (int)act, sms, p.BN, p.split, p.plan.n_stages, p.smem); return 1; } while (0)
+int main() {
+  const int Ms[] = {1, 77, 128, 129, 300, 2048, 4096, 8192, 32768, 50000, 131072};
+  const int Ks[] = {64, 128, 192, 256, 512, 1024, 2048};
+  const int smss[] = {148, 132, 8};
+  long long cases = 0, deep = 0, split = 0, narrowed = 0;
+  for (int sms : smss)
+    for (int M : Ms)
+      for (int N = 16; N <= 4096; N += (N < 1024 ? 16 : 112))
+        for (int Kmem : Ks)
+          for (int out = 0; out < 3; ++out)                     // 0 fp32, 1 bf16, 2 split pairs
+            for (int a = 0; a < 2; ++a) {
+              const bool act = a == 1, f32 = out == 0, bf16 = out == 1;
+              if (out == 2 && N % 32) continue;                 // split-pair rows hold whole groups of 32 columns
+              if (act && N > 2048) continue;                    // the fused ActNorm epilogue supports N <= 2048
+              const TcNtPlan p = tc_nt_plan(M, N, Kmem, f32, bf16, act, sms, 256, 74, 1, 1);
+              ++cases;
+              const int cpb = bf16 ? 64 : 32;
+              if (p.BN > 256 || p.BN % 16 || p.BN < 16) FAIL("BN out of range");
+              if (f32 && p.BN > 128) FAIL("fp32 output BN > 128");
+              if (p.num_n > 1 && p.BN % cpb) FAIL("several N blocks, BN not whole store boxes");
+              if (p.num_n * p.BN < N || (p.num_n - 1) * p.BN >= N) FAIL("N blocks do not cover N exactly");
+              if (p.tiles != (M + TC_BM - 1) / TC_BM * p.num_n) FAIL("tile count");
+              if (p.grid != (p.tiles < sms ? p.tiles : sms)) FAIL("grid");
+              if (p.plan.n_stages < 2 || p.plan.n_stages > TC_MAX_STAGES) FAIL("n_stages out of range");
+              if (p.smem > TC_SMEM_MAX) FAIL("shared memory over 226 KB");
+              if (p.split && !tc_split_ok(p.tiles, p.grid, p.BN, N)) FAIL("split without tc_split_ok");
+              const int extra = act ? 2 * p.num_n * p.BN * 4 : 0;
+              if (p.smem != 1024 + p.plan.n_stages * p.plan.stage_bytes + p.plan.cstage_bytes + extra) FAIL("smem sum");
+              if (p.plan.stage_bytes < TC_A_BYTES + p.BN * TC_BK * 2) FAIL("stage smaller than its boxes");
+              // the staging buffer holds what one pass of the epilogue stores
+              const int pass_cols = p.plan.cpw * 64 < p.BN ? p.plan.cpw * 64 : p.BN;
+              if (p.plan.cstage_bytes < 128 * pass_cols * (bf16 ? 2 : 4)) FAIL("staging smaller than one pass");
+              if (p.plan.cpw == 1 ? p.plan.cstage_bytes != 128 * 64 * (bf16 ? 2 : 4) : p.plan.cstage_bytes != TC_CSTAGE_BYTES)
+                FAIL("staging size");
+              deep += p.plan.cpw == 1; split += p.split;
+              narrowed += p.BN < (N < (f32 ? 128 : 256) ? N : (f32 ? 128 : 256)) && p.num_n > 1;
+            }
+  printf("ok %lld cases, %lld deep, %lld split, %lld narrowed\n", cases, deep, split, narrowed);
+  return (deep && split && narrowed) ? 0 : 1;
+}
+"""
+
+
+def test_launch_plan_invariants(tmp_path):
+    src = tmp_path / "plan.cpp"
+    src.write_text(PLAN_HARNESS)
+    exe = tmp_path / "plan"
+    r = subprocess.run(["g++", "-std=c++17", "-O1", "-I", HDR, str(src), "-o", str(exe)], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-3000:]
+    r = subprocess.run([str(exe)], capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and r.stdout.startswith("ok"), r.stdout[-2000:]
